@@ -256,8 +256,19 @@ enum { SZB_TRAIN_FORWARD_ONLY = 1,   /* losses only */
 enum { SZB_TRAIN_PARAMS = 0,         /* parameters and BatchNorm running buffers */
        SZB_TRAIN_GRADS = 1,          /* gradients of the last step */
        SZB_TRAIN_EXP_AVG = 2, SZB_TRAIN_EXP_AVG_SQ = 3,    /* Adam moments */
-       SZB_TRAIN_ACTIVATIONS = 4 };  /* read-only: "logits" [n][4672], "value" [n] of the last step */
+       SZB_TRAIN_ACTIVATIONS = 4,    /* read-only: "logits" [n][4672], "value" [n] of the last step */
+       SZB_TRAIN_MOMENTUM_BUFFER = 5 };  /* SGD with momentum only: torch's per-parameter "momentum_buffer"; setting it marks the
+                                          * buffers as existing (a resumed state), so the next step blends into them */
+enum { SZB_TRAIN_ADAM = 0, SZB_TRAIN_SGD = 1 };
 int szb_train_create(szb_ctx *ctx, const szb_train_config *cfg);
+/* the optimiser of the trainer: Adam (the default, train_RL.py:187) or torch.optim.SGD(lr, momentum, dampening, weight_decay,
+ * nesterov) with StepLR(lr_step, lr_gamma) stepped per batch, the supervised recipe of train_supervised.py:84-92.  SGD reads lr,
+ * weight_decay, lr_step, lr_gamma and step0 from the config and ignores beta1, beta2 and eps; weight decay applies to every
+ * parameter, BatchNorm's included.  Call after szb_train_create and before the first szb_train_step (SZB_ERR_STATE after it);
+ * SZB_ERR_ARG for an unknown kind, negative momentum or dampening, or nesterov without momentum or with dampening.  Under SGD
+ * the Adam moment kinds of szb_train_get / szb_train_set return SZB_ERR_STATE, and SZB_TRAIN_MOMENTUM_BUFFER is valid when
+ * momentum is not 0. */
+int szb_train_set_optimizer(szb_ctx *ctx, int32_t kind, float momentum, float dampening, int32_t nesterov);
 int szb_train_destroy(szb_ctx *ctx);
 /* copy named tensors (host or device pointers, fp32, torch layout) into / out of the trainer; `kind` as above.  Setting
  * SZB_TRAIN_PARAMS needs every parameter and running buffer of the state_dict once before the first step. */

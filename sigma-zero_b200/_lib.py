@@ -56,7 +56,8 @@ class TrainConfig(ctypes.Structure):
 
 
 TRAIN_FORWARD_ONLY, TRAIN_NO_UPDATE = 1, 2
-TRAIN_PARAMS, TRAIN_GRADS, TRAIN_EXP_AVG, TRAIN_EXP_AVG_SQ, TRAIN_ACTIVATIONS = 0, 1, 2, 3, 4
+TRAIN_PARAMS, TRAIN_GRADS, TRAIN_EXP_AVG, TRAIN_EXP_AVG_SQ, TRAIN_ACTIVATIONS, TRAIN_MOMENTUM_BUFFER = 0, 1, 2, 3, 4, 5
+TRAIN_ADAM, TRAIN_SGD = 0, 1
 
 _vp, _i32, _u64, _f32 = ctypes.c_void_p, ctypes.c_int32, ctypes.c_uint64, ctypes.c_float
 SIGNATURES = {
@@ -93,6 +94,7 @@ SIGNATURES = {
     "szb_time_kernel": (ctypes.c_int, [_vp, _i32, _i32, _i32, ctypes.POINTER(_f32)]),
     "szb_tower_spans_record": (ctypes.c_int, [_vp, _i32, ctypes.POINTER(TowerSpans)]),
     "szb_train_create": (ctypes.c_int, [_vp, ctypes.POINTER(TrainConfig)]),
+    "szb_train_set_optimizer": (ctypes.c_int, [_vp, _i32, _f32, _f32, _i32]),
     "szb_train_destroy": (ctypes.c_int, [_vp]),
     "szb_train_set": (ctypes.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),
     "szb_train_get": (ctypes.c_int, [_vp, _i32, _i32, _vp, _vp, _vp]),

@@ -1188,6 +1188,30 @@ __global__ void k_adam(float* w, const float* g, float* m, float* v, size_t n, c
     w[i] = p - step_size * (mm / (sqrtf(vv) / bc2_sqrt + eps));
 }
 
+// torch.optim.SGD (_single_tensor_sgd): the same device step counter and StepLR learning rate, no bias correction.  hyper[1] records
+// whether the momentum buffers existed BEFORE this step (torch's first step clones the gradient instead of blending it in); the flag is
+// then raised for the steps after, all on the device, so a captured step replays the first and the later steps alike
+__global__ void k_hyper_sgd(long long* step, float lr0, float lr_gamma, int lr_step, int32_t* have_buf, float* hyper) {
+    const long long t = ++*step;
+    hyper[0] = (float)((double)lr0 * pow((double)lr_gamma, (double)((t - 1) / (lr_step > 0 ? lr_step : 1))));
+    hyper[1] = *have_buf ? 1.f : 0.f;
+    *have_buf = 1;
+}
+
+__global__ void k_sgd(float* w, const float* g, float* buf, size_t n, const float* hyper, float momentum, float dampening, int nesterov, float wd) {
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float lr = hyper[0];
+    const float p = w[i];
+    float d = g[i] + wd * p;
+    if (momentum != 0.f) {
+        const float b = hyper[1] != 0.f ? momentum * buf[i] + (1.f - dampening) * d : d;
+        buf[i] = b;
+        d = nesterov ? d + momentum * b : b;
+    }
+    w[i] = p - lr * d;
+}
+
 struct PackDesc {
     const float* w;      // master [cout_pad][taps][cin_pad]
     bf16* wf;            // forward pack, same layout
@@ -1291,6 +1315,12 @@ struct Trainer {
     int64_t rec_n = 0;
     int64_t step = 0;                            // host mirror of *d_step
     long long* d_step = nullptr; float* hyper = nullptr;
+    // optimiser (szb_train_set_optimizer): fixed before the first step, so no captured step depends on it.  SGD keeps its momentum
+    // buffers in `m` (Adam's first moment, unused under SGD); *d_have_buf: they hold a value (torch's "momentum_buffer" state exists)
+    int32_t opt_kind = SZB_TRAIN_ADAM;
+    float momentum = 0.f, dampening = 0.f;
+    int32_t nesterov = 0;
+    int32_t* d_have_buf = nullptr;
     int32_t* rows_host = nullptr;                // [ROWS_RING][cap] pinned staging of the steps' row numbers
     cudaEvent_t rows_ev[8] = {};
     bool rows_used[8] = {};
@@ -1491,6 +1521,7 @@ static int t_create(szb_ctx* ctx, const szb_train_config* cfg) {
         (rc = t_alloc(ctx, tr, &tr->v_running, 4)) || (rc = t_alloc(ctx, tr, &tr->vstat, 1)) || (rc = t_alloc(ctx, tr, &tr->losses, 2)) ||
         (rc = t_alloc(ctx, tr, &tr->error, 1)) || (rc = t_alloc(ctx, tr, &tr->rows, (size_t)cap)) ||
         (rc = t_alloc(ctx, tr, &tr->pack_descs, (size_t)T_LAYERS)) || (rc = t_alloc(ctx, tr, &tr->d_step, 1)) || (rc = t_alloc(ctx, tr, &tr->hyper, 2)) ||
+        (rc = t_alloc(ctx, tr, &tr->d_have_buf, 1)) ||
         (rc = t_alloc(ctx, tr, &tr->loss_hist, (size_t)2 * LOSS_HIST)) || (rc = t_alloc(ctx, tr, &tr->hist_count, 1)))
         return rc;
     SZB_CUDA(ctx, cudaMallocHost((void**)&tr->rows_host, (size_t)ROWS_RING * cap * 4));
@@ -1545,13 +1576,20 @@ static int t_pack(szb_ctx* ctx, Trainer* tr) {
     return 0;
 }
 
-static float* t_kind_base(Trainer* tr, int kind) { return kind == 0 ? tr->w : kind == 1 ? tr->g : kind == 2 ? tr->m : kind == 3 ? tr->v : nullptr; }
+static float* t_kind_base(Trainer* tr, int kind) {
+    return kind == 0 ? tr->w : kind == 1 ? tr->g : (kind == 2 || kind == SZB_TRAIN_MOMENTUM_BUFFER) ? tr->m : kind == 3 ? tr->v : nullptr;
+}
 
 // copy tensors by name between caller memory (host or device, torch layout) and the flat buffers
 static int t_transfer(szb_ctx* ctx, int kind, int32_t n_tensors, const char* const* names, float* const* data, const int64_t* numel, bool to_trainer) {
     Trainer* tr = ctx->trainer;
     if (!tr) return fail(ctx, SZB_ERR_ARG, "no trainer: call szb_train_create first");
-    if (kind < 0 || kind > 4 || n_tensors < 0 || (n_tensors && (!names || !data || !numel))) return fail(ctx, SZB_ERR_ARG, "szb_train_get/set: bad arguments");
+    if (kind < 0 || kind > SZB_TRAIN_MOMENTUM_BUFFER || n_tensors < 0 || (n_tensors && (!names || !data || !numel)))
+        return fail(ctx, SZB_ERR_ARG, "szb_train_get/set: bad arguments");
+    const bool sgd = tr->opt_kind == SZB_TRAIN_SGD;
+    if ((kind == SZB_TRAIN_EXP_AVG || kind == SZB_TRAIN_EXP_AVG_SQ) && sgd) return fail(ctx, SZB_ERR_STATE, "the trainer runs SGD: it has no Adam moments");
+    if (kind == SZB_TRAIN_MOMENTUM_BUFFER && !(sgd && tr->momentum != 0.f))
+        return fail(ctx, SZB_ERR_STATE, "momentum buffers exist only under SGD with momentum (szb_train_set_optimizer)");
     float* scratch = nullptr;
     int rc = 0;
     for (int i = 0; i < n_tensors && !rc; i++) {
@@ -1617,6 +1655,11 @@ static int t_transfer(szb_ctx* ctx, int kind, int32_t n_tensors, const char* con
         for (bool b : tr->have_param) tr->loaded = tr->loaded && b;
         for (bool b : tr->have_buffer) tr->loaded = tr->loaded && b;
         rc = t_pack(ctx, tr);
+    }
+    if (!rc && to_trainer && kind == SZB_TRAIN_MOMENTUM_BUFFER && n_tensors > 0) {
+        const int32_t one = 1;                   // a resumed torch state: the next step blends into these buffers instead of starting them
+        SZB_CUDA(ctx, cudaMemcpyAsync(tr->d_have_buf, &one, 4, cudaMemcpyHostToDevice, ctx->stream));
+        SZB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
     }
     return rc;
 }
@@ -1774,8 +1817,14 @@ static int t_step_launches(szb_ctx* ctx, Trainer* tr, int n, int flags) {
         if ((rc = t_wgrad(ctx, tr, 1, 38, n))) return rc;         // every tower convolution's weight gradient
         if (!(flags & SZB_TRAIN_NO_UPDATE)) {
             const szb_train_config& c = tr->cfg;
-            k_hyper<<<1, 1, 0, st>>>(tr->d_step, c.lr, c.lr_gamma, c.lr_step, c.beta1, c.beta2, tr->hyper);
-            k_adam<<<(unsigned)((tr->total + 255) / 256), 256, 0, st>>>(tr->w, tr->g, tr->m, tr->v, tr->total, tr->hyper, c.beta1, c.beta2, c.eps, c.weight_decay);
+            if (tr->opt_kind == SZB_TRAIN_SGD) {
+                k_hyper_sgd<<<1, 1, 0, st>>>(tr->d_step, c.lr, c.lr_gamma, c.lr_step, tr->d_have_buf, tr->hyper);
+                k_sgd<<<(unsigned)((tr->total + 255) / 256), 256, 0, st>>>(tr->w, tr->g, tr->m, tr->total, tr->hyper, tr->momentum, tr->dampening,
+                                                                          tr->nesterov, c.weight_decay);
+            } else {
+                k_hyper<<<1, 1, 0, st>>>(tr->d_step, c.lr, c.lr_gamma, c.lr_step, c.beta1, c.beta2, tr->hyper);
+                k_adam<<<(unsigned)((tr->total + 255) / 256), 256, 0, st>>>(tr->w, tr->g, tr->m, tr->v, tr->total, tr->hyper, c.beta1, c.beta2, c.eps, c.weight_decay);
+            }
             ctx->launches += 2;
             if ((rc = t_pack(ctx, tr))) return rc;
         }
@@ -1869,6 +1918,25 @@ int szb_train_create(szb_ctx* ctx, const szb_train_config* cfg) {
     cudaSetDevice(ctx->device);
     if (cfg->batch < 2 || cfg->batch > 4096) return fail(ctx, SZB_ERR_ARG, "szb_train_create: batch must be 2..4096");
     return t_create(ctx, cfg);
+}
+
+int szb_train_set_optimizer(szb_ctx* ctx, int32_t kind, float momentum, float dampening, int32_t nesterov) {
+    if (!ctx) return SZB_ERR_ARG;
+    Trainer* tr = ctx->trainer;
+    if (!tr) return fail(ctx, SZB_ERR_STATE, "no trainer: call szb_train_create first");
+    if (tr->steps_run > 0) return fail(ctx, SZB_ERR_STATE, "szb_train_set_optimizer: a step has already run");
+    if (kind != SZB_TRAIN_ADAM && kind != SZB_TRAIN_SGD) return fail(ctx, SZB_ERR_ARG, "szb_train_set_optimizer: unknown optimiser %d", (int)kind);
+    if (kind == SZB_TRAIN_SGD) {
+        // torch.optim.SGD's constructor rules (and a dampening that is a number, not negative)
+        if (!(momentum >= 0.f) || !(dampening >= 0.f)) return fail(ctx, SZB_ERR_ARG, "szb_train_set_optimizer: negative momentum or dampening");
+        if (nesterov && (momentum <= 0.f || dampening != 0.f))
+            return fail(ctx, SZB_ERR_ARG, "szb_train_set_optimizer: Nesterov momentum requires a momentum and zero dampening");
+    }
+    tr->opt_kind = kind;
+    tr->momentum = kind == SZB_TRAIN_SGD ? momentum : 0.f;
+    tr->dampening = kind == SZB_TRAIN_SGD ? dampening : 0.f;
+    tr->nesterov = kind == SZB_TRAIN_SGD && nesterov ? 1 : 0;
+    return 0;
 }
 
 int szb_train_destroy(szb_ctx* ctx) {

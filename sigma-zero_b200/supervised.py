@@ -1,5 +1,6 @@
-"""Supervised data path of the reference (SURVEY.md 8f rank 3): PGN games -> packed training positions with the played move as
-a one-hot policy target (generate_training_supervised.py:11-115), and the SGD recipe of train_supervised.py:84-92.
+"""Supervised path of the reference (SURVEY.md 8f rank 3): PGN games -> packed training positions with the played move as
+a one-hot policy target (generate_training_supervised.py:11-115), the SGD recipe of train_supervised.py:84-92, and main(), the
+training loop from a PGN file to supervised_model_best.pt on the library's trainer.
 
 The reference replays each PGN game through python-chess and ChessTensor one move at a time on the host and stores a
 bit-compressed uint8[119,8] tensor per position.  Here all selected games are replayed IN LOCK STEP on the GPU engine: one
@@ -248,7 +249,116 @@ def compressed_states(records, rows=None):
 
 
 def make_supervised_optimiser(model, lr=0.1, weight_decay=1e-4, lr_step_size=4000):
-    """SGD + StepLR(4000, 0.5) of train_supervised.py:84-92; train with train_RL.train_on_records(model, records, ...)"""
+    """SGD + StepLR(4000, 0.5) of train_supervised.py:84-92, the scheduler stepped per batch.  Train with
+    train_RL.train_on_records(model, records, optimiser=opt, lr_scheduler=sched): on a CUDA device the library's trainer runs the
+    SGD update (szb_train_set_optimizer), elsewhere torch does; main() below is the whole loop from PGN to checkpoint."""
     import torch
     opt = torch.optim.SGD(model.parameters(), lr=lr, weight_decay=weight_decay)
     return opt, torch.optim.lr_scheduler.StepLR(opt, step_size=lr_step_size, gamma=0.5)
+
+
+# ---------------------------------------------------------------------------------------------------
+# training from PGN: python -m sigma_zero_b200.supervised --pgn games.pgn.bz2
+# ---------------------------------------------------------------------------------------------------
+def split_holdout(games, fraction=0.02, seed=0):
+    """(train, held_out): a seeded random `fraction` of the GAMES is held out, so that no position of a held-out game is trained on.
+    At least one game is held out when fraction > 0 and at least one is kept for training; both lists keep file order."""
+    games = list(games)
+    n_hold = int(round(fraction * len(games)))
+    if fraction > 0 and len(games) >= 2:
+        n_hold = min(max(n_hold, 1), len(games) - 1)
+    hold = set(np.random.default_rng(seed).permutation(len(games))[:n_hold].tolist())
+    return [g for i, g in enumerate(games) if i not in hold], [g for i, g in enumerate(games) if i in hold]
+
+
+def main(pgn, num_games=0, holdout=0.02, epochs=10, batch_size=128, weights=None, out_dir=".", start_epoch=1, seed=0, model=None, log=print):
+    """Supervised pre-training, the loop of train_supervised.py on the GPU library: the balanced selection of `pgn`'s games
+    (select_balanced), a seeded held-out fraction of them (split_holdout), both replayed into records (pgn_to_records); then for each
+    epoch in [start_epoch, epochs]: one pass of SGD + StepLR (make_supervised_optimiser) over the training records on the library's
+    trainer, the held-out losses in eval mode (train_RL.evaluate_records), and out_dir/saves/supervised_{epoch}.pt,
+    supervised_opt_{epoch}.pt and supervised_sched_{epoch}.pt.  The epoch with the lowest held-out loss (mse + ce; the training loss
+    when nothing is held out) is also written as out_dir/supervised_model_best.pt -- the file train_RL.main(weights=...) and
+    PlayTensor(model_path=...) start from -- with its losses in supervised_model_best.json.  start_epoch N resumes weights,
+    optimiser and scheduler from epoch N - 1, as train_RL.main does.  Returns (model, per-epoch history)."""
+    import json
+    import os
+    import time
+
+    import torch
+
+    from .network import policyNN
+    from .train_RL import evaluate_records, train_on_records
+    games = select_balanced(read_pgn(pgn), num_games)
+    train_games, held_games = split_holdout(games, holdout, seed)
+    rec = pgn_to_records(train_games)
+    held = pgn_to_records(held_games) if held_games else None
+    if len(rec["z"]) < 2:
+        raise ValueError("%d training positions: too few to train on" % len(rec["z"]))
+    log("%d games (%d positions) to train on, %d held out (%d positions)"
+        % (len(train_games), len(rec["z"]), len(held_games), 0 if held is None else len(held["z"])))
+    if model is None:
+        model = policyNN({})
+    if weights:
+        model.load_state_dict(torch.load(weights, map_location="cpu"))
+    model.to("cuda")                     # before the optimiser exists: a resumed optimiser state must live where the parameters train
+    optimiser, scheduler = make_supervised_optimiser(model)
+    saves = os.path.join(out_dir, "saves")
+    os.makedirs(saves, exist_ok=True)
+    path = lambda kind, epoch: os.path.join(saves, "supervised_%s%d.pt" % (kind, epoch))
+    best_pt, best_json = os.path.join(out_dir, "supervised_model_best.pt"), os.path.join(out_dir, "supervised_model_best.json")
+    best = None
+    if start_epoch > 1:
+        try:
+            model.load_state_dict(torch.load(path("", start_epoch - 1), map_location="cpu"))
+            optimiser.load_state_dict(torch.load(path("opt_", start_epoch - 1), map_location="cpu"))
+            scheduler.load_state_dict(torch.load(path("sched_", start_epoch - 1), map_location="cpu"))
+            if os.path.exists(best_json):
+                with open(best_json) as f:
+                    best = json.load(f)
+        except OSError:
+            log("No saved weights from epoch %d found!" % (start_epoch - 1))
+            start_epoch = 1
+    history = []
+    for epoch in range(start_epoch, epochs + 1):
+        t0 = time.perf_counter()
+        hist = train_on_records(model, rec, epochs=1, batch_size=batch_size, optimiser=optimiser, lr_scheduler=scheduler, device="cuda",
+                                seed=seed + epoch)
+        seconds = time.perf_counter() - t0
+        mse, ce = (float(x) for x in np.mean(hist, axis=0))
+        h_mse, h_ce = evaluate_records(model, held) if held is not None else (float("nan"), float("nan"))
+        torch.save(model.state_dict(), path("", epoch))
+        torch.save(optimiser.state_dict(), path("opt_", epoch))
+        torch.save(scheduler.state_dict(), path("sched_", epoch))
+        loss = h_mse + h_ce if held is not None else mse + ce
+        if best is None or loss < best["loss"]:
+            best = {"epoch": epoch, "loss": loss, "heldout_mse": h_mse, "heldout_ce": h_ce, "train_mse": mse, "train_ce": ce}
+            torch.save(model.state_dict(), best_pt)
+            with open(best_json, "w") as f:
+                json.dump(best, f)
+        positions = len(hist) * min(batch_size, len(rec["z"]))
+        history.append({"epoch": epoch, "steps": len(hist), "train_mse": mse, "train_ce": ce, "heldout_mse": h_mse, "heldout_ce": h_ce,
+                        "seconds": seconds, "positions_per_sec": positions / seconds, "lr": scheduler.get_last_lr()[0]})
+        log("epoch %d: train mse %.4f ce %.4f | held-out mse %.4f ce %.4f | %.2f s, %.0f positions/s%s"
+            % (epoch, mse, ce, h_mse, h_ce, seconds, positions / seconds, " (best)" if best["epoch"] == epoch else ""))
+    return model, history
+
+
+def parse_args(argv=None):
+    """command line -> keyword arguments of main()"""
+    import argparse
+    ap = argparse.ArgumentParser(description="supervised pre-training on PGN games (SGD + StepLR, train_supervised.py) on the B200 "
+                                             "library's trainer; writes supervised_model_best.pt for train_RL --weights")
+    ap.add_argument("--pgn", required=True, help="PGN file, plain text or .bz2")
+    ap.add_argument("--num_games", type=int, default=0, help="balanced selection of this many games (0: every game with a result)")
+    ap.add_argument("--holdout", type=float, default=0.02, help="fraction of the games held out for the eval-mode loss")
+    ap.add_argument("--epochs", type=int, default=10, help="last epoch to train")
+    ap.add_argument("--batch_size", type=int, default=128)
+    ap.add_argument("--weights", default=None, help="state_dict to start from")
+    ap.add_argument("--out_dir", default=".")
+    ap.add_argument("--start_epoch", type=int, default=1, help="resume from the files of epoch start_epoch - 1")
+    ap.add_argument("--seed", type=int, default=0, help="held-out split and batch order")
+    return vars(ap.parse_args(argv))
+
+
+if __name__ == "__main__":
+    main(**parse_args())

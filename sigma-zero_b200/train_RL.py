@@ -16,6 +16,8 @@ import os
 
 import torch
 
+from ._lib import EVAL_NET_BF16
+
 DEFAULT_ARGS = {
     'C': 2,
     'num_searches': 100,
@@ -139,24 +141,45 @@ def _batches(n, batch_size, epochs, seed):
             yield rows
 
 
-def train_on_records_cuda(model, rec, epochs=1, batch_size=64, optimiser=None, lr_scheduler=None, seed=0, log=None, engine=None):
-    """train_on_records on the GPU library's trainer (szb_train_*, csrc/train.cu): same batches, same recipe, no torch op in the step.
-    `optimiser` / `lr_scheduler` (torch objects, optional) carry the state between calls and into checkpoints: their moments, step
-    counter and hyper-parameters are loaded into the trainer first and written back after the last batch."""
-    from . import runtime
-    from .trainer import Trainer
-    eng = engine if engine is not None else runtime.get_engine()
-    hp, step0 = {}, 0
+def trainer_hparams(optimiser, lr_scheduler):
+    """(optimiser kind, Trainer hyper-parameters, step0) of a torch optimiser and StepLR scheduler (either may be None).
+    torch.optim.Adam and torch.optim.SGD with one param group are what the library's trainer implements; anything else raises
+    TypeError -- train it with backend="torch"."""
+    kind, hp, step0 = "adam", {}, 0
     if optimiser is not None:
+        if type(optimiser) not in (torch.optim.Adam, torch.optim.SGD):
+            raise TypeError("the CUDA trainer implements torch.optim.Adam and torch.optim.SGD, not %s: use backend=\"torch\""
+                            % type(optimiser).__name__)
+        if len(optimiser.param_groups) != 1:
+            raise TypeError("the CUDA trainer takes one param group, not %d: use backend=\"torch\"" % len(optimiser.param_groups))
         g = optimiser.param_groups[0]
-        hp = dict(lr=float(g.get("initial_lr", g["lr"])), beta1=float(g["betas"][0]), beta2=float(g["betas"][1]), eps=float(g["eps"]),
-                  weight_decay=float(g["weight_decay"]))
+        if g.get("maximize", False):
+            raise TypeError("the CUDA trainer minimises; maximize=True needs backend=\"torch\"")
+        if type(optimiser) is torch.optim.SGD:
+            kind = "sgd"
+            hp = dict(lr=float(g["initial_lr"] if lr_scheduler is not None and "initial_lr" in g else g["lr"]), weight_decay=float(g["weight_decay"]),
+                      momentum=float(g["momentum"]), dampening=float(g["dampening"]), nesterov=bool(g["nesterov"]))
+        else:
+            hp = dict(lr=float(g.get("initial_lr", g["lr"])), beta1=float(g["betas"][0]), beta2=float(g["betas"][1]), eps=float(g["eps"]),
+                      weight_decay=float(g["weight_decay"]))
     if lr_scheduler is not None:
         hp.update(lr_step=int(lr_scheduler.step_size), lr_gamma=float(lr_scheduler.gamma))
         step0 = int(lr_scheduler.last_epoch)
     else:
         hp.update(lr_step=1 << 30, lr_gamma=1.0)
-    tr = Trainer(eng, model, batch_size=batch_size, step0=step0, **hp)
+    return kind, hp, step0
+
+
+def train_on_records_cuda(model, rec, epochs=1, batch_size=64, optimiser=None, lr_scheduler=None, seed=0, log=None, engine=None):
+    """train_on_records on the GPU library's trainer (szb_train_*, csrc/train.cu): same batches, same recipe, no torch op in the step.
+    `optimiser` / `lr_scheduler` (torch objects, optional: torch.optim.Adam or torch.optim.SGD, StepLR) carry the state between calls
+    and into checkpoints: their moments or momentum buffers, step counter and hyper-parameters are loaded into the trainer first and
+    written back after the last batch."""
+    from . import runtime
+    from .trainer import Trainer
+    kind, hp, step0 = trainer_hparams(optimiser, lr_scheduler)
+    eng = engine if engine is not None else runtime.get_engine()
+    tr = Trainer(eng, model, batch_size=batch_size, step0=step0, optimizer=kind, **hp)
     try:
         if optimiser is not None and optimiser.state_dict()["state"]:
             tr.load_optimiser_state(optimiser.state_dict())
@@ -190,6 +213,36 @@ def train_on_records_cuda(model, rec, epochs=1, batch_size=64, optimiser=None, l
         tr.close()
     model.eval()
     return history
+
+
+def evaluate_records(model, rec, evaluator=EVAL_NET_BF16):
+    """Held-out losses (mse, ce) of `model` on packed records, in eval mode: the library's inference network (`evaluator` EVAL_NET_BF16
+    or EVAL_NET_FP32; BatchNorm with the running statistics; it already holds the weights train_on_records_cuda trained, else the
+    model's are sent to it) gives the logits and values in chunks of the engine's capacity, and the host computes, in float64, the
+    mean of (v - z)^2 and of the cross entropy -sum(pi * log_softmax(logits)) against the CSR policy targets.  Changes no weights,
+    running statistics or trainer state."""
+    import numpy as np
+    from . import runtime
+    n = len(rec["z"])
+    if n == 0:
+        raise ValueError("evaluate_records: no records")
+    eng = runtime.get_engine(min_games=min(n, 1024))                  # grown (and the model's weights re-sent) only when it is smaller
+    runtime.sync_weights(eng, model)
+    chunk = eng.max_games * eng.leaves_per_tree
+    off = np.asarray(rec["pi_off"], dtype=np.int64)
+    se = ce = 0.0
+    for lo in range(0, n, chunk):
+        hi = min(n, lo + chunk)
+        logits, value = eng.net_forward(rec["states"][lo:hi], evaluator, logits=True)
+        lg = logits.astype(np.float64)
+        mx = lg.max(axis=1)
+        lse = mx + np.log(np.exp(lg - mx[:, None]).sum(axis=1))
+        a, b = int(off[lo]), int(off[hi])
+        row = np.repeat(np.arange(hi - lo), np.diff(off[lo:hi + 1]))
+        logp = lg[row, np.asarray(rec["pi_index"][a:b], dtype=np.int64)] - lse[row]
+        ce -= float(np.dot(np.asarray(rec["pi_prob"][a:b], dtype=np.float64), logp))
+        se += float(((value.astype(np.float64) - np.asarray(rec["z"][lo:hi], dtype=np.float64)) ** 2).sum())
+    return se / n, ce / n
 
 
 def train_on_records(model, rec, epochs=1, batch_size=64, optimiser=None, lr_scheduler=None, device=None, seed=0, log=None, backend=None):

@@ -2,12 +2,13 @@
 
     loss = mse_loss(v, z) + cross_entropy(logits, pi)    (train_RL.py:103-113)
     Adam(lr 1e-4, weight_decay 1e-4) (:187), StepLR(500, 0.95) stepped per batch (:199, :123-124)
+    or, optimizer="sgd", the supervised recipe: SGD(lr 0.1, weight_decay 1e-4), StepLR(4000, 0.5) (train_supervised.py:84-92)
 
-`Trainer` owns the library's training state for one model: fp32 master weights, Adam moments, BatchNorm buffers.  Records
-(records.pack_records) are copied to the GPU once; a step sends only the row numbers of its batch.  After training,
+`Trainer` owns the library's training state for one model: fp32 master weights, Adam moments or SGD momentum buffers, BatchNorm
+buffers.  Records (records.pack_records) are copied to the GPU once; a step sends only the row numbers of its batch.  After training,
 `write_back(model)` puts the weights (and running statistics) back into the torch module and `optimiser_state(...)` produces a
-torch.optim.Adam state_dict, so checkpoints stay interchangeable with the torch trainer's.  There is no CPU path: without
-libszb200.so or a GPU the constructor raises."""
+torch.optim.Adam or torch.optim.SGD state_dict, so checkpoints stay interchangeable with the torch trainer's.  There is no CPU path:
+without libszb200.so or a GPU the constructor raises."""
 import ctypes
 
 import numpy as np
@@ -15,6 +16,7 @@ import numpy as np
 from . import _lib
 
 ADAM_DEFAULTS = dict(lr=1e-4, beta1=0.9, beta2=0.999, eps=1e-8, weight_decay=1e-4, lr_step=500, lr_gamma=0.95)
+SGD_DEFAULTS = dict(lr=0.1, weight_decay=1e-4, lr_step=4000, lr_gamma=0.5)          # supervised.make_supervised_optimiser
 
 
 def _names(keys):
@@ -22,15 +24,31 @@ def _names(keys):
 
 
 class Trainer:
-    def __init__(self, engine, model, batch_size=128, step0=0, bn_momentum=0.1, bn_eps=1e-5, _probe=(0, 0), **adam):
+    def __init__(self, engine, model, batch_size=128, step0=0, bn_momentum=0.1, bn_eps=1e-5, _probe=(0, 0), optimizer="adam", momentum=0.0,
+                 dampening=0.0, nesterov=False, **hp):
+        """optimizer "adam" (hp: lr, beta1, beta2, eps, weight_decay, lr_step, lr_gamma; ADAM_DEFAULTS) or "sgd" (hp: lr, weight_decay,
+        lr_step, lr_gamma; SGD_DEFAULTS) with torch.optim.SGD's momentum, dampening and nesterov"""
         import torch
+        if optimizer not in ("adam", "sgd"):
+            raise ValueError("optimizer must be 'adam' or 'sgd', not %r" % (optimizer,))
         self.engine, self.lib, self.batch_size = engine, engine.lib, int(batch_size)
-        hp = dict(ADAM_DEFAULTS)
-        hp.update(adam)
+        self.optimizer = optimizer
+        full = dict(ADAM_DEFAULTS)
+        if optimizer == "sgd":
+            unknown = set(hp) - set(SGD_DEFAULTS)
+            if unknown:
+                raise TypeError("SGD has no hyper-parameter %s" % ", ".join(sorted(unknown)))
+            full.update(SGD_DEFAULTS)
+        full.update(hp)
+        hp = full
         self.hp = hp
+        self.momentum, self.dampening, self.nesterov = float(momentum), float(dampening), bool(nesterov)
+        self._have_buffers = False                   # SGD with momentum: torch's "momentum_buffer" state exists (after a step or a load)
         cfg = _lib.TrainConfig(self.batch_size, hp["lr"], hp["beta1"], hp["beta2"], hp["eps"], hp["weight_decay"], hp["lr_step"], hp["lr_gamma"],
                                bn_momentum, bn_eps, int(step0), int(_probe[0]), int(_probe[1]))
         engine._check(self.lib.szb_train_create(engine._h, ctypes.byref(cfg)))
+        if optimizer == "sgd":
+            engine._check(self.lib.szb_train_set_optimizer(engine._h, _lib.TRAIN_SGD, self.momentum, self.dampening, int(self.nesterov)))
         sd = model.state_dict()
         self.keys = [k for k in sd if not k.endswith("num_batches_tracked")]
         self.param_keys = [k for k, _ in model.named_parameters()]
@@ -108,6 +126,7 @@ class Trainer:
         self.engine._check(self.lib.szb_train_step(self.engine._h, len(rows), rows.ctypes.data_as(ctypes.c_void_p), int(flags),
                                                    ctypes.cast(losses, ctypes.c_void_p) if want_losses else None))
         self.steps_run += 1
+        self._have_buffers = self._have_buffers or not (flags & (_lib.TRAIN_NO_UPDATE | _lib.TRAIN_FORWARD_ONLY))
         return (float(losses[0]), float(losses[1])) if want_losses else None
 
     def loss_history(self, first=0, count=None):
@@ -146,9 +165,12 @@ class Trainer:
         return flat
 
     def optimiser_state(self, model):
-        """a torch.optim.Adam state_dict (per-parameter step / exp_avg / exp_avg_sq, one param group) of the trainer's state"""
+        """a torch.optim.Adam state_dict (per-parameter step / exp_avg / exp_avg_sq, one param group) of the trainer's state, or under
+        SGD a torch.optim.SGD one (per-parameter momentum_buffer when momentum is not 0 and the buffers exist, else an empty state)"""
         import torch
         shapes = {k: tuple(p.shape) for k, p in model.named_parameters()}
+        if self.optimizer == "sgd":
+            return self._sgd_state(shapes)
         m = self.get_tensors(_lib.TRAIN_EXP_AVG)
         v = self.get_tensors(_lib.TRAIN_EXP_AVG_SQ)
         step, hp = self.step_count, self.hp
@@ -160,10 +182,30 @@ class Trainer:
                  "params": list(range(len(self.param_keys)))}
         return {"state": state, "param_groups": [group]}
 
+    def _sgd_state(self, shapes):
+        hp, state = self.hp, {}
+        if self.momentum != 0 and self._have_buffers:
+            buf = self.get_tensors(_lib.TRAIN_MOMENTUM_BUFFER)
+            state = {i: {"momentum_buffer": buf[k].view(shapes[k])} for i, k in enumerate(self.param_keys)}
+        lr = hp["lr"] * hp["lr_gamma"] ** (self.step_count // hp["lr_step"])
+        group = {"lr": lr, "momentum": self.momentum, "dampening": self.dampening, "weight_decay": hp["weight_decay"], "nesterov": self.nesterov,
+                 "maximize": False, "foreach": None, "differentiable": False, "fused": None, "initial_lr": hp["lr"],
+                 "params": list(range(len(self.param_keys)))}
+        return {"state": state, "param_groups": [group]}
+
     def load_optimiser_state(self, opt_state):
-        """continue from a torch.optim.Adam state_dict (moments and step counter)"""
+        """continue from a torch.optim.Adam state_dict (moments and step counter) or, under SGD, a torch.optim.SGD one (momentum
+        buffers; SGD keeps no step counter, the learning rate follows step0 / step_count)"""
         st = opt_state.get("state", {})
         if not st:
+            return
+        if self.optimizer == "sgd":
+            buf = {k: st[i]["momentum_buffer"] for i, k in enumerate(self.param_keys) if st.get(i, {}).get("momentum_buffer") is not None}
+            if buf and self.momentum != 0:
+                if len(buf) != len(self.param_keys):
+                    raise ValueError("the SGD state has momentum buffers for %d of %d parameters" % (len(buf), len(self.param_keys)))
+                self.set_tensors(_lib.TRAIN_MOMENTUM_BUFFER, buf)
+                self._have_buffers = True
             return
         m = {k: st[i]["exp_avg"] for i, k in enumerate(self.param_keys) if i in st}
         v = {k: st[i]["exp_avg_sq"] for i, k in enumerate(self.param_keys) if i in st}
