@@ -181,6 +181,30 @@ int szb_selfplay_ply(szb_ctx *ctx, int32_t num_searches, float c_puct, int32_t l
  * moves do not depend on which rank / shard plays it (train_RL.py:219-239 fans games out to workers). */
 int szb_set_game_id_base(szb_ctx *ctx, uint64_t base);
 
+/* Opt-in AlphaZero exploration for self-play (NOT the reference's rule: every parity statement of this library is about the
+ * default, which is off).  Applies to the szb_search / szb_selfplay_ply calls made after it, until it is changed.
+ *   - Root noise, when dirichlet_alpha > 0 and the search runs with learning != 0: when a search expands its root, the normalised
+ *     priors of the children that survive the zero-prior drop (ascending policy index) become
+ *     fl32((1 - (double)eps) * (double)p + (double)eps * (double)fl32(eta)), eta ~ Dir(alpha) over those children, mixed in double
+ *     without FMA contraction and rounded once (at eps = 1 a root prior is exactly fl32(eta)).  Every other node of such a search
+ *     gets the raw normalised priors: the reference's constant rule (mcts.py:91-96, a one-category Dirichlet) is not applied.
+ *     eta of a child is a function of (seed, global game id = game id base + game, the root position's ply, the child's policy
+ *     index) only: not of the slot, the cohort split, the shard, leaves_per_tree or the other children.
+ *     With learning == 0 or dirichlet_alpha == 0 nothing changes (the constant rule still applies under learning != 0).
+ *   - Sampling horizon, for szb_selfplay_ply(..., sample = 1, ...): moves are sampled proportional to visits (with the same RNG
+ *     key, so the same moves as without the horizon) while the root position's ply < sample_plies, and from then on the arg-max
+ *     (first maximum, lowest index on ties) is played.  0 = sample every ply (sim.py:68).
+ * x == NULL switches everything off.  SZB_ERR_ARG (setting unchanged) for an alpha that is not finite or is negative, an epsilon
+ * outside [0, 1] or sample_plies < 0. */
+typedef struct szb_exploration {
+    float dirichlet_alpha;         /* 0 = off (the reference's rule); AlphaZero chess: 0.3 */
+    float dirichlet_epsilon;       /* in [0, 1]; 0.25 */
+    uint64_t seed;                 /* keys the root noise */
+    int32_t sample_plies;          /* 0 = sample every ply (sim.py:68); k = arg-max from ply k on */
+    int32_t reserved;
+} szb_exploration;
+int szb_set_exploration(szb_ctx *ctx, const szb_exploration *x);
+
 /* ---- counters (SURVEY.md 5: metrics) -------------------------------------------------------------- */
 typedef struct szb_stats {
     uint64_t simulations;          /* iterations of mcts.py:49 executed */

@@ -55,6 +55,11 @@ class TrainConfig(ctypes.Structure):
                 ("probe_lbo", ctypes.c_int32), ("probe_sbo", ctypes.c_int32)]
 
 
+class Exploration(ctypes.Structure):
+    _fields_ = [("dirichlet_alpha", ctypes.c_float), ("dirichlet_epsilon", ctypes.c_float), ("seed", ctypes.c_uint64),
+                ("sample_plies", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
 TRAIN_FORWARD_ONLY, TRAIN_NO_UPDATE = 1, 2
 TRAIN_PARAMS, TRAIN_GRADS, TRAIN_EXP_AVG, TRAIN_EXP_AVG_SQ, TRAIN_ACTIVATIONS, TRAIN_MOMENTUM_BUFFER = 0, 1, 2, 3, 4, 5
 TRAIN_ADAM, TRAIN_SGD = 0, 1
@@ -88,6 +93,7 @@ SIGNATURES = {
                                                                           ctypes.POINTER(_i32), ctypes.POINTER(_i32)]),
     "szb_selfplay_ply": (ctypes.c_int, [_vp, _i32, _f32, _i32, _i32, _u64, _i32, _vp, _vp]),
     "szb_set_game_id_base": (ctypes.c_int, [_vp, _u64]),
+    "szb_set_exploration": (ctypes.c_int, [_vp, ctypes.POINTER(Exploration)]),
     "szb_get_stats": (ctypes.c_int, [_vp, ctypes.POINTER(Stats)]),
     "szb_set_profiling": (ctypes.c_int, [_vp, _i32]),
     "szb_get_phase_times": (ctypes.c_int, [_vp, ctypes.POINTER(PhaseTimes)]),

@@ -7,6 +7,7 @@
 //   evaluator : hash kernel or the network (net.cu)                         (mcts.py:72-75)
 //   k_finish  : warp per tree, mask/normalise/noise, child allocation, backup (mcts.py:77-109, mctsnode.py:39-63)
 // Opt-in multi-leaf mode (szb_config.leaves_per_tree > 1, not the reference's algorithm): k_select_vl / k_finish_vl.
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -684,9 +685,44 @@ __device__ __forceinline__ int count_legal(const uint64_t* mk, int lane) {
 //      are dealt to the lanes in three rounds, a warp scan places each lane's set bits, and ALL prior loads are in flight at once;
 //   2. torch.sum's cascade order over the masked policy (tree.cuh): lane t adds the entries with index = t (mod 32) in ascending
 //      order, closing a 16-step block when the next entry belongs to a later one -- cascade_lane_sparse on the compact list;
-//   3. every lane normalises entries lane, lane + 32, ... and a ballot places the survivors.
-__device__ __forceinline__ int create_children(const Dev& d, const uint64_t* mk, const float* pol, unsigned long long e0, int learning, int lane,
-                                               uint16_t* idx_sh, float* p_sh) {
+//   3. every lane normalises entries lane, lane + 32, ... and a ballot places the survivors;
+//   4. the root of a search with exploration on (PRIOR_ROOT_NOISE) mixes Dirichlet noise into the survivors' priors (root_noise).
+// How the priors of the expanded node are set: the normalised policy (learning == 0, and every non-root node when exploration is
+// on), the reference's constant rule (learning != 0, exploration off), or the normalised policy mixed with the root's noise.
+enum { PRIOR_RAW = 0, PRIOR_CONST = 1, PRIOR_ROOT_NOISE = 2 };
+__device__ __forceinline__ int prior_rule(const Dev& d, int learning, int node) {
+    if (!learning) return PRIOR_RAW;
+    if (!(d.dir_alpha > 0.0f)) return PRIOR_CONST;
+    return node == 0 ? PRIOR_ROOT_NOISE : PRIOR_RAW;
+}
+// The noise key of game g's root: (seed, global game id, the root position's ply).
+__device__ __forceinline__ uint64_t root_noise_key(const Dev& d, int g) {
+    return dir_root_key(d.dir_seed, d.game_id_base + (uint64_t)g, d.pool[(size_t)g * d.pool_stride + d.cur[g]].ply);
+}
+// Priors of the root's `count` children at e0 (ascending policy index) -> fl32((1 - eps) p + eps fl32(eta)), eta ~ Dir(alpha) over
+// them (tree.cuh).  Lane t owns the children t, t + 32, ...; their log-gamma draws wait in e_w (these new edges' value sums, zeroed
+// again at the end) between the passes.  Max and sum are reduced in a fixed order, so its host build (tests/host_harness/exploration.cpp) recomputes eta.
+__device__ __forceinline__ void root_noise(const Dev& d, unsigned long long e0, int count, uint64_t key, int lane) {
+    __syncwarp();                                            // the ballot pass wrote the children from other lanes
+    double mx = -INFINITY;
+    for (int k = lane; k < count; k += 32) {
+        const double l = dir_log_gamma(key, d.e_move[e0 + k], (double)d.dir_alpha);
+        d.e_w[e0 + k] = l;
+        mx = fmax(mx, l);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) mx = fmax(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, off));
+    double part = 0.0;
+    for (int k = lane; k < count; k += 32) part = d_add(part, exp(d_add(d.e_w[e0 + k], -mx)));
+    const double total = dir_combine([&](int t) -> double { return __shfl_sync(0xFFFFFFFFu, part, t); });
+    for (int k = lane; k < count; k += 32) {
+        const double eta = exp(d_add(d.e_w[e0 + k], -mx)) / total;
+        d.e_p[e0 + k] = dir_mix(d.e_p[e0 + k], d2f(eta), d.dir_eps);
+        d.e_w[e0 + k] = 0.0;
+    }
+}
+__device__ __forceinline__ int create_children(const Dev& d, const uint64_t* mk, const float* pol, unsigned long long e0, int rule,
+                                               uint64_t noise_key, int lane, uint16_t* idx_sh, float* p_sh) {
     int n = 0;
 #pragma unroll 1
     for (int w = lane; w < 96; w += 32) {
@@ -732,12 +768,13 @@ __device__ __forceinline__ int create_children(const Dev& d, const uint64_t* mk,
             const unsigned long long at = e0 + (unsigned long long)(count + __popc(ballot & ((1u << lane) - 1)));
             d.e_n[at] = 0;
             d.e_w[at] = 0.0;
-            d.e_p[at] = learning ? noisy_prior(pr) : pr;
+            d.e_p[at] = rule == PRIOR_CONST ? noisy_prior(pr) : pr;
             d.e_move[at] = idx_sh[k];
             d.e_link[at] = link_pack(-1, 0, NO_CHILD);
         }
         count += __popc(ballot);
     }
+    if (rule == PRIOR_ROOT_NOISE) root_noise(d, e0, count, noise_key, lane);
     return count;
 }
 
@@ -794,7 +831,9 @@ __device__ __forceinline__ void finish_block(const Dev& d, int learning, int slo
         if (e0 + (unsigned long long)n_legal > d.edge_cap) {
             if (lane == 0) atomicExch(d.error_flag, SZB_ERR_ARENA);
         } else {
-            count = create_children(d, mk, d.policy + (size_t)slot * N_ACTIONS, e0, learning, lane, idx_sh, p_sh);
+            const int rule = prior_rule(d, learning, node);
+            count = create_children(d, mk, d.policy + (size_t)slot * N_ACTIONS, e0, rule, rule == PRIOR_ROOT_NOISE ? root_noise_key(d, g) : 0ull,
+                                    lane, idx_sh, p_sh);
         }
         if (lane == 0) {
             d.node_edge0[r + node] = (int32_t)e0;
@@ -1042,7 +1081,9 @@ __global__ void __launch_bounds__(32 * MAX_LEAVES) k_finish_vl(Dev d, int learni
         if (e0 + (unsigned long long)n_legal > d.edge_cap) {
             if (lane == 0) atomicExch(d.error_flag, SZB_ERR_ARENA);
         } else {
-            count = create_children(d, mk, d.policy + (size_t)ps * N_ACTIONS, e0, learning, lane, idx_vl[j], p_vl[j]);
+            const int rule = prior_rule(d, learning, node);
+            count = create_children(d, mk, d.policy + (size_t)ps * N_ACTIONS, e0, rule, rule == PRIOR_ROOT_NOISE ? root_noise_key(d, g) : 0ull,
+                                    lane, idx_vl[j], p_vl[j]);
         }
         if (lane == 0) {
             d.node_edge0[r + node] = (int32_t)e0;
@@ -1183,8 +1224,9 @@ __global__ void k_tree_export(Dev d, int g, int max_nodes, int max_edges, int32_
     if (lane == 0) { totals[0] = overflow ? -1 : n_nodes; totals[1] = off; totals[2] = d.root_n[g]; }
 }
 
-// choose a move from the root visit counts (sim.py:68 sampling, or arg-max first-index as in eval.py:92-100)
-__global__ void k_pick(Dev d, uint64_t seed, uint64_t game_id_base, int sample, int32_t* moves) {
+// choose a move from the root visit counts (sim.py:68 sampling, or arg-max first-index as in eval.py:92-100); with sample_plies > 0
+// sampling stops at that ply of the game (szb_exploration)
+__global__ void k_pick(Dev d, uint64_t seed, int sample, int sample_plies, int32_t* moves) {
     const int g = blockIdx.x * blockDim.x + threadIdx.x;
     if (g >= d.n_games) return;
     const size_t r = (size_t)g * d.nodes_per_game;
@@ -1194,8 +1236,8 @@ __global__ void k_pick(Dev d, uint64_t seed, uint64_t game_id_base, int sample, 
     long long total = 0;
     for (int i = 0; i < n; i++) total += d.e_n[e0 + i];
     int pick = 0;
-    if (sample && total > 0) {
-        const uint64_t rnd = mix64(mix64(seed ^ (0x9E3779B97F4A7C15ull * (game_id_base + (uint64_t)g + 1))) + (uint64_t)p.ply);
+    if (sample && (sample_plies == 0 || p.ply < sample_plies) && total > 0) {
+        const uint64_t rnd = mix64(mix64(seed ^ (0x9E3779B97F4A7C15ull * (d.game_id_base + (uint64_t)g + 1))) + (uint64_t)p.ply);
         const long long target = (long long)__umul64hi(rnd, (uint64_t)total);      // uniform in [0, total)
         long long acc = 0;
         for (int i = 0; i < n; i++) { acc += d.e_n[e0 + i]; if (acc > target) { pick = i; break; } }
@@ -1903,7 +1945,7 @@ int szb_selfplay_ply(szb_ctx* ctx, int32_t num_searches, float c_puct, int32_t l
     const int G = d.n_games;
     int32_t* d_active = ctx->d_moves + ctx->cfg.max_games;
     SZB_CUDA(ctx, cudaMemsetAsync(d_active, 0, sizeof(int32_t), ctx->stream));
-    k_pick<<<(G + 127) / 128, 128, 0, ctx->stream>>>(d, seed, ctx->game_id_base, sample, ctx->d_moves);
+    k_pick<<<(G + 127) / 128, 128, 0, ctx->stream>>>(d, seed, sample, ctx->sample_plies, ctx->d_moves);
     k_push_picked<<<(G + 31) / 32, 32, 0, ctx->stream>>>(d, ctx->d_moves, d_active);
     ctx->launches += 2;
     SZB_CUDA(ctx, cudaGetLastError());
@@ -1918,7 +1960,24 @@ int szb_selfplay_ply(szb_ctx* ctx, int32_t num_searches, float c_puct, int32_t l
 int szb_set_game_id_base(szb_ctx* ctx, uint64_t base) {
     if (ctx) cudaSetDevice(ctx->device);       // whichever device the calling thread had current
     if (!ctx) return SZB_ERR_ARG;
-    ctx->game_id_base = base;
+    ctx->d.game_id_base = base;
+    return 0;
+}
+
+int szb_set_exploration(szb_ctx* ctx, const szb_exploration* x) {
+    if (ctx) cudaSetDevice(ctx->device);       // whichever device the calling thread had current
+    if (!ctx) return SZB_ERR_ARG;
+    const szb_exploration off{};
+    const szb_exploration& e = x ? *x : off;
+    if (!std::isfinite(e.dirichlet_alpha) || e.dirichlet_alpha < 0.0f)
+        return fail(ctx, SZB_ERR_ARG, "szb_set_exploration: dirichlet_alpha %g is not a finite value >= 0", (double)e.dirichlet_alpha);
+    if (!(e.dirichlet_epsilon >= 0.0f && e.dirichlet_epsilon <= 1.0f))
+        return fail(ctx, SZB_ERR_ARG, "szb_set_exploration: dirichlet_epsilon %g outside [0, 1]", (double)e.dirichlet_epsilon);
+    if (e.sample_plies < 0) return fail(ctx, SZB_ERR_ARG, "szb_set_exploration: sample_plies %d < 0", e.sample_plies);
+    ctx->d.dir_alpha = e.dirichlet_alpha;
+    ctx->d.dir_eps = e.dirichlet_epsilon;
+    ctx->d.dir_seed = e.seed;
+    ctx->sample_plies = e.sample_plies;
     return 0;
 }
 

@@ -94,6 +94,11 @@ struct Dev {
     unsigned long long* step_trace;  // measurement aid (SZB_STEP_TRACE): %globaltimer stamps of the first tree's warp through k_tree_step, or null
     unsigned long long* gstats;  // [max_games][8] the same counters per game: the step kernels bump their own game's row
                                  // (no same-address atomics on the hot path), k_fold_stats folds the rows into `stats`
+    // ---- keys and opt-in exploration (szb_set_game_id_base, szb_set_exploration) --------------------
+    uint64_t game_id_base;       // global id of game 0 of this context (RNG keys; sharding)
+    float dir_alpha;             // > 0: searches with learning != 0 put Dirichlet(dir_alpha) noise on the root's priors
+    float dir_eps;
+    uint64_t dir_seed;
 };
 
 }  // namespace szb
@@ -125,7 +130,7 @@ struct szb_ctx {
     szb::Trainer* trainer = nullptr;
     // self-play records
     int32_t* d_moves = nullptr;
-    uint64_t game_id_base = 0;                 // global id of game 0 of this context (move-sampling RNG key; sharding)
+    int32_t sample_plies = 0;                  // szb_exploration.sample_plies: sampled moves only while the root's ply is below it
     // profiling
     bool profiling = false;
     std::vector<cudaEvent_t> prof_events;

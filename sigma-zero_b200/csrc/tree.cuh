@@ -3,6 +3,7 @@
 //   puct_score        <- mctsnode.py:33-37  Node.get_ucb as torch (CPU, fp32) evaluates it
 //   cascade_lane/...  <- mcts.py:79         torch.sum over the masked fp32[4672] policy (ATen cascade_sum)
 //   noisy_prior       <- mcts.py:91-96      learning=True: one-category Dirichlet == constant
+//   dir_log_gamma/... <- szb_exploration    opt-in: AlphaZero's Dirichlet noise over the root's children (not the reference's rule)
 //
 // No FMA contraction is allowed anywhere in here: every operation goes through an explicit
 // round-to-nearest intrinsic on the device (and the host harness is built with -ffp-contract=off).
@@ -20,6 +21,8 @@ SZB_HD float f_mul(float a, float b) { return __fmul_rn(a, b); }
 SZB_HD float f_div(float a, float b) { return __fdiv_rn(a, b); }
 SZB_HD float d2f(double a) { return __double2float_rn(a); }
 SZB_HD double d_sqrt(double a) { return __dsqrt_rn(a); }
+SZB_HD double d_add(double a, double b) { return __dadd_rn(a, b); }
+SZB_HD double d_mul(double a, double b) { return __dmul_rn(a, b); }
 #else
 SZB_HD float f_add(float a, float b) { volatile float r = a + b; return r; }
 SZB_HD float f_sub(float a, float b) { volatile float r = a - b; return r; }
@@ -27,6 +30,8 @@ SZB_HD float f_mul(float a, float b) { volatile float r = a * b; return r; }
 SZB_HD float f_div(float a, float b) { volatile float r = a / b; return r; }
 SZB_HD float d2f(double a) { return (float)a; }
 SZB_HD double d_sqrt(double a) { return sqrt(a); }
+SZB_HD double d_add(double a, double b) { volatile double r = a + b; return r; }
+SZB_HD double d_mul(double a, double b) { volatile double r = a * b; return r; }
 #endif
 
 // sqrt(N_parent) as the reference feeds it to torch: math.sqrt in double, then cast to fp32 by the
@@ -122,6 +127,61 @@ SZB_HD float he_policy(uint64_t h, int i) {
 SZB_HD float he_value(uint64_t h) {
     const uint64_t r = mix64(h ^ HE_VALUE_SALT) >> 40;
     return f_sub(f_mul((float)(uint32_t)r, 1.1920928955078125e-07f), 1.0f);      // 2^-23
+}
+
+
+// ---- opt-in root exploration (szb_exploration): AlphaZero's Dirichlet(alpha) noise over the ROOT's children --------------------
+// Keyed, not stateful: a child's draw is a function of (seed, global game id, root ply, the child's policy index) only, so it does
+// not depend on the slot, the cohort split, the shard, leaves_per_tree or which other children the root has.  The stream is
+// separated from k_pick's move-sampling RNG by DIR_SALT; the uniforms of one child come from a splitmix64 sequence (its counter
+// drives the rejection loop).  Arithmetic in double; the engine is built with --fmad=false and its host build with
+// -ffp-contract=off, so host and device agree up to the last bits of the libm functions.
+constexpr uint64_t DIR_SALT = 0x6A09E667F3BCC908ull;
+SZB_HD uint64_t dir_root_key(uint64_t seed, uint64_t game_id, int ply) {
+    return mix64(mix64(seed ^ DIR_SALT ^ (HE_GOLDEN * (game_id + 1))) + (uint64_t)ply);
+}
+struct DirStream {
+    uint64_t state;
+    SZB_HD double uniform() {                              // in (0, 1): 52 random bits + 1/2, exact in double
+        state += HE_GOLDEN;
+        return ((double)(mix64(state) >> 12) + 0.5) * 2.220446049250313080847263336181640625e-16;    // 2^-52
+    }
+    SZB_HD double normal() {                               // Box-Muller, cosine branch
+        const double r = d_sqrt(d_mul(-2.0, log(uniform())));
+        return d_mul(r, cos(d_mul(6.283185307179586, uniform())));
+    }
+};
+// log of a Gamma(alpha, 1) draw for the child with policy index `move`.  alpha >= 1: Marsaglia-Tsang; alpha < 1: the boost
+// log G(alpha) = log G(alpha + 1) + log(U) / alpha, kept in the log domain because U^(1/alpha) underflows for small alpha.
+// The rejection loop accepts with probability > 0.95 per try; after 64 rejected tries (probability < 1e-83) it returns log(d).
+SZB_HD double dir_log_gamma(uint64_t root_key, int move, double alpha) {
+    DirStream s{mix64(root_key + (uint64_t)(move + 1) * HE_GOLDEN)};
+    const double a = alpha < 1.0 ? d_add(alpha, 1.0) : alpha;
+    const double d = d_add(a, -1.0 / 3.0), c = 1.0 / d_sqrt(d_mul(9.0, d));
+    double lg = log(d);
+    for (int tries = 0; tries < 64; tries++) {
+        const double x = s.normal();
+        double v = d_add(1.0, d_mul(c, x));
+        if (v <= 0.0) continue;
+        v = d_mul(d_mul(v, v), v);
+        const double u = s.uniform();
+        const double x2 = d_mul(x, x);
+        if (log(u) < d_add(d_mul(0.5, x2), d_mul(d, d_add(d_add(1.0, -v), log(v))))) { lg = d_add(log(d), log(v)); break; }
+    }
+    if (alpha < 1.0) lg = d_add(lg, log(s.uniform()) / alpha);
+    return lg;
+}
+// eta_i = exp(l_i - max l) / sum_j exp(l_j - max l): the sum in the device's fixed order -- lane t = k mod 32 adds the children k of
+// its lane in ascending k, then the 32 lane sums are added in lane order (dir_combine).
+template <class Lane>
+SZB_HD double dir_combine(Lane lane_value) {
+    double total = 0.0;
+    for (int t = 0; t < 32; t++) total = d_add(total, lane_value(t));
+    return total;
+}
+// the mixed root prior fl32((1 - eps) p + eps fl32(eta)), in double, no contraction, one rounding
+SZB_HD float dir_mix(float p, float eta32, float eps) {
+    return d2f(d_add(d_mul(d_add(1.0, -(double)eps), (double)p), d_mul((double)eps, (double)eta32)));
 }
 
 }  // namespace szb

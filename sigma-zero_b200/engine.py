@@ -228,6 +228,14 @@ class Engine:
         """global id of game 0 (keys the move-sampling RNG so that shards of one job play the same games)"""
         self._check(self.lib.szb_set_game_id_base(self._h, int(base)))
 
+    def set_exploration(self, alpha=0.0, epsilon=0.25, seed=0, sample_plies=0):
+        """Opt-in AlphaZero exploration for the searches and self-play plies that follow (szb_set_exploration): with alpha > 0,
+        searches with learning=True mix Dirichlet(alpha) noise into the root's priors with weight epsilon (keyed by seed, global
+        game id and ply) and give every other node its raw priors; sample_plies > 0 makes selfplay_ply(sample=True) play the
+        arg-max from that ply of the game on.  alpha=0, sample_plies=0: the reference's behaviour."""
+        x = _lib.Exploration(float(alpha), float(epsilon), int(seed) & (2 ** 64 - 1), int(sample_plies), 0)
+        self._check(self.lib.szb_set_exploration(self._h, ctypes.byref(x)))
+
     def set_profiling(self, on=True):
         self._check(self.lib.szb_set_profiling(self._h, int(bool(on))))
 

@@ -1,5 +1,6 @@
 """Process-wide engine management for the drop-in facade: one libszb200 context per GPU, grown on demand,
 with the model's weights pushed to it whenever they change.  Host logic only."""
+import math
 import os
 
 import numpy as np
@@ -35,6 +36,23 @@ def get_engine(min_games=1, min_searches=800, leaves_per_tree=None):
 def leaves_of(args):
     """args['leaves_per_tree'] (an extension of the reference's args dict; default 1 = the reference's search)"""
     return int((args or {}).get('leaves_per_tree', 1))
+
+
+def exploration_of(args):
+    """Engine.set_exploration keywords (alpha, epsilon, sample_plies) from the args-dict extensions 'dirichlet_alpha' (absent = off),
+    'dirichlet_epsilon' (default 0.25) and 'sample_plies' (default 0 = sample every ply).  Raises ValueError on a negative or
+    non-finite alpha, an epsilon outside [0, 1] or a negative sample_plies."""
+    args = args or {}
+    alpha = float(args.get('dirichlet_alpha', 0.0))
+    epsilon = float(args.get('dirichlet_epsilon', 0.25))
+    sample_plies = args.get('sample_plies', 0)
+    if not math.isfinite(alpha) or alpha < 0.0:
+        raise ValueError("dirichlet_alpha must be a finite value >= 0, not %r" % (args.get('dirichlet_alpha'),))
+    if not 0.0 <= epsilon <= 1.0:
+        raise ValueError("dirichlet_epsilon must lie in [0, 1], not %r" % (args.get('dirichlet_epsilon'),))
+    if int(sample_plies) != sample_plies or int(sample_plies) < 0:
+        raise ValueError("sample_plies must be an integer >= 0, not %r" % (sample_plies,))
+    return {"alpha": alpha, "epsilon": epsilon, "sample_plies": int(sample_plies)}
 
 
 def evaluator_of(model):

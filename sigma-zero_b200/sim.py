@@ -20,9 +20,12 @@ def selfplay_batch(model, args, num_games, c960=False, seed=None, start_ids=None
     """Plays num_games games in lock step.  Returns one history dict per game (sim.py:38-43 schema) plus counters.
 
     With a `seed`, everything random about a game -- its Chess960 start position (the reference draws random.randint(0,
-    959), chess_tensor.py:69) and the moves sampled from the visit counts (sim.py:68) -- is a function of (seed, global game
-    id = game_id_base + index) only, so a job sharded over ranks plays exactly the games a single process would."""
+    959), chess_tensor.py:69), the moves sampled from the visit counts (sim.py:68) and the root noise of the opt-in exploration
+    -- is a function of (seed, global game id = game_id_base + index) only, so a job sharded over ranks plays exactly the games
+    a single process would.  args may carry 'dirichlet_alpha', 'dirichlet_epsilon' and 'sample_plies' (runtime.exploration_of);
+    without them the engine's exploration is switched off."""
     n_search = int(args['num_searches'])
+    explore = runtime.exploration_of(args)
     eng = runtime.get_engine(min_games=num_games, min_searches=n_search, leaves_per_tree=runtime.leaves_of(args))
     runtime.sync_weights(eng, model)
     eng.owner = None
@@ -33,6 +36,7 @@ def selfplay_batch(model, args, num_games, c960=False, seed=None, start_ids=None
                      if c960 else np.full(num_games, -1))
     eng.reset(start_ids)
     eng.set_game_id_base(game_id_base)
+    eng.set_exploration(seed=int(seed), **explore)
     seed64 = int(seed)
     games = [_empty_history() for _ in range(num_games)]
     evaluator = runtime.evaluator_of(model)
@@ -81,6 +85,7 @@ def selfplay_records(model, args, num_games, c960=False, seed=None, start_ids=No
     by game, then ply -- exactly records.pack_records(selfplay_batch(...)[0]).  records["result"] holds one outcome code
     per game: 1 white won, -1 black won, 0 draw, 2 unfinished (max_plies)."""
     n_search = int(args['num_searches'])
+    explore = runtime.exploration_of(args)
     eng = runtime.get_engine(min_games=num_games, min_searches=n_search, leaves_per_tree=runtime.leaves_of(args))
     runtime.sync_weights(eng, model)
     eng.owner = None
@@ -91,6 +96,7 @@ def selfplay_records(model, args, num_games, c960=False, seed=None, start_ids=No
                      if c960 else np.full(num_games, -1))
     eng.reset(start_ids)
     eng.set_game_id_base(game_id_base)
+    eng.set_exploration(seed=int(seed), **explore)
     evaluator = runtime.evaluator_of(model)
     col = np.arange(256)[None, :]
     st, gm, pl, ix, pr, ln = [], [], [], [], [], []

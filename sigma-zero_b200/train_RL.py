@@ -357,7 +357,10 @@ def main(args=None, model=None, weights=None, num_games=None, out_dir=".", seed=
     return model, history
 
 
-if __name__ == "__main__":
+def build_parser():
+    """the command line of `python -m sigma_zero_b200.train_RL`: DEFAULT_ARGS as flags plus the run's settings and the opt-in
+    extensions of the args dict (--leaves_per_tree, and --dirichlet_alpha / --dirichlet_epsilon / --sample_plies for AlphaZero's
+    root noise and sampling horizon in self-play; the defaults are the reference's behaviour)"""
     import argparse
     ap = argparse.ArgumentParser(description="self-play + fine-tuning loop of the reference's train_RL.py on the B200 engine "
                                              "(under torchrun the games of an epoch are split over the ranks)")
@@ -368,11 +371,23 @@ if __name__ == "__main__":
     ap.add_argument("--weights", default=None, help="state_dict to start from, e.g. supervised_model_best.pt")
     ap.add_argument("--out_dir", default=".")
     ap.add_argument("--leaves_per_tree", type=int, default=1)
-    ns = vars(ap.parse_args())
+    ap.add_argument("--dirichlet_alpha", type=float, default=0.0,
+                    help="Dirichlet noise on the root's priors in self-play (AlphaZero chess: 0.3); 0 = off, the reference's rule")
+    ap.add_argument("--dirichlet_epsilon", type=float, default=0.25, help="weight of the root noise")
+    ap.add_argument("--sample_plies", type=int, default=0,
+                    help="sample moves from the visit counts for this many plies of a game, then play the arg-max; 0 = sample every ply")
+    return ap
+
+
+CLI_ARGS = list(DEFAULT_ARGS) + ["start_epoch", "leaves_per_tree", "dirichlet_alpha", "dirichlet_epsilon", "sample_plies"]
+
+
+if __name__ == "__main__":
+    ns = vars(build_parser().parse_args())
     if "RANK" in os.environ:
         import torch.distributed as dist
         torch.cuda.set_device(int(os.environ.get("LOCAL_RANK", 0)))
         dist.init_process_group("nccl")
-    cli = {k: ns[k] for k in list(DEFAULT_ARGS) + ["start_epoch", "leaves_per_tree"]}
+    cli = {k: ns[k] for k in CLI_ARGS}
     cli["chess960"] = bool(cli["chess960"])
     main(cli, weights=ns["weights"], num_games=ns["num_games"], out_dir=ns["out_dir"], train_device="cuda")
