@@ -19,19 +19,6 @@ using namespace szb;
 
 struct Args { int n; int count; int dual; int walk; int sbo; long long* out; const uint8_t* src; int copy_bytes; int commit_every; };
 
-__device__ __forceinline__ void mma1(uint32_t d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc, uint32_t acc) {
-    asm volatile("{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\tmov.b64 da, {%1, %2};\n\tmov.b64 db, {%3, %4};\n\tsetp.ne.b32 p, %6, 0;\n\t"
-                 "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t}" ::"r"(d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void mma2(uint32_t d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc, uint32_t acc) {
-    asm volatile("{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\tmov.b64 da, {%1, %2};\n\tmov.b64 db, {%3, %4};\n\tsetp.ne.b32 p, %6, 0;\n\t"
-                 "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %5, p;\n\t}" ::"r"(d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(acc) : "memory");
-}
-
-__device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-
 // cta_group::1, M = 128
 __global__ void __launch_bounds__(128, 1) k_rate1(const Args a) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -47,12 +34,9 @@ __global__ void __launch_bounds__(128, 1) k_rate1(const Args a) {
         mbar_init(smem_u32(&sbar), 1);
         stop_sh = 0;
         copied_sh = 0;
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
-    if (threadIdx.x < 32) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (threadIdx.x < 32) tc_tmem_alloc(smem_u32(&tmem_base_sh), 512);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     tc_fence_before();
     __syncthreads();
@@ -63,13 +47,13 @@ __global__ void __launch_bounds__(128, 1) k_rate1(const Args a) {
         const uint32_t cdst = base + 160 * 1024;
         uint32_t ph[4] = {0, 0, 0, 0};
         long long n = 0;
-        for (int i = 0; i < 4; i++) { mbar_expect_tx(smem_u32(&cbar[i]), a.copy_bytes); bulk_g2s(cdst + i * 16384, a.src + (size_t)i * 16384, a.copy_bytes, smem_u32(&cbar[i])); }
+        for (int i = 0; i < 4; i++) { mbar_expect_tx(smem_u32(&cbar[i]), a.copy_bytes); bulk_load(cdst + i * 16384, a.src + (size_t)i * 16384, a.copy_bytes, smem_u32(&cbar[i])); }
         for (int i = 0; !stop_sh; i = (i + 1) & 3) {
             while (!mbar_try_wait(smem_u32(&cbar[i]), ph[i])) {}
             ph[i] ^= 1;
             n += a.copy_bytes;
             mbar_expect_tx(smem_u32(&cbar[i]), a.copy_bytes);
-            bulk_g2s(cdst + i * 16384, a.src + (size_t)((n >> 14) & 63) * 16384, a.copy_bytes, smem_u32(&cbar[i]));
+            bulk_load(cdst + i * 16384, a.src + (size_t)((n >> 14) & 63) * 16384, a.copy_bytes, smem_u32(&cbar[i]));
         }
         for (int i = 0; i < 4; i++) while (!mbar_try_wait(smem_u32(&cbar[i]), ph[i])) {}
         copied_sh = n;
@@ -83,10 +67,10 @@ __global__ void __launch_bounds__(128, 1) k_rate1(const Args a) {
             const uint32_t st = a.walk ? (uint32_t)((i >> 2) & 3) : 0u;                 // A stages of 32 KB / 4, B stages of 32 KB: 4 each inside 160 KB
             const uint32_t al = a_lo0 + st * (8192 >> 4), bl = b_lo0 + st * (32768 >> 4);
             const uint32_t d1 = tm + (a.dual ? 256u : 0u);
-            mma1(tm, al, hi, bl, hib, idesc, i != 0);
-            mma1(d1, al + 2, hi, bl + 2, hib, idesc, a.dual ? (i != 0) : 1u);
-            mma1(tm, al + 4, hi, bl + 4, hib, idesc, 1u);
-            mma1(d1, al + 6, hi, bl + 6, hib, idesc, 1u);
+            tc1_mma_bf16_split(tm, al, hi, bl, hib, idesc, i != 0);
+            tc1_mma_bf16_split(d1, al + 2, hi, bl + 2, hib, idesc, a.dual ? (i != 0) : 1u);
+            tc1_mma_bf16_split(tm, al + 4, hi, bl + 4, hib, idesc, 1u);
+            tc1_mma_bf16_split(d1, al + 6, hi, bl + 6, hib, idesc, 1u);
             if (a.commit_every && (i + 4) % a.commit_every == 0 && i + 4 < a.count) tc_commit(smem_u32(&sbar));      // a commit per stage, as a pipeline issues them (barrier nobody waits on)
         }
         tc_commit(smem_u32(&bar));
@@ -101,7 +85,7 @@ __global__ void __launch_bounds__(128, 1) k_rate1(const Args a) {
     __syncthreads();
     tc_fence_after();
     if (threadIdx.x == 0) a.out[2] = copied_sh;
-    if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tm), "r"(512) : "memory");
+    if (threadIdx.x < 32) tc_tmem_dealloc(tm, 512);
 }
 
 // cta_group::2, M = 256 (128 rows per CTA), N split between the CTAs
@@ -109,18 +93,14 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128, 1) k_rate2(cons
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bar, sbar;
     __shared__ uint32_t tmem_base_sh;
-    uint32_t rank;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(rank));
+    const uint32_t rank = cluster_ctarank();
     const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     for (uint32_t i = threadIdx.x; i < 160 * 1024 / 4; i += blockDim.x) reinterpret_cast<uint32_t*>(smem_raw)[i] = 0x3c003c00u + (i & 3);
-    if (threadIdx.x == 0) { mbar_init(smem_u32(&bar), 1); mbar_init(smem_u32(&sbar), 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-    if (threadIdx.x < 32) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
+    if (threadIdx.x == 0) { mbar_init(smem_u32(&bar), 1); mbar_init(smem_u32(&sbar), 1); fence_mbarrier_init(); }
+    if (threadIdx.x < 32) tc2_tmem_alloc(smem_u32(&tmem_base_sh), 512);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     tc_fence_before();
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+    cluster_sync_all();
     tc_fence_after();
     const uint32_t tm = tmem_base_sh;
     if (rank == 0 && threadIdx.x == 0) {
@@ -132,12 +112,12 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128, 1) k_rate2(cons
             const uint32_t st = a.walk ? (uint32_t)((i >> 2) & 3) : 0u;
             const uint32_t al = a_lo0 + st * (8192 >> 4), bl = b_lo0 + st * (32768 >> 4);
             const uint32_t d1 = tm + (a.dual ? 256u : 0u);
-            mma2(tm, al, hi, bl, hib, idesc, i != 0);
-            mma2(d1, al + 2, hi, bl + 2, hib, idesc, a.dual ? (i != 0) : 1u);
-            mma2(tm, al + 4, hi, bl + 4, hib, idesc, 1u);
-            mma2(d1, al + 6, hi, bl + 6, hib, idesc, 1u);
+            tc2_mma_bf16_split(tm, al, hi, bl, hib, idesc, i != 0);
+            tc2_mma_bf16_split(d1, al + 2, hi, bl + 2, hib, idesc, a.dual ? (i != 0) : 1u);
+            tc2_mma_bf16_split(tm, al + 4, hi, bl + 4, hib, idesc, 1u);
+            tc2_mma_bf16_split(d1, al + 6, hi, bl + 6, hib, idesc, 1u);
             if (a.commit_every && (i + 4) % a.commit_every == 0 && i + 4 < a.count)        // stage release to BOTH CTAs, as k_tower_tc2 issues it
-                asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(&sbar)), "h"((uint16_t)3) : "memory");
+                tc2_commit(smem_u32(&sbar));
         }
         asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(smem_u32(&bar)), "h"((uint16_t)1) : "memory");
         const long long t1 = clock64();
@@ -147,9 +127,9 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(128, 1) k_rate2(cons
         a.out[1] = t2 - t0;
     }
     tc_fence_before();
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+    cluster_sync_all();
     tc_fence_after();
-    if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tm), "r"(512) : "memory");
+    if (threadIdx.x < 32) tc2_tmem_dealloc(tm, 512);
 }
 
 int main() {

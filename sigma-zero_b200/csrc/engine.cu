@@ -595,7 +595,7 @@ __device__ __forceinline__ bool expand_warp(const Dev& d, const Tables& T, int s
         }
     }
     __syncwarp();                                              // lane 0's shared / global writes -> the other lanes
-    if (tr) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); tr[4] = t; }
+    if (tr) tr[4] = global_ns();
     term = __shfl_sync(0xFFFFFFFFu, term, 0);
     qslot = __shfl_sync(0xFFFFFFFFu, qslot, 0);
     // all lanes: legal moves into shared memory (a terminal node that already exists needs none), then the outcome
@@ -625,7 +625,7 @@ __device__ __forceinline__ bool expand_warp(const Dev& d, const Tables& T, int s
         }
     }
     __syncwarp();
-    if (tr) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); tr[5] = t; }
+    if (tr) tr[5] = global_ns();
     term = __shfl_sync(0xFFFFFFFFu, term, 0);
     if (term) return false;
     for (int k = lane; k < cnt; k += 32) {
@@ -895,7 +895,7 @@ __global__ void __launch_bounds__(32 * FINISH_WARPS) k_tree_step(Dev d, float c_
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     const bool active = slot < d.g_end;
     unsigned long long* tr = (d.step_trace && slot == d.g_begin && lane == 0) ? d.step_trace : nullptr;
-    auto stamp = [&](int k) { if (tr) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); tr[k] = t; } };
+    auto stamp = [&](int k) { if (tr) tr[k] = global_ns(); };
     pdl_trigger();                                             // the tower launch behind me may begin its set-up and weight prefetch
     if (phases & STEP_SELECT) load_tables(&T, d.tables);       // (constant tables: before the wait)
     pdl_wait();                                                // the evaluator's priors / values; its completion counters are idle now

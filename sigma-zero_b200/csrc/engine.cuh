@@ -1,5 +1,6 @@
 // engine.cuh -- context layout shared by engine.cu (games, tree, search, perft) and net.cu (network).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <string>
@@ -154,6 +155,12 @@ namespace szb {
 // anything the predecessor wrote.  Without the attribute both instructions are no-ops.
 __device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+// device time in ns (%globaltimer): the stamps of the measurement aids (SZB_STEP_TRACE, SZB_TOWER_TRACE, SZB_TRAIN_TRACE, ...)
+__device__ __forceinline__ unsigned long long global_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
 template <class... KArgs, class... Args>
 inline cudaError_t launch_kernel(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t stream, bool pdl, Args&&... args) {
     cudaLaunchConfig_t cfg = {};
@@ -181,6 +188,16 @@ void trainer_destroy(szb_ctx* ctx);
 int net_check_error(szb_ctx* ctx);
 // net.cu: fold the recorded conv event pairs into ctx->conv_ms (call after the stream is synchronised)
 void net_collect_conv_times(szb_ctx* ctx);
+// net.cu: bf16 tensor maps with 128-byte swizzle (net.cu and train.cu).  net_tmap_init looks cuTensorMapEncodeTiled up once; a builder
+// that fails reports "cuTensorMapEncodeTiled(<what>) failed".
+int net_tmap_init(szb_ctx* ctx);
+// halo activations [boards][10][10][channels]: box = 64 channels x 8 x 8 x box_boards (the interior of a board's halo tile)
+int net_tmap_act(szb_ctx* ctx, CUtensorMap* tm, void* base, int channels, int boards, int box_boards, const char* what);
+// the same seen as (c, x, board, y): box = 64 channels x 10 x box_boards x 10 -> shared-memory rows [y][board][x], a whole halo chunk
+// (strides need not ascend: probed, scripts/desc_probe.cu)
+int net_tmap_halo(szb_ctx* ctx, CUtensorMap* tm, void* base, int channels, int boards, int box_boards, const char* what);
+// K-major rows [rows][k_total]: box = 64 k x box_rows rows
+int net_tmap_rows(szb_ctx* ctx, CUtensorMap* tm, void* base, int k_total, int rows, int box_rows, const char* what);
 }  // namespace szb
 
 #define SZB_CUDA(ctx, call)                                             \

@@ -114,7 +114,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 static EncodeTiledFn g_encode = nullptr;
 
-static int get_encode(szb_ctx* ctx) {
+int net_tmap_init(szb_ctx* ctx) {
     if (g_encode) return 0;
     void* fn = nullptr;
     cudaDriverEntryPointQueryResult q;
@@ -124,39 +124,31 @@ static int get_encode(szb_ctx* ctx) {
     return 0;
 }
 
-// activations [B][10][10][C] bf16: box = 64 channels x 8 x 8 x 2 boards, 128B swizzle
-static int make_act_map(szb_ctx* ctx, CUtensorMap* tm, void* base, int channels, int boards) {
-    cuuint64_t dims[4] = {(cuuint64_t)channels, HALO, HALO, (cuuint64_t)boards};
-    cuuint64_t strides[3] = {(cuuint64_t)channels * 2, (cuuint64_t)channels * 2 * HALO, (cuuint64_t)channels * 2 * HALO * HALO};
-    cuuint32_t box[4] = {TC_BLOCK_K, 8, 8, 2};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = g_encode(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+static int encode_bf16(szb_ctx* ctx, CUtensorMap* tm, int rank, void* base, const cuuint64_t* dims, const cuuint64_t* strides,
+                       const cuuint32_t* box, const char* what) {
+    const cuuint32_t estr[4] = {1, 1, 1, 1};
+    CUresult r = g_encode(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, (cuuint32_t)rank, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                           CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(activations) failed: %d", (int)r);
+    if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(%s) failed: %d", what, (int)r);
     return 0;
 }
-// activations [B][10][10][C] bf16 seen as (c, x, board, y): box = 64 channels x 10 x 2 boards x 10 -> shared memory rows
-// [y][board][x], the resident halo chunk of k_tower_tc2 (strides need not ascend: probed, scripts/desc_probe.cu)
-static int make_halo_map(szb_ctx* ctx, CUtensorMap* tm, void* base, int channels, int boards) {
-    cuuint64_t dims[4] = {(cuuint64_t)channels, HALO, (cuuint64_t)boards, HALO};
-    cuuint64_t strides[3] = {(cuuint64_t)channels * 2, (cuuint64_t)channels * 2 * HALO * HALO, (cuuint64_t)channels * 2 * HALO};
-    cuuint32_t box[4] = {TC_BLOCK_K, HALO, 2, HALO};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = g_encode(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(halo activations) failed: %d", (int)r);
-    return 0;
+int net_tmap_act(szb_ctx* ctx, CUtensorMap* tm, void* base, int channels, int boards, int box_boards, const char* what) {
+    const cuuint64_t dims[4] = {(cuuint64_t)channels, HALO, HALO, (cuuint64_t)boards};
+    const cuuint64_t strides[3] = {(cuuint64_t)channels * 2, (cuuint64_t)channels * 2 * HALO, (cuuint64_t)channels * 2 * HALO * HALO};
+    const cuuint32_t box[4] = {TC_BLOCK_K, 8, 8, (cuuint32_t)box_boards};
+    return encode_bf16(ctx, tm, 4, base, dims, strides, box, what);
 }
-// weights [cout_pad][K] bf16: box = 64 k x cout_pad rows
-static int make_w_map(szb_ctx* ctx, CUtensorMap* tm, void* base, int k_total, int cout_pad) {
-    cuuint64_t dims[2] = {(cuuint64_t)k_total, (cuuint64_t)cout_pad};
-    cuuint64_t strides[1] = {(cuuint64_t)k_total * 2};
-    cuuint32_t box[2] = {TC_BLOCK_K, (cuuint32_t)cout_pad};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = g_encode(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                          CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(weights) failed: %d", (int)r);
-    return 0;
+int net_tmap_halo(szb_ctx* ctx, CUtensorMap* tm, void* base, int channels, int boards, int box_boards, const char* what) {
+    const cuuint64_t dims[4] = {(cuuint64_t)channels, HALO, (cuuint64_t)boards, HALO};
+    const cuuint64_t strides[3] = {(cuuint64_t)channels * 2, (cuuint64_t)channels * 2 * HALO * HALO, (cuuint64_t)channels * 2 * HALO};
+    const cuuint32_t box[4] = {TC_BLOCK_K, HALO, (cuuint32_t)box_boards, HALO};
+    return encode_bf16(ctx, tm, 4, base, dims, strides, box, what);
+}
+int net_tmap_rows(szb_ctx* ctx, CUtensorMap* tm, void* base, int k_total, int rows, int box_rows, const char* what) {
+    const cuuint64_t dims[2] = {(cuuint64_t)k_total, (cuuint64_t)rows};
+    const cuuint64_t strides[1] = {(cuuint64_t)k_total * 2};
+    const cuuint32_t box[2] = {TC_BLOCK_K, (cuuint32_t)box_rows};
+    return encode_bf16(ctx, tm, 2, base, dims, strides, box, what);
 }
 
 
@@ -182,7 +174,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1)
 k_conv_tc(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_w, const TcArgs a) {
     constexpr int B_BYTES = N_TILE * TC_BLOCK_K * 2;
     constexpr int STAGE_BYTES = TC_A_BYTES + B_BYTES;
-    constexpr uint32_t IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N_TILE >> 3) << 17) | ((uint32_t)(TC_BLOCK_M >> 4) << 24);
+    constexpr uint32_t IDESC = idesc_bf16(TC_BLOCK_M, N_TILE);
     constexpr int ACC_COLS = 256;                                // column stride between the two accumulator stages
 
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -199,13 +191,10 @@ k_conv_tc(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUte
         abort_sh = 0;
         for (int s = 0; s < TC_STAGES; s++) { mbar_init(smem_u32(&bar_full[s]), 1); mbar_init(smem_u32(&bar_empty[s]), 1); }
         for (int s = 0; s < 2; s++) { mbar_init(smem_u32(&bar_acc_full[s]), 1); mbar_init(smem_u32(&bar_acc_empty[s]), 4); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
     for (int i = threadIdx.x; i < N_TILE; i += blockDim.x) bias_sh[i] = a.bias[i];
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 1) tc_tmem_alloc(smem_u32(&tmem_base_sh), 512);
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
@@ -328,9 +317,7 @@ k_conv_tc(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUte
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-    }
+    if (warp == 1) tc_tmem_dealloc(tmem_base, 512);
     if (threadIdx.x == 0 && abort_sh) atomicExch(a.error, 1);
 }
 
@@ -368,7 +355,6 @@ constexpr int T2_BIG_BYTES = 2 * T2_B_BYTES;
 constexpr int T2_SMEM = T2_A_CHUNKS * T2_A_CHUNK_BYTES + T2_B_STAGES * T2_B_BYTES + 1024;
 constexpr int MAX_TOWER_LAYERS = 41;                      // stem + 38 tower convolutions + policy 1x1 + policy output (256 -> 73)
 constexpr int POLICY_LAYER = MAX_TOWER_LAYERS - 1;
-constexpr uint32_t PEER_MASK = 0xFEFFFFFFu;               // shared::cluster address of the same offset in the pair's even CTA
 constexpr int READY_PER_ITEM = 8;                         // 4 epilogue warps x 2 CTAs
 constexpr int SPAN_CAP = 1 << 17;                         // launches recorded by szb_tower_spans_record / SZB_TOWER_SPAN (a c2 bench run: 32,000)
 
@@ -453,79 +439,6 @@ __device__ __forceinline__ TowerItem tower_item(const TowerArgs& a, int item) {
 __device__ __noinline__ float sm_exp(float x, float mx) { return expf(__fsub_rn(x, mx)); }
 __device__ __noinline__ float vh_tanh(float x) { return tanhf(x); }
 
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// 2-CTA TMA loads: data lands in THIS CTA's shared memory, the transaction bytes are counted on the LEADER's barrier
-__device__ __forceinline__ void tma2_load_4d(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1, int c2, int c3) {
-    asm volatile("cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-                 ::"r"(dst), "l"(tm), "r"(bar & PEER_MASK), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-                 : "memory");
-}
-__device__ __forceinline__ void tma2_load_2d(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1) {
-    asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                 ::"r"(dst), "l"(tm), "r"(bar & PEER_MASK), "r"(c0), "r"(c1)
-                 : "memory");
-}
-// MMA completion -> one arrival on the barrier at this offset in BOTH CTAs of the pair
-__device__ __forceinline__ void tc2_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(bar), "h"((uint16_t)3) : "memory");
-}
-__device__ __forceinline__ void tc2_mma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// same, with the two shared-memory descriptors given as (lo, hi) halves
-__device__ __forceinline__ void tc2_mma_bf16_split(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc,
-                                                   uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %2};\n\t"
-        "mov.b64 db, {%3, %4};\n\t"
-        "setp.ne.b32 p, %6, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %5, p;\n\t}"
-        ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_leader(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(bar & PEER_MASK) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_32x32b_x32(uint32_t taddr, uint32_t* v) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]),
-          "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]),
-          "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]),
-          "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ unsigned long long global_ns() {
-    unsigned long long t;
-    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-    return t;
-}
-__device__ __forceinline__ int ld_acquire_gpu(const int32_t* p) {
-    int v;
-    asm volatile("ld.acquire.gpu.global.b32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-
-// descriptor high words of k_tower_tc2's operands: SBO, version 1, SWIZZLE_128B
-constexpr uint32_t T2_A_HI = (uint32_t)(T2_A_SBO >> 4) | (1u << 14) | (2u << 29);
-constexpr uint32_t T2_B_HI = (uint32_t)(1024 >> 4) | (1u << 14) | (2u << 29);
-
 // small-batch MMA issue of one K chunk of a 3x3 layer: nine taps in weight stages of TPS taps (4 + 4 + 1 or 2 + 2 + 2 + 2 + 1),
 // each tap four K = 16 MMAs; straight-line, all descriptor offsets immediates.  Called warp-convergently by the leader's MMA warp.
 template <int TPS>
@@ -544,10 +457,10 @@ __device__ __forceinline__ bool mma_chunk_3x3(uint32_t d_tmem, uint32_t chunk_lo
                 if (tap < 9) {
                     const uint32_t a_lo = chunk_lo + (uint32_t)((tap / 3) * 2 * HALO + tap % 3) * (128 >> 4);     // halo pixel (ky, board 0, kx)
                     const uint32_t b_lo = b_base + u * TILE_LO;
-                    tc2_mma_bf16_split(d_tmem, a_lo, T2_A_HI, b_lo, T2_B_HI, idesc, tap == 0 ? accumulate : 1u);
-                    tc2_mma_bf16_split(d_tmem, a_lo + 2, T2_A_HI, b_lo + 2, T2_B_HI, idesc, 1u);
-                    tc2_mma_bf16_split(d_tmem, a_lo + 4, T2_A_HI, b_lo + 4, T2_B_HI, idesc, 1u);
-                    tc2_mma_bf16_split(d_tmem, a_lo + 6, T2_A_HI, b_lo + 6, T2_B_HI, idesc, 1u);
+                    tc2_mma_bf16_split(d_tmem, a_lo, desc_hi(T2_A_SBO), b_lo, desc_hi(1024), idesc, tap == 0 ? accumulate : 1u);
+                    tc2_mma_bf16_split(d_tmem, a_lo + 2, desc_hi(T2_A_SBO), b_lo + 2, desc_hi(1024), idesc, 1u);
+                    tc2_mma_bf16_split(d_tmem, a_lo + 4, desc_hi(T2_A_SBO), b_lo + 4, desc_hi(1024), idesc, 1u);
+                    tc2_mma_bf16_split(d_tmem, a_lo + 6, desc_hi(T2_A_SBO), b_lo + 6, desc_hi(1024), idesc, 1u);
                 }
             }
             tc2_commit(bar_be0 + bs * 8);
@@ -573,10 +486,10 @@ __device__ __forceinline__ bool mma_chunk_3x3_big(uint32_t d_tmem, uint32_t chun
                 if (tap < 9) {
                     const uint32_t a_lo = chunk_lo + (uint32_t)((tap / 3) * 2 * HALO + tap % 3) * (128 >> 4);
                     const uint32_t b_lo = b_base + u * (T2_B_BYTES >> 4);
-                    tc2_mma_bf16_split(d_tmem, a_lo, T2_A_HI, b_lo, T2_B_HI, idesc, tap == 0 ? accumulate : 1u);
-                    tc2_mma_bf16_split(d_tmem, a_lo + 2, T2_A_HI, b_lo + 2, T2_B_HI, idesc, 1u);
-                    tc2_mma_bf16_split(d_tmem, a_lo + 4, T2_A_HI, b_lo + 4, T2_B_HI, idesc, 1u);
-                    tc2_mma_bf16_split(d_tmem, a_lo + 6, T2_A_HI, b_lo + 6, T2_B_HI, idesc, 1u);
+                    tc2_mma_bf16_split(d_tmem, a_lo, desc_hi(T2_A_SBO), b_lo, desc_hi(1024), idesc, tap == 0 ? accumulate : 1u);
+                    tc2_mma_bf16_split(d_tmem, a_lo + 2, desc_hi(T2_A_SBO), b_lo + 2, desc_hi(1024), idesc, 1u);
+                    tc2_mma_bf16_split(d_tmem, a_lo + 4, desc_hi(T2_A_SBO), b_lo + 4, desc_hi(1024), idesc, 1u);
+                    tc2_mma_bf16_split(d_tmem, a_lo + 6, desc_hi(T2_A_SBO), b_lo + 6, desc_hi(1024), idesc, 1u);
                 }
             }
             tc2_commit(bar_be0 + bs * 8);
@@ -589,7 +502,7 @@ __device__ __forceinline__ bool mma_chunk_3x3_big(uint32_t d_tmem, uint32_t chun
 
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
 k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ TowerArgs a) {
-    constexpr uint32_t IDESC_BASE = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(256 >> 4) << 24);      // M = 256, N per layer
+    constexpr uint32_t IDESC_BASE = idesc_bf16(256, 0);                    // M = 256, N per layer
     constexpr int ACC_COLS = 256;
 
     extern __shared__ __align__(1024) uint8_t smem_raw[];
@@ -620,12 +533,9 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
         for (int s = 0; s < T2_A_CHUNKS; s++) { mbar_init(smem_u32(&bar_a_full[s]), 1); mbar_init(smem_u32(&bar_a_empty[s]), 1); }
         for (int s = 0; s < T2_B_STAGES; s++) { mbar_init(smem_u32(&bar_b_full[s]), 1); mbar_init(smem_u32(&bar_b_empty[s]), 1); }
         for (int s = 0; s < 2; s++) { mbar_init(smem_u32(&bar_acc_full[s]), 1); mbar_init(smem_u32(&bar_acc_empty[s]), READY_PER_ITEM); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
+    if (warp == 1) tc2_tmem_alloc(smem_u32(&tmem_base_sh), 512);
     tc_fence_before();
     cluster_sync_all();                                           // both CTAs' barriers and TMEM exist from here on
     tc_fence_after();
@@ -653,7 +563,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                     if (__any_sync(0xFFFFFFFFu, give_up)) return false;
                 }
             }
-            asm volatile("fence.proxy.async.global;" ::: "memory");     // generic-proxy stores -> this thread's TMA reads
+            fence_proxy_async_global();     // generic-proxy stores -> this thread's TMA reads
             return true;
         };
         if (a.nsplit == 1) {
@@ -774,8 +684,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
         // The whole warp runs the loop convergently (so the compiler keeps descriptors and barrier addresses in uniform
         // registers instead of broadcasting them per MMA); one elected lane issues.
         if (rank == 0) {
-            constexpr uint32_t LO_FLAGS = 1u << 16;                                              // LBO field (unused for swizzled K-major) = 1
-            const uint32_t a_lo0 = ((smem_a >> 4) & 0x3FFFu) | LO_FLAGS, b_lo0 = ((smem_b >> 4) & 0x3FFFu) | LO_FLAGS;
+            const uint32_t a_lo0 = ((smem_a >> 4) & 0x3FFFu) | DESC_LO_FLAGS, b_lo0 = ((smem_b >> 4) & 0x3FFFu) | DESC_LO_FLAGS;
             const uint32_t bar_af0 = smem_u32(&bar_a_full[0]), bar_ae0 = smem_u32(&bar_a_empty[0]);
             const uint32_t bar_bf0 = smem_u32(&bar_b_full[0]), bar_be0 = smem_u32(&bar_b_empty[0]);
             const uint32_t bar_cf0 = smem_u32(&bar_acc_full[0]), bar_ce0 = smem_u32(&bar_acc_empty[0]);
@@ -814,10 +723,10 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                         const uint32_t a_lo = chunk_lo + (uint32_t)(2 * HALO + 1) * (128 >> 4);
                         const uint32_t b_lo = b_lo0 + bs * ((big ? T2_BIG_BYTES : T2_B_BYTES) >> 4);
                         if (elect_one()) {
-                            tc2_mma_bf16_split(d_tmem, a_lo, T2_A_HI, b_lo, T2_B_HI, idesc, accumulate);
-                            tc2_mma_bf16_split(d_tmem, a_lo + 2, T2_A_HI, b_lo + 2, T2_B_HI, idesc, 1u);
-                            tc2_mma_bf16_split(d_tmem, a_lo + 4, T2_A_HI, b_lo + 4, T2_B_HI, idesc, 1u);
-                            tc2_mma_bf16_split(d_tmem, a_lo + 6, T2_A_HI, b_lo + 6, T2_B_HI, idesc, 1u);
+                            tc2_mma_bf16_split(d_tmem, a_lo, desc_hi(T2_A_SBO), b_lo, desc_hi(1024), idesc, accumulate);
+                            tc2_mma_bf16_split(d_tmem, a_lo + 2, desc_hi(T2_A_SBO), b_lo + 2, desc_hi(1024), idesc, 1u);
+                            tc2_mma_bf16_split(d_tmem, a_lo + 4, desc_hi(T2_A_SBO), b_lo + 4, desc_hi(1024), idesc, 1u);
+                            tc2_mma_bf16_split(d_tmem, a_lo + 6, desc_hi(T2_A_SBO), b_lo + 6, desc_hi(1024), idesc, 1u);
                             tc2_commit(bar_be0 + bs * 8);
                         }
                         __syncwarp();
@@ -848,7 +757,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
             const uint32_t acc_phase = (local >> 1) & 1;
             bias_sh[acc][etid] = a.bias[l * C_TOWER + etid];
             bias_sh[acc][etid + 128] = a.bias[l * C_TOWER + etid + 128];
-            asm volatile("bar.sync 1, 128;" ::: "memory");
+            named_bar_sync<1, 128>();
             // accumulator row (TMEM lane) = (oy * 2 + board-in-CTA) * 8 + ox
             const int row = lane_group * 32 + lane;
             const int board = a.board0 + (t * 2 + (int)rank) * 2 + ((row >> 3) & 1);
@@ -909,7 +818,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                 mx = fmaxf(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, 4));
                 mx = fmaxf(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, 16));
                 if ((lane & 0x17) == 0) hd_red[0][rb][lane_group] = mx;
-                asm volatile("bar.sync 1, 128;" ::: "memory");
+                named_bar_sync<1, 128>();
                 mx = fmaxf(fmaxf(hd_red[0][rb][0], hd_red[0][rb][1]), fmaxf(hd_red[0][rb][2], hd_red[0][rb][3]));
                 float ssum = 0.f;
 #pragma unroll 1
@@ -926,7 +835,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                 ssum = __fadd_rn(ssum, __shfl_xor_sync(0xFFFFFFFFu, ssum, 4));
                 ssum = __fadd_rn(ssum, __shfl_xor_sync(0xFFFFFFFFu, ssum, 16));
                 if ((lane & 0x17) == 0) hd_red[1][rb][lane_group] = ssum;           // squares [16 g, 16 g + 16), g = lane_group
-                asm volatile("bar.sync 1, 128;" ::: "memory");
+                named_bar_sync<1, 128>();
                 const float tot = __fadd_rn(__fadd_rn(__fadd_rn(hd_red[1][rb][0], hd_red[1][rb][1]), hd_red[1][rb][2]), hd_red[1][rb][3]);
                 float* prow = a.heads.policy + (size_t)row_slot * N_ACTIONS + sq;
 #pragma unroll 1
@@ -960,7 +869,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                     }
                 }
                 hd_plane[rb][sq] = fmaxf(__fadd_rn(__fadd_rn(__fadd_rn(p4[0], p4[1]), __fadd_rn(p4[2], p4[3])), a.heads.scalars[0]), 0.f);
-                asm volatile("bar.sync 1, 128;" ::: "memory");
+                named_bar_sync<1, 128>();
 #pragma unroll 1
                 for (int k2 = 0; k2 < 4; k2++) {
                     const int bb = k2 >> 1, o = etid + 128 * (k2 & 1);
@@ -972,7 +881,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                     for (int off = 16; off > 0; off >>= 1) h = __fadd_rn(h, __shfl_xor_sync(0xFFFFFFFFu, h, off));
                     if (lane == 0) hd_fc[bb][(k2 & 1) * 4 + (etid >> 5)] = h;
                 }
-                asm volatile("bar.sync 1, 128;" ::: "memory");
+                named_bar_sync<1, 128>();
                 if (etid < 2) {
                     const int brd = cta_board0 + etid;
                     if (brd < a.board0 + a.n_boards && a.heads.need_eval[brd + a.heads.row_delta]) {
@@ -1047,8 +956,8 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                 mbar_arrive_leader(smem_u32(&bar_acc_empty[acc]));            // accumulator stage free again (leader's barrier)
                 // the warp's stores happen-before this lane's release (__syncwarp above; release is cumulative); the reader
                 // orders its TMA (async-proxy) loads after its acquire with fence.proxy.async
-                asm volatile("fence.proxy.async.global;" ::: "memory");
-                asm volatile("red.release.gpu.global.add.s32 [%0], %1;" ::"l"(a.ready + (size_t)l * a.n_pair_tiles + t), "r"(1) : "memory");
+                fence_proxy_async_global();
+                red_release_gpu_add(a.ready + (size_t)l * a.n_pair_tiles + t, 1);
                 if (tracer) a.trace[(size_t)item * 4 + 3] = global_ns();                // outputs stored and released
             }
         }
@@ -1057,9 +966,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
     tc_fence_before();
     cluster_sync_all();
     tc_fence_after();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-    }
+    if (warp == 1) tc2_tmem_dealloc(tmem_base, 512);
     if (threadIdx.x == 0 && abort_sh) atomicExch(a.error, 1);
     if (threadIdx.x == 0 && a.span) {
         if (blockIdx.x == 0) { a.span[2] = (unsigned long long)clock64() - a.span[2]; a.span[3] = global_ns() - a.span[3]; }   // SM clocks per ns inside this launch
@@ -1111,7 +1018,6 @@ template <int CS> struct ClCfg {
 };
 constexpr uint32_t CL_LAYER_BYTES = 64 * C_TOWER * 2;         // a layer's output for one board
 constexpr int CL_MAX_BOARDS = 18;                             // 18 clusters x 8 = 144 of 148 SMs
-constexpr uint32_t CL_A_HI = (uint32_t)(T2_A_SBO >> 4) | (1u << 14) | (2u << 29);      // 8-row groups one halo row (1280 B) apart
 
 // Weight stream of k_tower_cl.  Through a tensor map a 32-row weight tile arrives as 32 separate 128-byte rows (4608 B apart in
 // w16_all) and a CTA ingests only ~44 GB/s that way -- measured: issuing HALF of a layer's MMAs left the layer's MMA phase at
@@ -1145,72 +1051,13 @@ struct ClusterArgs {
     TowerLayer L[MAX_TOWER_LAYERS];
 };
 
-// one contiguous global -> shared bulk copy (no tensor map); the bytes are counted on `bar`
-__device__ __forceinline__ void bulk_load(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t addr, uint32_t rank) {
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(addr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ void st_cluster_v4(uint32_t addr, const uint4& v) {
-    asm volatile("st.shared::cluster.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-// asynchronous 16-byte store into a peer's shared memory; the peer's mbarrier counts the bytes (complete_tx, release.cluster)
-__device__ __forceinline__ void st_async_v4(uint32_t remote_addr, const uint4& v, uint32_t remote_bar) {
-    asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];"
-                 ::"r"(remote_addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w), "r"(remote_bar) : "memory");
-}
-__device__ __forceinline__ void st_cluster_f32(uint32_t addr, float v) {
-    asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t remote_bar) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(remote_bar) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok)
-        : "r"(bar), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-// bounded wait with cluster-scope acquire (the arrivals come from other CTAs after their distributed-shared-memory stores)
-__device__ __forceinline__ bool mbar_wait_cluster(uint32_t bar, uint32_t parity, volatile int* abort_flag) {
-    if (mbar_try_wait_cluster(bar, parity)) return true;
-    const long long t0 = clock64();
-    for (;;) {
-        if (mbar_try_wait_cluster(bar, parity)) return true;
-        if (*abort_flag) return false;
-        if (clock64() - t0 > TC_TIMEOUT_CYCLES) { *abort_flag = 1; return false; }
-    }
-}
-__device__ __forceinline__ void tc1_mma_bf16_split(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc,
-                                                   uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %2};\n\t"
-        "mov.b64 db, {%3, %4};\n\t"
-        "setp.ne.b32 p, %6, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t}"
-        ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// absolute-address 128-byte swizzle (what TMA and tcgen05.mma apply): address bits 4..6 ^= bits 7..9
-__device__ __forceinline__ uint32_t swz128(uint32_t addr) { return addr ^ (((addr >> 7) & 7u) << 4); }
-
 template <int CS>
 __global__ void __cluster_dims__(CS, 1, 1) __launch_bounds__(TC_THREADS, 1)
 k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ ClusterArgs a) {
     constexpr int CL_SIZE = CS, CL_N = ClCfg<CS>::N, CL_B_STAGES = ClCfg<CS>::STAGES, CL_TILE_BYTES = ClCfg<CS>::TILE_BYTES,
                   CL_STAGE_BYTES = ClCfg<CS>::STAGE_BYTES, CL_NP = ClCfg<CS>::NP;
     constexpr size_t CL_W_RANK_ELEMS = CL_W_LAYER_ELEMS / CS;
-    constexpr uint32_t IDESC_M64 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(64 >> 4) << 24);        // bf16 x bf16 -> fp32, M = 64
+    constexpr uint32_t IDESC_M64 = idesc_bf16(64, 0);                     // M = 64, N per layer
 
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bar_b_full[CL_MAX_STAGES], bar_b_empty[CL_MAX_STAGES], bar_acc_full, bar_act[2], bar_in, bar_lg;
@@ -1238,7 +1085,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
         mbar_init(smem_u32(&bar_act[1]), 1);
         mbar_init(smem_u32(&bar_in), 1);
         mbar_init(smem_u32(&bar_lg), 4 * CL_SIZE);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
         mbar_expect_tx(smem_u32(&bar_act[0]), CL_LAYER_BYTES);            // layer 0's and layer 1's outputs
         mbar_expect_tx(smem_u32(&bar_act[1]), CL_LAYER_BYTES);
     }
@@ -1247,11 +1094,8 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
         uint4* z = reinterpret_cast<uint4*>(smem_raw + (smem_act - smem_u32(smem_raw)));
         for (int i = threadIdx.x; i < 2 * CL_BUF_BYTES / 16; i += blockDim.x) z[i] = make_uint4(0, 0, 0, 0);
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(32) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("fence.proxy.async;" ::: "memory");                      // the zeros (generic proxy) -> TMA writes / tensor-core reads
+    if (warp == 1) tc_tmem_alloc(smem_u32(&tmem_base_sh), 32);
+    fence_proxy_async();                      // the zeros (generic proxy) -> TMA writes / tensor-core reads
     tc_fence_before();
     cluster_sync_all();                                                   // every CTA's barriers and zeroed buffers exist from here on
     tc_fence_after();
@@ -1299,8 +1143,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
         }
     } else if (warp == 1) {
         // ===== MMA issuer: warp-convergent loop, one elected lane issues (straight-line taps, see k_tower_tc2) =====
-        constexpr uint32_t LO_FLAGS = 1u << 16;
-        const uint32_t a_lo0 = ((smem_act >> 4) & 0x3FFFu) | LO_FLAGS, b_lo0 = ((smem_b >> 4) & 0x3FFFu) | LO_FLAGS;
+        const uint32_t a_lo0 = ((smem_act >> 4) & 0x3FFFu) | DESC_LO_FLAGS, b_lo0 = ((smem_b >> 4) & 0x3FFFu) | DESC_LO_FLAGS;
         const uint32_t bar_bf0 = smem_u32(&bar_b_full[0]), bar_be0 = smem_u32(&bar_b_empty[0]);
         uint32_t bs = 0, b_phase = 0;
         bool ok = true;
@@ -1315,7 +1158,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
             // re-arm that barrier for the output of layer l + 1 (bytes of it cannot be sent before this CTA has finished layer l)
             if (l >= 1 && l + 1 <= POLICY_LAYER - 1 && elect_one()) mbar_expect_tx(smem_u32(&bar_act[(l - 1) & 1]), CL_LAYER_BYTES);
             __syncwarp();
-            asm volatile("fence.proxy.async;" ::: "memory");                  // peers' generic-proxy stores -> tensor-core reads
+            fence_proxy_async();                  // peers' generic-proxy stores -> tensor-core reads
             tc_fence_after();
             if (a.trace && blockIdx.x == 0 && lane == 0) a.trace[l * 8 + 0] = global_ns();
             const uint32_t buf_lo = a_lo0 + (uint32_t)(l & 1) * (CL_BUF_BYTES >> 4);
@@ -1336,10 +1179,10 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
                             if (t < T) {
                                 const uint32_t a_lo = buf_lo + (uint32_t)kc * (CL_CHUNK_BYTES >> 4) + (uint32_t)((tap / 3) * HALO + tap % 3) * (128 >> 4);   // halo pixel (ky, kx)
                                 const uint32_t b_lo = b_base + u * (CL_TILE_BYTES >> 4);
-                                tc1_mma_bf16_split(tmem_base, a_lo, CL_A_HI, b_lo, T2_B_HI, idesc, t == 0 ? 0u : 1u);
-                                tc1_mma_bf16_split(tmem_base, a_lo + 2, CL_A_HI, b_lo + 2, T2_B_HI, idesc, 1u);
-                                tc1_mma_bf16_split(tmem_base, a_lo + 4, CL_A_HI, b_lo + 4, T2_B_HI, idesc, 1u);
-                                tc1_mma_bf16_split(tmem_base, a_lo + 6, CL_A_HI, b_lo + 6, T2_B_HI, idesc, 1u);
+                                tc1_mma_bf16_split(tmem_base, a_lo, desc_hi(T2_A_SBO), b_lo, desc_hi(1024), idesc, t == 0 ? 0u : 1u);
+                                tc1_mma_bf16_split(tmem_base, a_lo + 2, desc_hi(T2_A_SBO), b_lo + 2, desc_hi(1024), idesc, 1u);
+                                tc1_mma_bf16_split(tmem_base, a_lo + 4, desc_hi(T2_A_SBO), b_lo + 4, desc_hi(1024), idesc, 1u);
+                                tc1_mma_bf16_split(tmem_base, a_lo + 6, desc_hi(T2_A_SBO), b_lo + 6, desc_hi(1024), idesc, 1u);
                             }
                         }
                         tc_commit(bar_be0 + bs * 8);
@@ -1358,10 +1201,10 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
                     for (int kc = 0; kc < C_TOWER / TC_BLOCK_K; kc++) {
                         const uint32_t a_lo = buf_lo + (uint32_t)kc * (CL_CHUNK_BYTES >> 4) + (uint32_t)(HALO + 1) * (128 >> 4);
                         const uint32_t b_lo = b_base + kc * tile_lo;
-                        tc1_mma_bf16_split(tmem_base, a_lo, CL_A_HI, b_lo, T2_B_HI, idesc, kc == 0 ? 0u : 1u);
-                        tc1_mma_bf16_split(tmem_base, a_lo + 2, CL_A_HI, b_lo + 2, T2_B_HI, idesc, 1u);
-                        tc1_mma_bf16_split(tmem_base, a_lo + 4, CL_A_HI, b_lo + 4, T2_B_HI, idesc, 1u);
-                        tc1_mma_bf16_split(tmem_base, a_lo + 6, CL_A_HI, b_lo + 6, T2_B_HI, idesc, 1u);
+                        tc1_mma_bf16_split(tmem_base, a_lo, desc_hi(T2_A_SBO), b_lo, desc_hi(1024), idesc, kc == 0 ? 0u : 1u);
+                        tc1_mma_bf16_split(tmem_base, a_lo + 2, desc_hi(T2_A_SBO), b_lo + 2, desc_hi(1024), idesc, 1u);
+                        tc1_mma_bf16_split(tmem_base, a_lo + 4, desc_hi(T2_A_SBO), b_lo + 4, desc_hi(1024), idesc, 1u);
+                        tc1_mma_bf16_split(tmem_base, a_lo + 6, desc_hi(T2_A_SBO), b_lo + 6, desc_hi(1024), idesc, 1u);
                     }
                     tc_commit(bar_be0 + bs * 8);
                 }
@@ -1390,7 +1233,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
             const TowerLayer L = a.L[l];
             const int n = L.mode == 1 ? CL_NP : CL_N;
             if (etid < n) bias_sh[l & 1][etid] = a.bias[l * C_TOWER + (int)rank * n + etid];
-            asm volatile("bar.sync 1, 128;" ::: "memory");
+            named_bar_sync<1, 128>();
             ok = __all_sync(0xFFFFFFFFu, mbar_wait(smem_u32(&bar_acc_full), (uint32_t)(l & 1), abort_flag));
             if (!ok) break;
             tc_fence_after();
@@ -1480,7 +1323,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
                 for (int off = 1; off < 16; off <<= 1) mx = fmaxf(mx, __shfl_xor_sync(0xFFFFFFFFu, mx, off));
                 if ((lane & 15) == 0) hd_red[0][sq >> 4] = mx;
             }
-            asm volatile("bar.sync 1, 128;" ::: "memory");
+            named_bar_sync<1, 128>();
             mx = fmaxf(fmaxf(hd_red[0][0], hd_red[0][1]), fmaxf(hd_red[0][2], hd_red[0][3]));
             if (etid < 64) {
 #pragma unroll 1
@@ -1489,7 +1332,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
                 for (int off = 1; off < 16; off <<= 1) ssum = __fadd_rn(ssum, __shfl_xor_sync(0xFFFFFFFFu, ssum, off));
                 if ((lane & 15) == 0) hd_red[1][sq >> 4] = ssum;
             }
-            asm volatile("bar.sync 1, 128;" ::: "memory");
+            named_bar_sync<1, 128>();
             const float tot = __fadd_rn(__fadd_rn(__fadd_rn(hd_red[1][0], hd_red[1][1]), hd_red[1][2]), hd_red[1][3]);
             if (want) {
                 // two threads per square: planes of equal parity
@@ -1510,7 +1353,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
             // (complete and visible: this warp's accumulator waits of layers 39 / 40 are ordered after the MMA warp's acquire of it)
             hd_vw[etid] = a.heads.v_w[etid];
             hd_vw[etid + 128] = a.heads.v_w[etid + 128];
-            asm volatile("bar.sync 1, 128;" ::: "memory");
+            named_bar_sync<1, 128>();
             const int sq = etid >> 1, half = etid & 1;
             const uint32_t px = smem_act + CL_BUF_BYTES + (uint32_t)(((sq >> 3) + 1) * HALO + (sq & 7) + 1) * 128;
             float p2[2] = {0.f, 0.f};
@@ -1529,7 +1372,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
             float s = __fadd_rn(p2[0], p2[1]);                               // (p0 + p1) | (p2 + p3)
             s = __fadd_rn(s, __shfl_xor_sync(0xFFFFFFFFu, s, 1));
             if (half == 0) hd_plane[sq] = fmaxf(__fadd_rn(s, a.heads.scalars[0]), 0.f);
-            asm volatile("bar.sync 1, 128;" ::: "memory");
+            named_bar_sync<1, 128>();
 #pragma unroll 1
             for (int k2 = 0; k2 < 2; k2++) {
                 const int o = etid + 128 * k2;
@@ -1541,7 +1384,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
                 for (int off = 16; off > 0; off >>= 1) h = __fadd_rn(h, __shfl_xor_sync(0xFFFFFFFFu, h, off));
                 if (lane == 0) hd_fc[k2 * 4 + (etid >> 5)] = h;
             }
-            asm volatile("bar.sync 1, 128;" ::: "memory");
+            named_bar_sync<1, 128>();
             if (etid == 0 && ok) {
                 const long row_slot = (long)board + a.heads.row_delta;
                 if (a.heads.mask == nullptr || a.heads.need_eval[row_slot]) {
@@ -1557,9 +1400,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
     tc_fence_before();
     cluster_sync_all();
     tc_fence_after();
-    if (warp == 1) {
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(32) : "memory");
-    }
+    if (warp == 1) tc_tmem_dealloc(tmem_base, 32);
     if (threadIdx.x == 0 && abort_sh) atomicExch(a.error, 1);
 }
 
@@ -1821,7 +1662,7 @@ static int alloc_conv(szb_ctx* ctx, Net* net, ConvLayer& L, int cin, int taps, i
     if ((rc = net_alloc(ctx, net, &L.w32, K * cout_pad, false))) return rc;
     if ((rc = net_alloc(ctx, net, &L.bias, (size_t)cout_pad, false))) return rc;
     if ((rc = net_alloc(ctx, net, &L.w16, K * cout_pad, false))) return rc;
-    return make_w_map(ctx, &L.tm_w, L.w16, (int)K, cout_pad);
+    return net_tmap_rows(ctx, &L.tm_w, L.w16, (int)K, cout_pad, cout_pad, "weights");
 }
 static int fold_conv(szb_ctx* ctx, ConvLayer& L, const float* w, int cin_src, const BN* bn, const float* conv_bias) {
     const size_t total = (size_t)L.cout_pad * L.cin * L.taps;
@@ -1864,9 +1705,9 @@ static int net_alloc_activations(szb_ctx* ctx, Net* net) {
     for (int i = 0; i < 3; i++) {
         if ((rc = net_alloc(ctx, net, &net->act16[i], cap * HALO * HALO * C_TOWER))) return rc;
         if ((rc = net_alloc(ctx, net, &net->act32[i], cap * HALO * HALO * C_TOWER))) return rc;
-        if ((rc = make_act_map(ctx, &net->tm_act16[i], net->act16[i], C_TOWER, net->cap))) return rc;
+        if ((rc = net_tmap_act(ctx, &net->tm_act16[i], net->act16[i], C_TOWER, net->cap, 2, "activations"))) return rc;
     }
-    if ((rc = make_act_map(ctx, &net->tm_in16, net->in16, C_IN_PAD, net->cap))) return rc;
+    if ((rc = net_tmap_act(ctx, &net->tm_in16, net->in16, C_IN_PAD, net->cap, 2, "activations"))) return rc;
     if ((rc = net_alloc(ctx, net, &net->logits, cap * N_ACTIONS))) return rc;
     if ((rc = net_alloc(ctx, net, &net->tc_error, 1))) return rc;
     return 0;
@@ -1922,41 +1763,20 @@ static int net_setup_tower(szb_ctx* ctx, Net* net) {
     a.bias = net->bias_all;
     for (int i = 0; i < 3; i++) a.act[i] = net->act16[i];
     a.error = net->tc_error;
-    if ((rc = make_halo_map(ctx, &net->tower_maps->a[0], net->in16, C_IN_PAD, net->cap))) return rc;
+    if ((rc = net_tmap_halo(ctx, &net->tower_maps->a[0], net->in16, C_IN_PAD, net->cap, 2, "halo activations"))) return rc;
     for (int i = 0; i < 3; i++)
-        if ((rc = make_halo_map(ctx, &net->tower_maps->a[1 + i], net->act16[i], C_TOWER, net->cap))) return rc;
+        if ((rc = net_tmap_halo(ctx, &net->tower_maps->a[1 + i], net->act16[i], C_TOWER, net->cap, 2, "halo activations"))) return rc;
+    // one board's halo tile of the input planes (k_tower_cl): box 64 x 10 x 1 x 10
+    if ((rc = net_tmap_halo(ctx, &net->tower_maps->in1, net->in16, C_IN_PAD, net->cap, 1, "single-board input"))) return rc;
     {
-        // one board's halo tile of the input planes (k_tower_cl): dims (c, x, board, y), box 64 x 10 x 1 x 10
-        cuuint64_t dims[4] = {(cuuint64_t)C_IN_PAD, HALO, (cuuint64_t)net->cap, HALO};
-        cuuint64_t strides[3] = {(cuuint64_t)C_IN_PAD * 2, (cuuint64_t)C_IN_PAD * 2 * HALO * HALO, (cuuint64_t)C_IN_PAD * 2 * HALO};
-        cuuint32_t box[4] = {TC_BLOCK_K, HALO, 1, HALO};
-        cuuint32_t estr[4] = {1, 1, 1, 1};
-        CUresult r = g_encode(&net->tower_maps->in1, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, net->in16, dims, strides, box, estr,
-                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(single-board input) failed: %d", (int)r);
-    }
-    {
-        cuuint64_t dims[2] = {(cuuint64_t)KMAX, (cuuint64_t)MAX_TOWER_LAYERS * C_TOWER};
-        cuuint64_t strides[1] = {(cuuint64_t)KMAX * 2};
-        cuuint32_t box[2] = {TC_BLOCK_K, 128};
-        cuuint32_t estr[2] = {1, 1};
-        CUresult r = g_encode(&net->tower_maps->w, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, net->w16_all, dims, strides, box, estr,
-                              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(tower weights) failed: %d", (int)r);
-        box[1] = 64;
-        r = g_encode(&net->tower_maps->w64, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, net->w16_all, dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(policy weights) failed: %d", (int)r);
-        CUtensorMap* small[3] = {&net->tower_maps->w32, &net->tower_maps->w16, &net->tower_maps->w8};
-        for (int i = 0; i < 3; i++) {
-            box[1] = 32u >> i;
-            r = g_encode(small[i], CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, net->w16_all, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                         CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(N-split weights) failed: %d", (int)r);
-        }
+        TowerMaps& m = *net->tower_maps;
+        const int rows = MAX_TOWER_LAYERS * C_TOWER;
+        if ((rc = net_tmap_rows(ctx, &m.w, net->w16_all, KMAX, rows, 128, "tower weights")) ||
+            (rc = net_tmap_rows(ctx, &m.w64, net->w16_all, KMAX, rows, 64, "policy weights")) ||
+            (rc = net_tmap_rows(ctx, &m.w32, net->w16_all, KMAX, rows, 32, "N-split weights")) ||
+            (rc = net_tmap_rows(ctx, &m.w16, net->w16_all, KMAX, rows, 16, "N-split weights")) ||
+            (rc = net_tmap_rows(ctx, &m.w8, net->w16_all, KMAX, rows, 8, "N-split weights")))
+            return rc;
     }
     const char* mode = getenv("SZB_TOWER_MODE");             // measurement aid: 0 single-CTA per layer, 1 pair per layer, 2 one launch
     if (mode && mode[0] >= '0' && mode[0] <= '2') net->tower_mode = mode[0] - '0';
@@ -2421,7 +2241,7 @@ static int net_ensure_allocated(szb_ctx* ctx) {
     const int cap = (ctx->cfg.max_games * ctx->d.K + 1) & ~1;           // one activation row per path slot
     if (ctx->net && ctx->net->cap == cap && ctx->net->allocated) return 0;
     int rc;
-    if ((rc = get_encode(ctx))) return rc;
+    if ((rc = net_tmap_init(ctx))) return rc;
     net_destroy(ctx);
     Net* net = new Net();
     ctx->net = net;
@@ -2435,7 +2255,7 @@ static int net_ensure_allocated(szb_ctx* ctx) {
     if ((rc = alloc_conv(ctx, net, net->p1, 256, 1, 256, 256))) return rc;
     // the fp32 kernel wants cout_pad % 64 == 0, the tcgen05 kernel reads POLICY_PAD rows: pad to 128 and map the first 80
     if ((rc = alloc_conv(ctx, net, net->p2, 256, 1, 73, 128))) return rc;
-    if ((rc = make_w_map(ctx, &net->p2.tm_w, net->p2.w16, 256, POLICY_PAD))) return rc;
+    if ((rc = net_tmap_rows(ctx, &net->p2.tm_w, net->p2.w16, 256, POLICY_PAD, POLICY_PAD, "weights"))) return rc;
     if ((rc = net_alloc(ctx, net, &net->v_w, 256, false)) || (rc = net_alloc(ctx, net, &net->fc1_w, 256 * 64, false)) ||
         (rc = net_alloc(ctx, net, &net->fc1_b, 256, false)) || (rc = net_alloc(ctx, net, &net->fc2_w, 256, false)) ||
         (rc = net_alloc(ctx, net, &net->head_scalars, 2, false)) || (rc = net_alloc(ctx, net, &net->digest, 1)))

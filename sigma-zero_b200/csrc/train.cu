@@ -66,19 +66,6 @@ constexpr int ROWS_RING = 8;
 
 __device__ __forceinline__ int halo_pix(int sq) { return ((sq >> 3) + 1) * TH + (sq & 7) + 1; }
 
-// MN-major operand, 128-byte swizzle: rows of 128 B are 64 consecutive M (or N) elements of ONE k; 8 consecutive k form a 1024 B atom;
-// SBO = distance between 8-k groups, LBO = distance between 64-element MN atoms (cute::UMMA canonical layout ((8,n),(8,k)):((1,LBO),(8,SBO))
-// in 16-byte units).
-__device__ __forceinline__ uint64_t make_smem_desc_mn(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    uint64_t d = 0;
-    d |= (uint64_t)((addr >> 4) & 0x3FFF);
-    d |= (uint64_t)((lbo_bytes >> 4) & 0x3FFF) << 16;
-    d |= (uint64_t)((sbo_bytes >> 4) & 0x3FFF) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
-    return d;
-}
-
 // =================================================================================================
 // forward / dgrad convolution: one 128-square x 128-channel tile per CTA
 // =================================================================================================
@@ -116,47 +103,8 @@ __device__ __forceinline__ float warp_col_sum32(float (&v)[32], int lane) {
     return v[0];
 }
 
-__device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1, uint16_t mask) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4}], [%2], %5;"
-                 ::"r"(dst), "l"(tm), "r"(bar), "r"(c0), "r"(c1), "h"(mask)
-                 : "memory");
-}
-__device__ __forceinline__ void tma_load_4d_mc(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1, int c2, int c3, uint16_t mask) {
-    asm volatile("cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-                 ::"r"(dst), "l"(tm), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "h"(mask)
-                 : "memory");
-}
-// MMA completion -> one arrival on the barrier at this offset in every CTA of the mask
-__device__ __forceinline__ void tc_commit_mc(uint32_t bar, uint16_t mask) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"(mask) : "memory");
-}
-__device__ __forceinline__ uint32_t t_cluster_rank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-__device__ __forceinline__ void t_cluster_sync() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-
-// tcgen05.mma with the 64-bit shared-memory descriptors given as (lo, hi) halves: hi is a constant of the operand's layout, lo = address
-// field, advanced by plain 32-bit adds -- the single issuing thread's instruction stream is what bounds 64-cycle MMAs
-__device__ __forceinline__ void t_mma_split(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %2};\n\t"
-        "mov.b64 db, {%3, %4};\n\t"
-        "setp.ne.b32 p, %6, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %5, p;\n\t}"
-        ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-constexpr uint32_t DESC_LO_FLAGS = 1u << 16;                                                  // LBO field (unused for swizzled K-major) = 1
-constexpr uint32_t DESC_HI_K1024 = (uint32_t)(1024 >> 4) | (1u << 14) | (2u << 29);          // K-major, SBO 1024, version 1, SWIZZLE_128B
-constexpr uint32_t DESC_HI_K1280 = (uint32_t)((TH * 128) >> 4) | (1u << 14) | (2u << 29);    // K-major, 8-row groups one halo row apart
-
 __device__ __forceinline__ void t_stamp(unsigned long long* tr, int k) {
-    if (tr) { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); tr[k] = t; }
+    if (tr) tr[k] = global_ns();
 }
 
 // Epilogue of the training convolutions (the four epilogue warps of a CTA; `tile` = index of this CTA's two boards): TMEM -> registers ->
@@ -174,7 +122,7 @@ __device__ __forceinline__ void tconv_epilogue(const TConvArgs& a, uint32_t tmem
     if (warp == 2 && lane == 0) t_stamp(trace, 5);
     if (ok) {
         tc_fence_after();
-        if (bwd) asm volatile("bar.sync 1, 256;" ::: "memory");
+        if (bwd) named_bar_sync<1, 256>();
         const int m = lane_group * 32 + lane;                          // row (oy * 2 + board) * 8 + ox
         const int board = tile * 2 + ((m >> 3) & 1), sq = (m >> 4) * 8 + (m & 7);
         const bool live = board < a.n_boards;
@@ -258,7 +206,7 @@ __device__ __forceinline__ void tconv_epilogue(const TConvArgs& a, uint32_t tmem
             }
         }
         if (stats) {
-            asm volatile("bar.sync 1, 256;" ::: "memory");
+            named_bar_sync<1, 256>();
             if (tile * 2 < a.n_boards) {
                 const int which = e >> 7, c = e & 127;
                 a.stat_part[((size_t)tile * 2 + which) * a.ldc + nh * 128 + c] = ((st_sh[which][0][c] + st_sh[which][1][c]) + st_sh[which][2][c]) + st_sh[which][3][c];
@@ -279,7 +227,7 @@ __device__ __forceinline__ void tconv_epilogue(const TConvArgs& a, uint32_t tmem
 template <int MODE>
 __global__ void __cluster_dims__(TR_CLUSTER, 1, 1) __launch_bounds__(TC_CONV_THREADS, 1)
 k_tconv(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_w, const TConvArgs a) {
-    constexpr uint32_t IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+    constexpr uint32_t IDESC = idesc_bf16(128, 128);
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bar_af[TR_A_CHUNKS], bar_ae[TR_A_CHUNKS], bar_bf[TR_B_STAGES], bar_be[TR_B_STAGES], bar_acc;
     __shared__ uint32_t tmem_base_sh;
@@ -299,18 +247,15 @@ k_tconv(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtens
         for (int s = 0; s < TR_A_CHUNKS; s++) { mbar_init(smem_u32(&bar_af[s]), 1); mbar_init(smem_u32(&bar_ae[s]), 1); }
         for (int s = 0; s < TR_B_STAGES; s++) { mbar_init(smem_u32(&bar_bf[s]), 1); mbar_init(smem_u32(&bar_be[s]), TR_CLUSTER); }
         mbar_init(smem_u32(&bar_acc), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(TR_DUAL_ACC ? 256 : 128) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 1) tc_tmem_alloc(smem_u32(&tmem_base_sh), TR_DUAL_ACC ? 256 : 128);
     tc_fence_before();
     __syncthreads();
-    t_cluster_sync();                               // every CTA's barriers exist before a peer's multicast or commit can reach them
+    cluster_sync_all();                             // every CTA's barriers exist before a peer's multicast or commit can reach them
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_sh;
-    const uint32_t crank = t_cluster_rank();
+    const uint32_t crank = cluster_ctarank();
     constexpr uint16_t CMASK = (uint16_t)((1u << TR_CLUSTER) - 1);
     if (threadIdx.x == 0) t_stamp(trace, 1);
     pdl_trigger();                                  // programmatic dependent launch: everything above overlapped the predecessor's tail
@@ -369,10 +314,10 @@ k_tconv(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtens
                             const uint32_t a_lo = chunk_lo + (uint32_t)((tap / 3) * 2 * TH + tap % 3) * (128 >> 4);
                             const uint32_t b_lo = b_lo0 + bs * (TR_B_STAGE_BYTES >> 4) + u * (TR_B_BYTES >> 4);
                             const uint32_t first = tap == 0 ? accumulate : 1u;
-                            t_mma_split(tmem_base, a_lo, DESC_HI_K1280, b_lo, DESC_HI_K1024, IDESC, first);
-                            t_mma_split(d1, a_lo + 2, DESC_HI_K1280, b_lo + 2, DESC_HI_K1024, IDESC, TR_DUAL_ACC ? first : 1u);
-                            t_mma_split(tmem_base, a_lo + 4, DESC_HI_K1280, b_lo + 4, DESC_HI_K1024, IDESC, 1u);
-                            t_mma_split(d1, a_lo + 6, DESC_HI_K1280, b_lo + 6, DESC_HI_K1024, IDESC, 1u);
+                            tc1_mma_bf16_split(tmem_base, a_lo, desc_hi(TH * 128), b_lo, desc_hi(1024), IDESC, first);
+                            tc1_mma_bf16_split(d1, a_lo + 2, desc_hi(TH * 128), b_lo + 2, desc_hi(1024), IDESC, TR_DUAL_ACC ? first : 1u);
+                            tc1_mma_bf16_split(tmem_base, a_lo + 4, desc_hi(TH * 128), b_lo + 4, desc_hi(1024), IDESC, 1u);
+                            tc1_mma_bf16_split(d1, a_lo + 6, desc_hi(TH * 128), b_lo + 6, desc_hi(1024), IDESC, 1u);
                         }
                         tc_commit_mc(bar_be0 + bs * 8, CMASK);
                     }
@@ -386,10 +331,10 @@ k_tconv(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtens
                     const uint32_t a_lo = chunk_lo + (uint32_t)(2 * TH + 1) * (128 >> 4);            // centre tap
                     const uint32_t b_lo = b_lo0 + bs * (TR_B_STAGE_BYTES >> 4);
                     const uint32_t d1 = tmem_base + (TR_DUAL_ACC ? 128u : 0u);
-                    t_mma_split(tmem_base, a_lo, DESC_HI_K1280, b_lo, DESC_HI_K1024, IDESC, accumulate);
-                    t_mma_split(d1, a_lo + 2, DESC_HI_K1280, b_lo + 2, DESC_HI_K1024, IDESC, TR_DUAL_ACC ? accumulate : 1u);
-                    t_mma_split(tmem_base, a_lo + 4, DESC_HI_K1280, b_lo + 4, DESC_HI_K1024, IDESC, 1u);
-                    t_mma_split(d1, a_lo + 6, DESC_HI_K1280, b_lo + 6, DESC_HI_K1024, IDESC, 1u);
+                    tc1_mma_bf16_split(tmem_base, a_lo, desc_hi(TH * 128), b_lo, desc_hi(1024), IDESC, accumulate);
+                    tc1_mma_bf16_split(d1, a_lo + 2, desc_hi(TH * 128), b_lo + 2, desc_hi(1024), IDESC, TR_DUAL_ACC ? accumulate : 1u);
+                    tc1_mma_bf16_split(tmem_base, a_lo + 4, desc_hi(TH * 128), b_lo + 4, desc_hi(1024), IDESC, 1u);
+                    tc1_mma_bf16_split(d1, a_lo + 6, desc_hi(TH * 128), b_lo + 6, desc_hi(1024), IDESC, 1u);
                     tc_commit_mc(bar_be0 + bs * 8, CMASK);
                 }
                 __syncwarp();
@@ -408,8 +353,8 @@ k_tconv(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtens
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(TR_DUAL_ACC ? 256 : 128) : "memory");
-    t_cluster_sync();                               // no CTA leaves while a peer's commit may still arrive on its barriers
+    if (warp == 1) tc_tmem_dealloc(tmem_base, TR_DUAL_ACC ? 256 : 128);
+    cluster_sync_all();                             // no CTA leaves while a peer's commit may still arrive on its barriers
     if (threadIdx.x == 0) t_stamp(trace, 6);
     if (threadIdx.x == 0 && abort_sh) atomicExch(a.error, 1);
 }
@@ -422,40 +367,15 @@ k_tconv(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtens
 // loop at 128 boards), which rules shared-memory operand bandwidth out as the bound of the 64-cycle MMAs (DESIGN 3.5).  Barriers live on the
 // leader for "data landed" (both CTAs' TMA bytes are counted there) and in both CTAs for "stage free" / "accumulator ready" (the leader's
 // commits are multicast) -- the protocol of k_tower_tc2 (net.cu).
-constexpr uint32_t T2_PEER_MASK = 0xFEFFFFFFu;        // shared::cluster address of the same offset in the pair's even CTA
 constexpr int TP_B_STAGES = 6;
 constexpr int TP_B_BYTES = 64 * 64 * 2;               // this CTA's half of a 128-channel x 64-k weight tile
 constexpr int TP_B_STAGE_BYTES = TR_TPS * TP_B_BYTES;
 constexpr int TP_SMEM = TR_A_CHUNKS * TR_A_CHUNK_BYTES + TP_B_STAGES * TP_B_STAGE_BYTES + 1024;
 
-__device__ __forceinline__ void tp_tma_4d(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1, int c2, int c3) {
-    asm volatile("cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
-                 ::"r"(dst), "l"(tm), "r"(bar & T2_PEER_MASK), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-                 : "memory");
-}
-__device__ __forceinline__ void tp_tma_2d(uint32_t dst, const CUtensorMap* tm, uint32_t bar, int c0, int c1) {
-    asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                 ::"r"(dst), "l"(tm), "r"(bar & T2_PEER_MASK), "r"(c0), "r"(c1)
-                 : "memory");
-}
-__device__ __forceinline__ void tp_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(bar), "h"((uint16_t)3) : "memory");
-}
-__device__ __forceinline__ void tp_mma_split(uint32_t tmem_d, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t b_hi, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-        "mov.b64 da, {%1, %2};\n\t"
-        "mov.b64 db, {%3, %4};\n\t"
-        "setp.ne.b32 p, %6, 0;\n\t"
-        "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %5, p;\n\t}"
-        ::"r"(tmem_d), "r"(a_lo), "r"(a_hi), "r"(b_lo), "r"(b_hi), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-
 template <int MODE>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_CONV_THREADS, 1)
 k_tconv_pair(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_w, const TConvArgs a) {
-    constexpr uint32_t IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(128 >> 3) << 17) | ((uint32_t)(256 >> 4) << 24);      // M 256, N 128
+    constexpr uint32_t IDESC = idesc_bf16(256, 128);
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bar_af[TR_A_CHUNKS], bar_ae[TR_A_CHUNKS], bar_bf[TP_B_STAGES], bar_be[TP_B_STAGES], bar_acc;
     __shared__ uint32_t tmem_base_sh;
@@ -465,7 +385,7 @@ k_tconv_pair(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ C
     const uint32_t smem_a = (smem_u32(smem_raw) + 1023u) & ~1023u;
     const uint32_t smem_b = smem_a + TR_A_CHUNKS * TR_A_CHUNK_BYTES;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const uint32_t rank = t_cluster_rank();
+    const uint32_t rank = cluster_ctarank();
     const int tile = blockIdx.x, nh = blockIdx.y;          // tile = this CTA's two boards; the pair = tiles (2p, 2p + 1)
     volatile int* abort_flag = &abort_sh;
     unsigned long long* trace = (blockIdx.x == 0 && blockIdx.y == 0) ? a.trace : nullptr;
@@ -476,15 +396,12 @@ k_tconv_pair(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ C
         for (int s = 0; s < TR_A_CHUNKS; s++) { mbar_init(smem_u32(&bar_af[s]), 1); mbar_init(smem_u32(&bar_ae[s]), 1); }
         for (int s = 0; s < TP_B_STAGES; s++) { mbar_init(smem_u32(&bar_bf[s]), 1); mbar_init(smem_u32(&bar_be[s]), 1); }
         mbar_init(smem_u32(&bar_acc), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(128) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    }
+    if (warp == 1) tc2_tmem_alloc(smem_u32(&tmem_base_sh), 128);
     tc_fence_before();
     __syncthreads();
-    t_cluster_sync();                               // both CTAs' barriers and TMEM exist from here on
+    cluster_sync_all();                             // both CTAs' barriers and TMEM exist from here on
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_sh;
     if (threadIdx.x == 0) t_stamp(trace, 1);
@@ -501,7 +418,7 @@ k_tconv_pair(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ C
                 if (!(ok = mbar_wait(smem_u32(&bar_ae[ac]), a_phase ^ 1, abort_flag))) break;
                 const uint32_t af = smem_u32(&bar_af[ac]);
                 if (rank == 0) mbar_expect_tx(af, 2u * TR_A_CHUNK_BYTES);      // both CTAs' bytes land on the leader's barrier
-                tp_tma_4d(smem_a + ac * TR_A_CHUNK_BYTES, &tm_a, af, kc * 64, 0, tile * 2, 0);
+                tma2_load_4d(smem_a + ac * TR_A_CHUNK_BYTES, &tm_a, af, kc * 64, 0, tile * 2, 0);
                 if (++ac == TR_A_CHUNKS) { ac = 0; a_phase ^= 1; }
                 const int per = a.taps == 9 ? TR_TPS : 1;
                 for (int tap0 = 0; tap0 < a.taps; tap0 += per) {
@@ -509,7 +426,7 @@ k_tconv_pair(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ C
                     const uint32_t bf = smem_u32(&bar_bf[bs]);
                     if (rank == 0) mbar_expect_tx(bf, 2u * (uint32_t)per * TP_B_BYTES);
                     for (int u = 0; u < per; u++)
-                        tp_tma_2d(smem_b + bs * TP_B_STAGE_BYTES + u * TP_B_BYTES, &tm_w, bf, ((tap0 + u) * a.kchunks + kc) * 64, nh * 128 + (int)rank * 64);
+                        tma2_load_2d(smem_b + bs * TP_B_STAGE_BYTES + u * TP_B_BYTES, &tm_w, bf, ((tap0 + u) * a.kchunks + kc) * 64, nh * 128 + (int)rank * 64);
                     if (++bs == TP_B_STAGES) { bs = 0; b_phase ^= 1; }
                 }
             }
@@ -536,12 +453,12 @@ k_tconv_pair(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ C
                                 const int tap = s0 + u;
                                 const uint32_t a_lo = chunk_lo + (uint32_t)((tap / 3) * 2 * TH + tap % 3) * (128 >> 4);
                                 const uint32_t b_lo = b_lo0 + bs * (TP_B_STAGE_BYTES >> 4) + u * (TP_B_BYTES >> 4);
-                                tp_mma_split(tmem_base, a_lo, DESC_HI_K1280, b_lo, DESC_HI_K1024, IDESC, tap == 0 ? accumulate : 1u);
-                                tp_mma_split(tmem_base, a_lo + 2, DESC_HI_K1280, b_lo + 2, DESC_HI_K1024, IDESC, 1u);
-                                tp_mma_split(tmem_base, a_lo + 4, DESC_HI_K1280, b_lo + 4, DESC_HI_K1024, IDESC, 1u);
-                                tp_mma_split(tmem_base, a_lo + 6, DESC_HI_K1280, b_lo + 6, DESC_HI_K1024, IDESC, 1u);
+                                tc2_mma_bf16_split(tmem_base, a_lo, desc_hi(TH * 128), b_lo, desc_hi(1024), IDESC, tap == 0 ? accumulate : 1u);
+                                tc2_mma_bf16_split(tmem_base, a_lo + 2, desc_hi(TH * 128), b_lo + 2, desc_hi(1024), IDESC, 1u);
+                                tc2_mma_bf16_split(tmem_base, a_lo + 4, desc_hi(TH * 128), b_lo + 4, desc_hi(1024), IDESC, 1u);
+                                tc2_mma_bf16_split(tmem_base, a_lo + 6, desc_hi(TH * 128), b_lo + 6, desc_hi(1024), IDESC, 1u);
                             }
-                            tp_commit(bar_be0 + bs * 8);
+                            tc2_commit(bar_be0 + bs * 8);
                         }
                         __syncwarp();
                         if (++bs == TP_B_STAGES) { bs = 0; b_phase ^= 1; }
@@ -552,30 +469,30 @@ k_tconv_pair(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ C
                     if (elect_one()) {
                         const uint32_t a_lo = chunk_lo + (uint32_t)(2 * TH + 1) * (128 >> 4);
                         const uint32_t b_lo = b_lo0 + bs * (TP_B_STAGE_BYTES >> 4);
-                        tp_mma_split(tmem_base, a_lo, DESC_HI_K1280, b_lo, DESC_HI_K1024, IDESC, accumulate);
-                        tp_mma_split(tmem_base, a_lo + 2, DESC_HI_K1280, b_lo + 2, DESC_HI_K1024, IDESC, 1u);
-                        tp_mma_split(tmem_base, a_lo + 4, DESC_HI_K1280, b_lo + 4, DESC_HI_K1024, IDESC, 1u);
-                        tp_mma_split(tmem_base, a_lo + 6, DESC_HI_K1280, b_lo + 6, DESC_HI_K1024, IDESC, 1u);
-                        tp_commit(bar_be0 + bs * 8);
+                        tc2_mma_bf16_split(tmem_base, a_lo, desc_hi(TH * 128), b_lo, desc_hi(1024), IDESC, accumulate);
+                        tc2_mma_bf16_split(tmem_base, a_lo + 2, desc_hi(TH * 128), b_lo + 2, desc_hi(1024), IDESC, 1u);
+                        tc2_mma_bf16_split(tmem_base, a_lo + 4, desc_hi(TH * 128), b_lo + 4, desc_hi(1024), IDESC, 1u);
+                        tc2_mma_bf16_split(tmem_base, a_lo + 6, desc_hi(TH * 128), b_lo + 6, desc_hi(1024), IDESC, 1u);
+                        tc2_commit(bar_be0 + bs * 8);
                     }
                     __syncwarp();
                     if (++bs == TP_B_STAGES) { bs = 0; b_phase ^= 1; }
                 }
                 accumulate = 1;
-                if (ok && elect_one()) tp_commit(bar_ae0 + ac * 8);
+                if (ok && elect_one()) tc2_commit(bar_ae0 + ac * 8);
                 __syncwarp();
                 if (++ac == TR_A_CHUNKS) { ac = 0; a_phase ^= 1; }
             }
-            if (ok && elect_one()) { tp_commit(smem_u32(&bar_acc)); t_stamp(trace, 4); }
+            if (ok && elect_one()) { tc2_commit(smem_u32(&bar_acc)); t_stamp(trace, 4); }
             __syncwarp();
         }
     } else {
         tconv_epilogue<MODE>(a, tmem_base, tile, nh, warp, lane, smem_u32(&bar_acc), abort_flag, st_sh, mi_sh, trace);
     }
     tc_fence_before();
-    t_cluster_sync();
+    cluster_sync_all();
     tc_fence_after();
-    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(128) : "memory");
+    if (warp == 1) tc2_tmem_dealloc(tmem_base, 128);
     if (threadIdx.x == 0) t_stamp(trace, 6);
     if (threadIdx.x == 0 && abort_sh) atomicExch(a.error, 1);
 }
@@ -614,7 +531,7 @@ k_wgrad(const WgLayer* __restrict__ layers, const WgArgs a) {
     const CUtensorMap* tm_x = &wl->tm_x;
     constexpr int N = NB * 64;
     constexpr int STAGE = (2 + NB) * WG_BOX;
-    constexpr uint32_t IDESC = (1u << 4) | (1u << 7) | (1u << 10) | (1u << 15) | (1u << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+    constexpr uint32_t IDESC = idesc_bf16(128, N, true, true);          // both operands MN-major
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bar_full[WG_STAGES], bar_empty[WG_STAGES], bar_acc;
     __shared__ uint32_t tmem_base_sh;
@@ -632,18 +549,15 @@ k_wgrad(const WgLayer* __restrict__ layers, const WgArgs a) {
         abort_sh = 0;
         for (int s = 0; s < WG_STAGES; s++) { mbar_init(smem_u32(&bar_full[s]), 1); mbar_init(smem_u32(&bar_empty[s]), CS); }
         mbar_init(smem_u32(&bar_acc), 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_mbarrier_init();
     }
-    if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_base_sh)), "r"(256) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    if (warp == 1) tc_tmem_alloc(smem_u32(&tmem_base_sh), 256);
     tc_fence_before();
     __syncthreads();
-    if (CS > 1) t_cluster_sync();                  // the peer's barriers exist before a multicast or a commit can reach them
+    if (CS > 1) cluster_sync_all();                // the peer's barriers exist before a multicast or a commit can reach them
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_sh;
-    const uint32_t crank = CS > 1 ? t_cluster_rank() : 0u;
+    const uint32_t crank = CS > 1 ? cluster_ctarank() : 0u;
     constexpr uint16_t CMASK = (uint16_t)((1u << CS) - 1);
     pdl_trigger();
     pdl_wait();
@@ -669,7 +583,7 @@ k_wgrad(const WgLayer* __restrict__ layers, const WgArgs a) {
         }
     } else if (warp == 1) {
         // warp-convergent loop, one elected lane issues; descriptors as (lo, hi) halves advanced with 32-bit adds (see k_tconv)
-        const uint32_t lo_flags = ((a.lbo >> 4) & 0x3FFFu) << 16, hi = ((a.sbo >> 4) & 0x3FFFu) | (1u << 14) | (2u << 29);
+        const uint32_t lo_flags = ((a.lbo >> 4) & 0x3FFFu) << 16, hi = desc_hi(a.sbo);
         const uint32_t s_lo0 = ((smem_base >> 4) & 0x3FFFu) | lo_flags;
         const uint32_t bar_f0 = smem_u32(&bar_full[0]), bar_e0 = smem_u32(&bar_empty[0]);
         uint32_t stage = 0, phase = 0, accumulate = 0;
@@ -679,10 +593,10 @@ k_wgrad(const WgLayer* __restrict__ layers, const WgArgs a) {
             tc_fence_after();
             if (elect_one()) {
                 const uint32_t a_lo = s_lo0 + stage * (STAGE >> 4), b_lo2 = a_lo + ((2 * WG_BOX) >> 4);
-                t_mma_split(tmem_base, a_lo, hi, b_lo2, hi, IDESC, accumulate);
-                t_mma_split(tmem_base, a_lo + 128, hi, b_lo2 + 128, hi, IDESC, 1u);
-                t_mma_split(tmem_base, a_lo + 256, hi, b_lo2 + 256, hi, IDESC, 1u);
-                t_mma_split(tmem_base, a_lo + 384, hi, b_lo2 + 384, hi, IDESC, 1u);
+                tc1_mma_bf16_split(tmem_base, a_lo, hi, b_lo2, hi, IDESC, accumulate);
+                tc1_mma_bf16_split(tmem_base, a_lo + 128, hi, b_lo2 + 128, hi, IDESC, 1u);
+                tc1_mma_bf16_split(tmem_base, a_lo + 256, hi, b_lo2 + 256, hi, IDESC, 1u);
+                tc1_mma_bf16_split(tmem_base, a_lo + 384, hi, b_lo2 + 384, hi, IDESC, 1u);
                 if (CS > 1) tc_commit_mc(bar_e0 + stage * 8, CMASK); else tc_commit(bar_e0 + stage * 8);
             }
             __syncwarp();
@@ -715,8 +629,8 @@ k_wgrad(const WgLayer* __restrict__ layers, const WgArgs a) {
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
-    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(256) : "memory");
-    if (CS > 1) t_cluster_sync();                  // no CTA leaves while the peer's commit may still arrive on its barriers
+    if (warp == 1) tc_tmem_dealloc(tmem_base, 256);
+    if (CS > 1) cluster_sync_all();                // no CTA leaves while the peer's commit may still arrive on its barriers
     if (threadIdx.x == 0 && abort_sh) atomicExch(a.error, 1);
 }
 
@@ -1336,53 +1250,6 @@ struct Trainer {
     std::vector<void*> allocs;
 };
 
-typedef CUresult (*EncodeTiledFnT)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                                   const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static EncodeTiledFnT t_encode = nullptr;
-
-static int t_get_encode(szb_ctx* ctx) {
-    if (t_encode) return 0;
-    void* fn = nullptr;
-    cudaDriverEntryPointQueryResult q;
-    cudaError_t e = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &q);
-    if (e != cudaSuccess || q != cudaDriverEntryPointSuccess || !fn) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled unavailable");
-    t_encode = (EncodeTiledFnT)fn;
-    return 0;
-}
-// halo activations [B][10][10][C]: box = 64 channels x 8 x 8 x `boards`
-static int t_act_map(szb_ctx* ctx, CUtensorMap* tm, void* base, int channels, int cap, int boards) {
-    cuuint64_t dims[4] = {(cuuint64_t)channels, TH, TH, (cuuint64_t)cap};
-    cuuint64_t strides[3] = {(cuuint64_t)channels * 2, (cuuint64_t)channels * 2 * TH, (cuuint64_t)channels * 2 * TPIX};
-    cuuint32_t box[4] = {64, 8, 8, (cuuint32_t)boards};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = t_encode(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                          CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(training activations) failed: %d", (int)r);
-    return 0;
-}
-// halo activations seen as (c, x, board, y): box = 64 channels x 10 x 2 boards x 10 -> shared-memory rows [y][board][x] (k_tconv's chunk)
-static int t_halo_map(szb_ctx* ctx, CUtensorMap* tm, void* base, int channels, int cap) {
-    cuuint64_t dims[4] = {(cuuint64_t)channels, TH, (cuuint64_t)cap, TH};
-    cuuint64_t strides[3] = {(cuuint64_t)channels * 2, (cuuint64_t)channels * 2 * TPIX, (cuuint64_t)channels * 2 * TH};
-    cuuint32_t box[4] = {64, TH, 2, TH};
-    cuuint32_t estr[4] = {1, 1, 1, 1};
-    CUresult r = t_encode(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                          CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(training halo activations) failed: %d", (int)r);
-    return 0;
-}
-// weight pack [rows][k]: box = 64 k x 32 rows (a quarter of k_tconv's 128-row tile: one CTA's share of the multicast)
-static int t_w_map(szb_ctx* ctx, CUtensorMap* tm, void* base, int k_total, int rows, int box_rows) {
-    cuuint64_t dims[2] = {(cuuint64_t)k_total, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)k_total * 2};
-    cuuint32_t box[2] = {64, (cuuint32_t)box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = t_encode(tm, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, base, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                          CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(ctx, SZB_ERR_CUDA, "cuTensorMapEncodeTiled(training weights) failed: %d", (int)r);
-    return 0;
-}
-
 template <class T>
 static int t_alloc(szb_ctx* ctx, Trainer* tr, T** p, size_t count) {
     SZB_CUDA(ctx, cudaMalloc((void**)p, count * sizeof(T)));
@@ -1458,7 +1325,7 @@ static std::string t_layer_bn_name(int l) {
 
 static int t_create(szb_ctx* ctx, const szb_train_config* cfg) {
     int rc;
-    if ((rc = t_get_encode(ctx))) return rc;
+    if ((rc = net_tmap_init(ctx))) return rc;
     trainer_destroy(ctx);
     Trainer* tr = new Trainer();
     ctx->trainer = tr;
@@ -1468,11 +1335,20 @@ static int t_create(szb_ctx* ctx, const szb_train_config* cfg) {
     t_build_params(tr);
     const int cap = tr->cap;
     const size_t act = (size_t)cap * TPIX * TC;
+    // the two tensor maps of an activation buffer (2-board halo chunks, 1-board boxes) and of a weight pack (32 / 64 rows): see TLayer
+    auto act_maps = [&](CUtensorMap* chunk, CUtensorMap* board, void* base, int channels) {
+        const int r = net_tmap_halo(ctx, chunk, base, channels, cap, 2, "training halo activations");
+        return r ? r : net_tmap_act(ctx, board, base, channels, cap, 1, "training activations");
+    };
+    auto w_maps = [&](CUtensorMap* tm, void* base, int k_total, int rows) {
+        const int r = net_tmap_rows(ctx, &tm[0], base, k_total, rows, 128 / TR_CLUSTER, "training weights");
+        return r ? r : net_tmap_rows(ctx, &tm[1], base, k_total, rows, 64, "training weights");
+    };
     if ((rc = t_alloc(ctx, tr, &tr->w, tr->total)) || (rc = t_alloc(ctx, tr, &tr->g, tr->total)) || (rc = t_alloc(ctx, tr, &tr->m, tr->total)) ||
         (rc = t_alloc(ctx, tr, &tr->v, tr->total)))
         return rc;
     if ((rc = t_alloc(ctx, tr, &tr->x_in, (size_t)cap * TPIX * TCIN))) return rc;
-    if ((rc = t_halo_map(ctx, &tr->tm_in2, tr->x_in, TCIN, cap)) || (rc = t_act_map(ctx, &tr->tm_in1, tr->x_in, TCIN, cap, 1))) return rc;
+    if ((rc = act_maps(&tr->tm_in2, &tr->tm_in1, tr->x_in, TCIN))) return rc;
     for (int l = 0; l < T_LAYERS; l++) {
         TLayer& L = tr->L[l];
         L.taps = (l == L_P1 || l == L_P2) ? 1 : 9;
@@ -1481,14 +1357,10 @@ static int t_create(szb_ctx* ctx, const szb_train_config* cfg) {
         L.param = tr->index.at(t_layer_conv_name(l) + ".weight");
         const size_t wn = (size_t)L.cout_pad * L.taps * L.cin_pad;
         if ((rc = t_alloc(ctx, tr, &L.wf, wn))) return rc;
-        if ((rc = t_w_map(ctx, &L.tm_wf[0], L.wf, L.taps * L.cin_pad, L.cout_pad, 128 / TR_CLUSTER)) ||
-            (rc = t_w_map(ctx, &L.tm_wf[1], L.wf, L.taps * L.cin_pad, L.cout_pad, 64)))
-            return rc;
+        if ((rc = w_maps(L.tm_wf, L.wf, L.taps * L.cin_pad, L.cout_pad))) return rc;
         if (l != 0) {
             if ((rc = t_alloc(ctx, tr, &L.wd, wn))) return rc;
-            if ((rc = t_w_map(ctx, &L.tm_wd[0], L.wd, L.taps * L.cout_pad, L.cin_pad, 128 / TR_CLUSTER)) ||
-                (rc = t_w_map(ctx, &L.tm_wd[1], L.wd, L.taps * L.cout_pad, L.cin_pad, 64)))
-                return rc;
+            if ((rc = w_maps(L.tm_wd, L.wd, L.taps * L.cout_pad, L.cin_pad))) return rc;
         }
         if (l < T_BN) {
             L.gamma = tr->index.at(t_layer_bn_name(l) + ".weight");
@@ -1496,9 +1368,7 @@ static int t_create(szb_ctx* ctx, const szb_train_config* cfg) {
             if ((rc = t_alloc(ctx, tr, &L.y, act)) || (rc = t_alloc(ctx, tr, &L.o, act)) || (rc = t_alloc(ctx, tr, &L.dy, act)) ||
                 (rc = t_alloc(ctx, tr, &L.bn, 4 * 256)))
                 return rc;
-            if ((rc = t_halo_map(ctx, &L.tm_o2, L.o, TC, cap)) || (rc = t_act_map(ctx, &L.tm_o1, L.o, TC, cap, 1)) ||
-                (rc = t_halo_map(ctx, &L.tm_dy2, L.dy, TC, cap)) || (rc = t_act_map(ctx, &L.tm_dy1, L.dy, TC, cap, 1)))
-                return rc;
+            if ((rc = act_maps(&L.tm_o2, &L.tm_o1, L.o, TC)) || (rc = act_maps(&L.tm_dy2, &L.tm_dy1, L.dy, TC))) return rc;
             tr->buffers.push_back({t_layer_bn_name(l) + ".running_mean", 256, L.bn});
             tr->buffers.push_back({t_layer_bn_name(l) + ".running_var", 256, L.bn + 256});
         }
@@ -1506,8 +1376,7 @@ static int t_create(szb_ctx* ctx, const szb_train_config* cfg) {
     if (        (rc = t_alloc(ctx, tr, &tr->gm1, act)) || (rc = t_alloc(ctx, tr, &tr->skip[0], act)) || (rc = t_alloc(ctx, tr, &tr->skip[1], act)) ||
         (rc = t_alloc(ctx, tr, &tr->dl, (size_t)cap * TPIX * DL_C)))
         return rc;
-    if ((rc = t_halo_map(ctx, &tr->tm_dl2, tr->dl, DL_C, cap)) || (rc = t_act_map(ctx, &tr->tm_dl1, tr->dl, DL_C, cap, 1)))
-        return rc;
+    if ((rc = act_maps(&tr->tm_dl2, &tr->tm_dl1, tr->dl, DL_C))) return rc;
     tr->partial_floats = (size_t)WG_MAX_SPLIT * 256 * 256;                      // 1x1 layers: up to 64 splits of 256 x 256
     if (tr->partial_floats < (size_t)8 * 256 * 2304) tr->partial_floats = (size_t)8 * 256 * 2304;
     if ((rc = t_alloc(ctx, tr, &tr->partial, tr->partial_floats)) || (rc = t_alloc(ctx, tr, &tr->logits, (size_t)cap * T_ACTIONS)) ||
