@@ -205,6 +205,34 @@ typedef struct szb_exploration {
 } szb_exploration;
 int szb_set_exploration(szb_ctx *ctx, const szb_exploration *x);
 
+/* Opt-in evaluation cache (off by default).  Per game an open-addressed table of slots_per_game entries keyed on the EXACT evaluator
+ * input: a 128-bit hash of the leaf's 119 packed planes, its legal-move mask and the evaluator id.  A leaf whose key is live in its
+ * game's table (written or hit by this search or the previous one, under the current weights) takes the stored priors and value
+ * instead of an evaluation, and the evaluator runs only on the leaves that missed.  A board's evaluation does not depend on its batch,
+ * so every visit count, prior, value, move and record is bit-identical with the cache on and off; szb_stats counts a hit as an
+ * evaluation either way.  The one accepted risk is a 128-bit key collision (~2^-128 per comparison), as in a transposition table.
+ * Consulted by szb_search / szb_selfplay_ply with leaves_per_tree = 1 and the bf16 network (fused step) or the hash evaluator; the
+ * fp32 evaluator, profiling and SZB_NO_FUSE run without it.  Loading weights (szb_net_load, szb_net_load_device) or resizing
+ * invalidates every entry.  Memory: max_games x slots_per_game x 928 bytes (1024 games x 2048 slots: 1.9 GB).
+ * slots_per_game: 0 = off (frees the table), otherwise a power of two in [64, 65536] (SZB_ERR_ARG otherwise); the current size keeps
+ * the table.  SZB_ERR_UNSUPPORTED for leaves_per_tree > 1, SZB_ERR_CUDA if the table cannot be allocated; the setting is unchanged
+ * on any failure. */
+int szb_set_eval_cache(szb_ctx *ctx, int32_t slots_per_game);
+
+typedef struct szb_eval_cache_stats {
+    uint64_t lookups;              /* non-terminal leaves that consulted the cache (cumulative) */
+    uint64_t hits;
+    uint64_t inserts;              /* entries written */
+    uint64_t dropped_inserts;      /* misses whose probe window had no free entry */
+    uint64_t boards_evaluated;     /* boards the evaluator ran on in those searches: the sum of its per-step input-row counts, kept
+                                      on the device (every lookup that misses takes one row, so it equals lookups - hits) */
+    uint64_t bytes;                /* device memory of the table */
+    int32_t slots_per_game;        /* 0 = off */
+    int32_t reserved;
+} szb_eval_cache_stats;
+/* game_hits (optional, [n_games]): hits of each game in the last search. */
+int szb_get_eval_cache_stats(szb_ctx *ctx, szb_eval_cache_stats *out, uint32_t *game_hits);
+
 /* ---- counters (SURVEY.md 5: metrics) -------------------------------------------------------------- */
 typedef struct szb_stats {
     uint64_t simulations;          /* iterations of mcts.py:49 executed */

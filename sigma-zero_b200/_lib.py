@@ -60,6 +60,12 @@ class Exploration(ctypes.Structure):
                 ("sample_plies", ctypes.c_int32), ("reserved", ctypes.c_int32)]
 
 
+class EvalCacheStats(ctypes.Structure):
+    _fields_ = [("lookups", ctypes.c_uint64), ("hits", ctypes.c_uint64), ("inserts", ctypes.c_uint64),
+                ("dropped_inserts", ctypes.c_uint64), ("boards_evaluated", ctypes.c_uint64), ("bytes", ctypes.c_uint64),
+                ("slots_per_game", ctypes.c_int32), ("reserved", ctypes.c_int32)]
+
+
 TRAIN_FORWARD_ONLY, TRAIN_NO_UPDATE = 1, 2
 TRAIN_PARAMS, TRAIN_GRADS, TRAIN_EXP_AVG, TRAIN_EXP_AVG_SQ, TRAIN_ACTIVATIONS, TRAIN_MOMENTUM_BUFFER = 0, 1, 2, 3, 4, 5
 TRAIN_ADAM, TRAIN_SGD = 0, 1
@@ -94,6 +100,8 @@ SIGNATURES = {
     "szb_selfplay_ply": (ctypes.c_int, [_vp, _i32, _f32, _i32, _i32, _u64, _i32, _vp, _vp]),
     "szb_set_game_id_base": (ctypes.c_int, [_vp, _u64]),
     "szb_set_exploration": (ctypes.c_int, [_vp, ctypes.POINTER(Exploration)]),
+    "szb_set_eval_cache": (ctypes.c_int, [_vp, _i32]),
+    "szb_get_eval_cache_stats": (ctypes.c_int, [_vp, ctypes.POINTER(EvalCacheStats), _vp]),
     "szb_get_stats": (ctypes.c_int, [_vp, ctypes.POINTER(Stats)]),
     "szb_set_profiling": (ctypes.c_int, [_vp, _i32]),
     "szb_get_phase_times": (ctypes.c_int, [_vp, ctypes.POINTER(PhaseTimes)]),

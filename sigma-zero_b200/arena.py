@@ -9,6 +9,7 @@ games (szb_search works on a context's whole batch) and each game takes the move
 move in it.  Host logic only -- all chess and all search runs in the CUDA library."""
 import numpy as np
 
+from . import runtime
 from .engine import Engine, EVAL_NET_BF16, EVAL_NET_FP32
 
 
@@ -16,8 +17,10 @@ def _evaluator(model):
     return EVAL_NET_FP32 if getattr(model, "precision", "bf16") == "fp32" else EVAL_NET_BF16
 
 
-def play_match(model_a, model_b, num_games, args, c960=False, seed=0, max_plies=None, device=0, leaves_per_tree=None):
-    """Plays num_games games between model_a and model_b (arg-max of the visit counts, learning=False).
+def play_match(model_a, model_b, num_games, args, c960=False, seed=0, max_plies=None, device=0, leaves_per_tree=None,
+               eval_cache_slots=None):
+    """Plays num_games games between model_a and model_b (arg-max of the visit counts, learning=False).  eval_cache_slots (default:
+    args' 'eval_cache_slots', absent = off) gives each side's engine the exact evaluation cache: the same games, fewer evaluations.
 
     Returns {"score_a": points of model_a (win 1, draw 0.5), "results": per-game "1-0" / "0-1" / "1/2-1/2" / "*",
              "a_is_white": per-game bool, "plies": plies played, "moves": per-game list of the policy indices played}."""
@@ -26,12 +29,14 @@ def play_match(model_a, model_b, num_games, args, c960=False, seed=0, max_plies=
     a_white = np.arange(num_games) % 2 == 0
     start_ids = ([int(np.random.default_rng([int(seed), g // 2]).integers(0, 960)) for g in range(num_games)]
                  if c960 else [-1] * num_games)                       # both colours of a pair start from the same position
+    cache_slots = runtime.eval_cache_of(args if eval_cache_slots is None else {"eval_cache_slots": eval_cache_slots})
     engines = []
     for model in (model_a, model_b):
         e = Engine(max_games=num_games, max_searches=n_search, device=device, cohorts=1,
                    leaves_per_tree=int(args.get("leaves_per_tree", 1)) if leaves_per_tree is None else int(leaves_per_tree))
         e.load_state_dict(model.state_dict())
         e.reset(start_ids)
+        e.set_eval_cache(cache_slots)
         engines.append(e)
     ev = (_evaluator(model_a), _evaluator(model_b))
     moves = [[] for _ in range(num_games)]

@@ -656,9 +656,15 @@ __global__ void __launch_bounds__(128) k_expand(Dev d) {
     expand_path(d, T, ps, d.planes + (size_t)ps * PLANE_STRIDE);
 }
 
-// block per tree: policy[i] / value from the integer hash of the packed planes
+// block per tree: policy[i] / value from the integer hash of the packed planes.  EC (evaluation cache, fused step): block i serves
+// compacted row g_begin + i while i is below the step's device count, and the row's slot (d.row_slot) addresses everything.
+template <bool EC>
 __global__ void __launch_bounds__(128) k_hash_eval(Dev d) {
-    const int ps = d.g_begin * d.K + blockIdx.x;
+    int ps = d.g_begin * d.K + blockIdx.x;
+    if (EC) {
+        if ((int)blockIdx.x >= d.ec_cnt[d.ec_par]) return;
+        ps = d.row_slot[ps];
+    }
     if (!d.need_eval[ps]) return;
     __shared__ uint64_t h_sh;
     if (threadIdx.x == 0) {
@@ -721,8 +727,12 @@ __device__ __forceinline__ void root_noise(const Dev& d, unsigned long long e0, 
         d.e_w[e0 + k] = 0.0;
     }
 }
+// EC (evaluation cache, k_tree_step<true>): hit != null takes the compacted evaluator output from a cache entry instead of pol
+// (k-th legal move, ascending); ins != null copies the compacted output into the entry reserved for this leaf.
+template <bool EC = false>
 __device__ __forceinline__ int create_children(const Dev& d, const uint64_t* mk, const float* pol, unsigned long long e0, int rule,
-                                               uint64_t noise_key, int lane, uint16_t* idx_sh, float* p_sh) {
+                                               uint64_t noise_key, int lane, uint16_t* idx_sh, float* p_sh,
+                                               const float* hit = nullptr, float* ins = nullptr) {
     int n = 0;
 #pragma unroll 1
     for (int w = lane; w < 96; w += 32) {
@@ -739,12 +749,14 @@ __device__ __forceinline__ int create_children(const Dev& d, const uint64_t* mk,
             const int e = w * 64 + lsb(x);
             x &= x - 1;
             idx_sh[at] = (uint16_t)e;
-            p_sh[at] = pol[e];
+            p_sh[at] = (EC && hit) ? hit[at] : pol[e];
             at++;
         }
         n += __shfl_sync(0xFFFFFFFFu, incl, 31);
     }
     __syncwarp();
+    if (EC && ins)
+        for (int k = lane; k < n; k += 32) ins[k] = p_sh[k];
     float a0 = 0.0f, a1 = 0.0f;
     int cur = 0;                                             // 16-step block the pending a0 belongs to
     for (int k = 0; k < n; k++) {
@@ -786,10 +798,17 @@ constexpr int FINISH_WARPS = 2;
 
 // Second half of a simulation for the block's four trees (mcts.py:77-109): children of the evaluated node, then backup.  Called by
 // ALL threads of the block (two block-wide barriers inside); mk: 80 words of shared memory of this warp.
+// EC (evaluation cache): a leaf that hit takes its evaluator output (compacted priors, value) from its cache entry; a leaf that
+// missed with an entry reserved writes the evaluator's output there.  Everything after that runs on the same bits either way.
+template <bool EC = false>
 __device__ __forceinline__ void finish_block(const Dev& d, int learning, int slot, bool active, int lane, int wib, int* want_sh,
                                              unsigned long long* base_sh, uint64_t* mk, uint16_t* idx_sh, float* p_sh) {
     const int g = active ? d.order[slot] : 0;
     const bool eval = active && d.need_eval[slot];
+    int ec_ent = -1;
+    bool ec_hit = false;
+    if (EC && eval) { ec_ent = d.ec_ent[slot]; ec_hit = d.ec_hit[slot] != 0; }
+    const size_t ec_e = (size_t)g * d.ec_slots + (size_t)(ec_ent < 0 ? 0 : ec_ent);
     // Everything the backup needs is requested NOW, so that these round trips run under the mask -> arena bump -> priors chain
     // below instead of after it: the path, the statistics of its edges (only this warp touches them; the children created below
     // are new edges), the leaf's value, the root's sums.
@@ -803,7 +822,7 @@ __device__ __forceinline__ void finish_block(const Dev& d, int learning, int slo
     int n0 = 0, n1 = 0;
     if (pe0 >= 0) { w0 = d.e_w[pe0]; n0 = d.e_n[pe0]; }
     if (pe1 >= 0) { w1 = d.e_w[pe1]; n1 = d.e_n[pe1]; }
-    const float v = !active ? 0.f : (eval ? d.value[slot] : d.leaf_value[slot]);
+    const float v = !active ? 0.f : (eval ? ((EC && ec_hit) ? d.ec_meta[ec_e].value : d.value[slot]) : d.leaf_value[slot]);
     double root_w = 0.0;
     int root_n = 0, pedge = -1;
     if (active && lane == 0) { root_w = d.root_w[g]; root_n = d.root_n[g]; pedge = d.node_pedge[r + node]; }
@@ -832,8 +851,20 @@ __device__ __forceinline__ void finish_block(const Dev& d, int learning, int slo
             if (lane == 0) atomicExch(d.error_flag, SZB_ERR_ARENA);
         } else {
             const int rule = prior_rule(d, learning, node);
-            count = create_children(d, mk, d.policy + (size_t)slot * N_ACTIONS, e0, rule, rule == PRIOR_ROOT_NOISE ? root_noise_key(d, g) : 0ull,
-                                    lane, idx_sh, p_sh);
+            float* ec_p = EC && ec_ent >= 0 ? d.ec_pri + ec_e * EC_PRI_STRIDE : nullptr;
+            count = create_children<EC>(d, mk, d.policy + (size_t)slot * N_ACTIONS, e0, rule, rule == PRIOR_ROOT_NOISE ? root_noise_key(d, g) : 0ull,
+                                        lane, idx_sh, p_sh, ec_hit ? ec_p : nullptr, ec_hit ? nullptr : ec_p);
+            if (EC && ec_p && !ec_hit && lane == 0) {
+                EcMeta m;
+                m.k0 = d.ec_key[2 * (size_t)slot];
+                m.k1 = d.ec_key[2 * (size_t)slot + 1];
+                m.epoch = d.ec_epoch;
+                m.gen = d.ec_gen;
+                m.n_legal = (uint32_t)n_legal;
+                m.value = v;
+                d.ec_meta[ec_e] = m;
+                d.ec_gstats[(size_t)g * 4 + 2] += 1ull;
+            }
         }
         if (lane == 0) {
             d.node_edge0[r + node] = (int32_t)e0;
@@ -880,12 +911,66 @@ __global__ void __launch_bounds__(32 * FINISH_WARPS) k_finish(Dev d, int learnin
     finish_block(d, learning, slot, slot < d.g_end, threadIdx.x & 31, wib, want_sh, &base_sh, mk_sh + wib * MASK_STRIDE, idx_sh[wib], p_sh[wib]);
 }
 
+// Evaluation cache lookup (szb_set_eval_cache) of the non-terminal leaf in S (planes and legal mask in shared memory) by its warp;
+// returns whether it hit.
+//   key: lane l mixes the words l, l + 32, ... of (119 planes, 73 mask words) together with their index into two 64-bit wrapping
+//        sums of independent mixes; the warp reduction of a sum does not depend on the order it combines in; the evaluator id is
+//        mixed into the result.  The mask belongs to the key because the fused heads emit a softmax over the legal moves only and
+//        the planes do not encode every legality detail (en passant).  Two different inputs share a key with probability ~2^-128
+//        per comparison: the one accepted risk, as in a transposition table.
+//   probe: lane i reads entry (h + i) mod S of game g's table, 32 entries in one round trip.  An entry is live while its epoch is
+//        current and this search or the previous one wrote or hit it.  A hit refreshes the entry's generation; a miss reserves the
+//        window's first dead entry for finish_block to fill in the next step (none: the insert is dropped).
+//   Only game g's warp touches g's table, one leaf per step: no races, and the hits do not depend on slot, cohort or shard.
+__device__ __forceinline__ bool ec_lookup(const Dev& d, int slot, int lane, const ExpandShared& S) {
+    uint64_t a = 0, b = 0;
+    for (int i = lane; i < N_PLANES + MASK_WORDS; i += 32) {
+        const uint64_t x = (i < N_PLANES ? S.planes[i] : S.mask[i - N_PLANES]) + (uint64_t)(i + 1) * 0x9E3779B97F4A7C15ull;
+        a += mix64(x);
+        b += mix64(x ^ 0xD1B54A32D192ED03ull);
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        a += __shfl_xor_sync(0xFFFFFFFFu, a, off);
+        b += __shfl_xor_sync(0xFFFFFFFFu, b, off);
+    }
+    const uint64_t k0 = mix64(a ^ ((uint64_t)d.ec_eval << 56)), k1 = mix64(b + (uint64_t)d.ec_eval + 1ull);
+    const int g = d.order[slot];
+    const uint32_t wrap = (uint32_t)d.ec_slots - 1u, h = (uint32_t)(k0 >> 32);
+    EcMeta* tab = d.ec_meta + (size_t)g * d.ec_slots;
+    const EcMeta m = tab[(h + (uint32_t)lane) & wrap];
+    const bool live = m.epoch == d.ec_epoch && d.ec_gen - m.gen <= 1u;
+    const unsigned hit = __ballot_sync(0xFFFFFFFFu, live && m.k0 == k0 && m.k1 == k1);
+    const unsigned dead = __ballot_sync(0xFFFFFFFFu, !live);
+    const int first = __ffs(hit ? hit : dead) - 1;
+    const int ent = first < 0 ? -1 : (int)((h + (uint32_t)first) & wrap);
+    if (lane == 0) {
+        d.ec_key[2 * (size_t)slot] = k0;
+        d.ec_key[2 * (size_t)slot + 1] = k1;
+        d.ec_ent[slot] = ent;
+        d.ec_hit[slot] = hit != 0;
+        unsigned long long* gs = d.ec_gstats + (size_t)g * 4;
+        gs[0] += 1ull;
+        if (hit) {
+            tab[ent].gen = d.ec_gen;
+            gs[1] += 1ull;
+            d.ec_ghits[g] += 1u;
+        } else if (ent < 0) {
+            gs[3] += 1ull;
+        }
+    }
+    return hit != 0;
+}
+
 // One launch per simulation step and cohort in the reference-exact mode: the second half of step s-1 (children + backup of the
 // evaluated leaves), the first half of step s (PUCT descent, then move / legality / planes / mask of the new leaf) -- the same
 // warp owns its tree through all of it -- and the hand-over to the network: the leaf's input planes are written straight into the
 // tower's bf16 NHWC input rows and the tower's per-item completion counters are cleared, so a step is this kernel + one tower
 // launch (k_tower_tc2, whose last layer's epilogue emits the priors and the value k_finish reads: net.cu).
+// EC: the evaluation cache is consulted (a template parameter, so that the step without it keeps its 6.4 KB of shared memory and its
+// registers): a leaf that hits takes no input row; a miss takes the next compacted row of its cohort (d.row_slot records its slot).
 constexpr int STEP_FINISH = 1, STEP_SELECT = 2;
+template <bool EC>
 __global__ void __launch_bounds__(32 * FINISH_WARPS) k_tree_step(Dev d, float c_puct, int learning, int phases) {
     __shared__ Tables T;
     __shared__ int want_sh[FINISH_WARPS];
@@ -899,11 +984,19 @@ __global__ void __launch_bounds__(32 * FINISH_WARPS) k_tree_step(Dev d, float c_
     pdl_trigger();                                             // the tower launch behind me may begin its set-up and weight prefetch
     if (phases & STEP_SELECT) load_tables(&T, d.tables);       // (constant tables: before the wait)
     pdl_wait();                                                // the evaluator's priors / values; its completion counters are idle now
+    // the next step's row counter: its last reader, the evaluator of the step before this one, has completed (never zeroed by the
+    // step that increments it, and no host memset inside the chain of programmatic dependent launches)
+    // Before zeroing, the count it holds (the rows the previous step's evaluator ran on; 0 at step 0) goes into the cohort's running
+    // total of evaluated boards (szb_eval_cache_stats.boards_evaluated).
+    if (EC && blockIdx.x == 0 && threadIdx.x == 0) {
+        *d.ec_boards += (unsigned long long)d.ec_cnt[d.ec_par ^ 1];
+        d.ec_cnt[d.ec_par ^ 1] = 0;
+    }
     stamp(0);
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < d.net_ready_n; i += gridDim.x * blockDim.x) d.net_ready[i] = 0;
     stamp(1);
     if (phases & STEP_FINISH)      // (the expansion's shared memory is idle during the finish phase: mask, move list and planes serve as its scratch)
-        finish_block(d, learning, slot, active, lane, wib, want_sh, &base_sh, ex_sh[wib].mask, ex_sh[wib].mv, reinterpret_cast<float*>(ex_sh[wib].planes));
+        finish_block<EC>(d, learning, slot, active, lane, wib, want_sh, &base_sh, ex_sh[wib].mask, ex_sh[wib].mv, reinterpret_cast<float*>(ex_sh[wib].planes));
     if (!(phases & STEP_SELECT) || !active) return;
     __syncwarp();                                              // this warp's tree updates -> every lane of the descent
     stamp(2);
@@ -913,6 +1006,17 @@ __global__ void __launch_bounds__(32 * FINISH_WARPS) k_tree_step(Dev d, float c_
     ExpandShared& S = ex_sh[wib];
     if (!expand_warp(d, T, slot, lane, S, tr)) return;
     stamp(6);
+    int row = slot;
+    if (EC) {
+        if (ec_lookup(d, slot, lane, S)) return;
+        // Rows are handed out in whatever order the warps get here, so a leaf's row is not deterministic; its results are, because
+        // a board's evaluation does not depend on its row, its batch or its neighbours (DESIGN.md 3).
+        if (lane == 0) {
+            row = d.g_begin + atomicAdd(d.ec_cnt + d.ec_par, 1);
+            d.row_slot[row] = slot;
+        }
+        row = __shfl_sync(0xFFFFFFFFu, row, 0);
+    }
     const uint64_t* pl = S.planes;
     if (d.net_in16) {
         // 64 squares x 128 channels of bf16 (0 / 1.0) into the interior of the slot's zero-haloed [10][10][128] input row.  A lane takes
@@ -920,7 +1024,7 @@ __global__ void __launch_bounds__(32 * FINISH_WARPS) k_tree_step(Dev d, float c_
         // every byte of the result is one square's 8 channels -> one 16-byte store through a 256-entry table (byte -> 8 bf16, 4 KB in
         // global memory: L1-resident, and not part of the block's shared-memory footprint).
         // Lanes 0..15 / 16..31 write two squares' 256 contiguous bytes per store.
-        uint4* in = reinterpret_cast<uint4*>(d.net_in16 + (size_t)slot * 100 * 128);
+        uint4* in = reinterpret_cast<uint4*>(d.net_in16 + (size_t)row * 100 * 128);
         const int cg = lane & 15;
 #pragma unroll
         for (int it = 0; it < 4; it++) {
@@ -1399,6 +1503,7 @@ void szb_destroy(szb_ctx* ctx) {
     for (Pos* p : ctx->perft_levels) if (p) cudaFree(p);
     if (ctx->perft_counter) cudaFree(ctx->perft_counter);
     if (ctx->stage) cudaFree(ctx->stage);
+    if (ctx->ec_mem) cudaFree(ctx->ec_mem);
     for (int c = 0; c < 2; c++) {
         if (ctx->cohort_stream[c]) cudaStreamDestroy(ctx->cohort_stream[c]);
         if (ctx->ev_join[c]) cudaEventDestroy(ctx->ev_join[c]);
@@ -1474,6 +1579,8 @@ int szb_create(int device, const szb_config* cfg, szb_ctx** out) {
     A(planes, P * PLANE_STRIDE); A(mask, P * MASK_STRIDE);
     A(policy, P * N_ACTIONS); A(value, P); A(root_val, G);
     A(stats, 8); A(gstats, G * 8);
+    // evaluation cache bookkeeping (small; the tables themselves come with szb_set_eval_cache)
+    A(ec_key, G * 2); A(ec_ent, G); A(ec_hit, G); A(row_slot, G); A(ec_cnt, 4); A(ec_boards, 2); A(ec_gstats, G * 4); A(ec_ghits, G);
 #undef A
     if ((rc = dev_alloc(ctx, &ctx->d_moves, G + 1))) return rc;
     SZB_CUDA(ctx, cudaMalloc((void**)&ctx->perft_counter, sizeof(unsigned long long)));
@@ -1681,10 +1788,6 @@ static int run_search(szb_ctx* ctx, int num_searches, float c_puct, int learning
     if ((prof && !trace) || NS < 8) n_cohorts = 1;
     int bounds[3] = {0, NS, NS};
     if (n_cohorts == 2) bounds[1] = ((NS / 2 + 3) / 4) * 4;       // network tiles are 4 boards wide
-    if (n_cohorts == 2) {
-        SZB_CUDA(ctx, cudaEventRecord(ctx->ev_fork, st));
-        for (int c = 0; c < 2; c++) SZB_CUDA(ctx, cudaStreamWaitEvent(ctx->cohort_stream[c], ctx->ev_fork, 0));
-    }
     // one simulation step of the slots [dc.g_begin, dc.g_end) on stream cs; ev: five events around its four phases, or null
     auto launch_step = [&](const Dev& dc, cudaStream_t cs, cudaEvent_t* ev) -> int {
         const int n = dc.g_end - dc.g_begin, paths = n * K;
@@ -1700,7 +1803,7 @@ static int run_search(szb_ctx* ctx, int num_searches, float c_puct, int learning
         ctx->launches += 2;
         int rc_eval = 0;
         if (evaluator == SZB_EVAL_HASH) {
-            k_hash_eval<<<paths, 128, 0, cs>>>(dc);
+            k_hash_eval<false><<<paths, 128, 0, cs>>>(dc);
             ctx->launches++;
         } else {
             rc_eval = net_evaluate_batch(ctx, evaluator, dc.g_begin * K, paths, false);
@@ -1725,6 +1828,21 @@ static int run_search(szb_ctx* ctx, int num_searches, float c_puct, int learning
         SZB_CUDA(ctx, cudaMemsetAsync(d_step_trace, 0, (size_t)(n_steps + 1) * 8 * sizeof(unsigned long long), st));
     }
     const bool net_fused = fused && net_fused_step(ctx, evaluator);
+    // evaluation cache: consulted by the fused reference-exact step with the bf16 network or the hash evaluator; every other path
+    // (fp32 evaluator, profiling, SZB_NO_FUSE, phase kernels) runs without it and leaves it untouched
+    const bool ec = d.ec_slots > 0 && fused && (evaluator == SZB_EVAL_HASH || net_fused);
+    if (d.ec_slots > 0) SZB_CUDA(ctx, cudaMemsetAsync(d.ec_ghits, 0, sizeof(uint32_t) * (size_t)G, st));
+    if (ec) {
+        d.ec_gen++;
+        d.ec_eval = (uint32_t)evaluator;
+        SZB_CUDA(ctx, cudaMemsetAsync(d.ec_cnt, 0, 4 * sizeof(int32_t), st));
+    }
+    // the cohort streams fork from the context's stream only here, after everything enqueued on it for this search (the memsets
+    // above included): the streams are non-blocking, so work recorded after the fork would not be ordered before the cohorts' kernels
+    if (n_cohorts == 2) {
+        SZB_CUDA(ctx, cudaEventRecord(ctx->ev_fork, st));
+        for (int c = 0; c < 2; c++) SZB_CUDA(ctx, cudaStreamWaitEvent(ctx->cohort_stream[c], ctx->ev_fork, 0));
+    }
     // programmatic dependent launch chains the two kernels of a step when one cohort runs alone (the latency-bound regime); the
     // two-cohort pipeline already overlaps one cohort's tree kernel with the other's tower
     ctx->pdl = net_fused && n_cohorts == 1 && !getenv("SZB_NO_PDL");
@@ -1734,15 +1852,18 @@ static int run_search(szb_ctx* ctx, int num_searches, float c_puct, int learning
         ctx->work = cs;
         dc.net_in16 = nullptr; dc.net_ready = nullptr; dc.net_ready_n = 0;
         if (net_fused && (phases & STEP_SELECT)) net_handover(ctx, dc.g_begin, n, &dc.net_in16, &dc.net_ready, &dc.net_ready_n);
-        launch_kernel(k_tree_step, dim3((n + FINISH_WARPS - 1) / FINISH_WARPS), dim3(32 * FINISH_WARPS), 0, cs, ctx->pdl, dc, c_puct, learning, phases);
+        const dim3 grid((n + FINISH_WARPS - 1) / FINISH_WARPS), block(32 * FINISH_WARPS);
+        if (ec) launch_kernel(k_tree_step<true>, grid, block, 0, cs, ctx->pdl, dc, c_puct, learning, phases);
+        else launch_kernel(k_tree_step<false>, grid, block, 0, cs, ctx->pdl, dc, c_puct, learning, phases);
         ctx->launches++;
         if (!(phases & STEP_SELECT)) return 0;
         if (evaluator == SZB_EVAL_HASH) {
-            k_hash_eval<<<n, 128, 0, cs>>>(dc);
+            if (ec) k_hash_eval<true><<<n, 128, 0, cs>>>(dc);
+            else k_hash_eval<false><<<n, 128, 0, cs>>>(dc);
             ctx->launches++;
             return 0;
         }
-        return net_evaluate_batch(ctx, evaluator, dc.g_begin, n, net_fused);
+        return net_evaluate_batch(ctx, evaluator, dc.g_begin, n, net_fused, ec ? dc.ec_cnt + dc.ec_par : nullptr);
     };
     int rc = 0;
     for (int s = 0; s <= n_steps && !rc && NS > 0; s++) {
@@ -1754,6 +1875,9 @@ static int run_search(szb_ctx* ctx, int num_searches, float c_puct, int learning
             cudaStream_t cs = n_cohorts == 2 ? ctx->cohort_stream[c] : st;
             if (fused) {
                 dc.step_trace = (d_step_trace && c == 0) ? d_step_trace + (size_t)s * 8 : nullptr;
+                dc.ec_cnt = d.ec_cnt + 2 * c;                    // per cohort, per step parity
+                dc.ec_par = s & 1;
+                dc.ec_boards = d.ec_boards + c;
                 rc = launch_fused(dc, cs, (s > 0 ? STEP_FINISH : 0) | (s < n_steps ? STEP_SELECT : 0));
             } else {
                 cudaEvent_t* ev = prof ? &ctx->prof_events[5 * ((size_t)s * (trace ? 2 : 1) + (trace ? c : 0))] : nullptr;
@@ -1978,6 +2102,73 @@ int szb_set_exploration(szb_ctx* ctx, const szb_exploration* x) {
     ctx->d.dir_eps = e.dirichlet_epsilon;
     ctx->d.dir_seed = e.seed;
     ctx->sample_plies = e.sample_plies;
+    return 0;
+}
+
+int szb_set_eval_cache(szb_ctx* ctx, int32_t slots_per_game) {
+    if (ctx) cudaSetDevice(ctx->device);       // whichever device the calling thread had current
+    if (!ctx) return SZB_ERR_ARG;
+    Dev& d = ctx->d;
+    if (slots_per_game == 0) {
+        if (ctx->ec_mem) {
+            SZB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+            cudaFree(ctx->ec_mem);
+        }
+        ctx->ec_mem = nullptr;
+        ctx->ec_bytes = 0;
+        d.ec_slots = 0; d.ec_meta = nullptr; d.ec_pri = nullptr;
+        return 0;
+    }
+    if (slots_per_game < EC_MIN_SLOTS || slots_per_game > EC_MAX_SLOTS || (slots_per_game & (slots_per_game - 1)))
+        return fail(ctx, SZB_ERR_ARG, "szb_set_eval_cache: %d slots per game is not 0 or a power of two in [%d, %d]", slots_per_game,
+                    EC_MIN_SLOTS, EC_MAX_SLOTS);
+    if (d.K > 1)
+        return fail(ctx, SZB_ERR_UNSUPPORTED, "szb_set_eval_cache: the evaluation cache serves one leaf per tree and step (leaves_per_tree = %d)", d.K);
+    if (slots_per_game == d.ec_slots) return 0;
+    const size_t entries = (size_t)ctx->cfg.max_games * (size_t)slots_per_game;
+    const size_t meta_bytes = entries * sizeof(EcMeta), bytes = meta_bytes + entries * EC_PRI_STRIDE * sizeof(float);
+    void* mem = nullptr;
+    const cudaError_t e = cudaMalloc(&mem, bytes);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(ctx, SZB_ERR_CUDA, "szb_set_eval_cache: cannot allocate %zu bytes (%d games x %d slots x %zu B): %s", bytes,
+                    ctx->cfg.max_games, slots_per_game, sizeof(EcMeta) + EC_PRI_STRIDE * sizeof(float), cudaGetErrorString(e));
+    }
+    SZB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    SZB_CUDA(ctx, cudaMemsetAsync(mem, 0, meta_bytes, ctx->stream));
+    if (ctx->ec_mem) cudaFree(ctx->ec_mem);
+    ctx->ec_mem = mem;
+    ctx->ec_bytes = bytes;
+    d.ec_slots = slots_per_game;
+    d.ec_meta = (EcMeta*)mem;
+    d.ec_pri = (float*)((char*)mem + meta_bytes);
+    d.ec_epoch++;                              // a new table: nothing in it is live (the zeroed entries carry epoch 0)
+    SZB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return 0;
+}
+
+int szb_get_eval_cache_stats(szb_ctx* ctx, szb_eval_cache_stats* out, uint32_t* game_hits) {
+    if (ctx) cudaSetDevice(ctx->device);       // whichever device the calling thread had current
+    if (!ctx || !out) return fail(ctx, SZB_ERR_ARG, "szb_get_eval_cache_stats: bad arguments");
+    const size_t G = (size_t)ctx->cfg.max_games;
+    std::vector<unsigned long long> h(G * 4);
+    unsigned long long boards[2] = {0, 0};
+    SZB_CUDA(ctx, cudaMemcpyAsync(h.data(), ctx->d.ec_gstats, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, ctx->stream));
+    SZB_CUDA(ctx, cudaMemcpyAsync(boards, ctx->d.ec_boards, sizeof boards, cudaMemcpyDeviceToHost, ctx->stream));
+    if (game_hits && ctx->d.n_games > 0)
+        SZB_CUDA(ctx, cudaMemcpyAsync(game_hits, ctx->d.ec_ghits, sizeof(uint32_t) * (size_t)ctx->d.n_games, cudaMemcpyDefault, ctx->stream));
+    SZB_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    unsigned long long t[4] = {0, 0, 0, 0};
+    for (size_t g = 0; g < G; g++)
+        for (int k = 0; k < 4; k++) t[k] += h[g * 4 + k];
+    memset(out, 0, sizeof *out);
+    out->lookups = t[0];
+    out->hits = t[1];
+    out->inserts = t[2];
+    out->dropped_inserts = t[3];
+    out->boards_evaluated = boards[0] + boards[1];     // the evaluator's own row counts, summed by the tree kernels
+    out->bytes = ctx->ec_bytes;
+    out->slots_per_game = ctx->d.ec_slots;
     return 0;
 }
 

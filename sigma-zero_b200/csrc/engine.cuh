@@ -31,6 +31,17 @@ __host__ __device__ __forceinline__ int32_t link_edge0(unsigned long long l) { r
 __host__ __device__ __forceinline__ int link_nchild(unsigned long long l) { return (int)((l >> 32) & 0xFFFFu); }
 __host__ __device__ __forceinline__ uint16_t link_child(unsigned long long l) { return (uint16_t)(l >> 48); }
 
+// One entry of the evaluation cache (32 bytes); its priors live in a parallel array of EC_PRI_STRIDE floats.
+struct alignas(32) EcMeta {
+    uint64_t k0, k1;         // 128-bit key: input planes, legal mask, evaluator id
+    uint32_t epoch;          // Dev::ec_epoch when written
+    uint32_t gen;            // Dev::ec_gen of the last search that wrote or hit it
+    uint32_t n_legal;
+    float value;
+};
+constexpr int EC_PRI_STRIDE = 224;         // 218 legal moves at most, padded
+constexpr int EC_MIN_SLOTS = 64, EC_MAX_SLOTS = 65536;
+
 struct Net;                                // net.cu
 struct Trainer;                            // train.cu
 
@@ -100,6 +111,23 @@ struct Dev {
     float dir_alpha;             // > 0: searches with learning != 0 put Dirichlet(dir_alpha) noise on the root's priors
     float dir_eps;
     uint64_t dir_seed;
+    // ---- opt-in evaluation cache (szb_set_eval_cache): per game an open-addressed table keyed on the exact evaluator input ---------
+    int ec_slots;                // entries per game (a power of two), 0 = off
+    uint32_t ec_epoch;           // bumped whenever the weights change or the table is resized: older entries are dead
+    uint32_t ec_gen;             // this search's generation; entries of this search and the previous one are live
+    uint32_t ec_eval;            // evaluator id, part of the key
+    EcMeta* ec_meta;             // [max_games][ec_slots]
+    float* ec_pri;               // [max_games][ec_slots][EC_PRI_STRIDE] evaluator output of the legal moves, ascending policy index
+    uint64_t* ec_key;            // [slot][2] key of the slot's leaf (lookup -> finish of the next step)
+    int32_t* ec_ent;             // [slot] entry the leaf hit (hit) or reserved (miss), -1: none
+    uint8_t* ec_hit;             // [slot]
+    int32_t* row_slot;           // [row] slot whose leaf the evaluator's compacted input row `row` holds
+    int32_t* ec_cnt;             // this cohort's two per-step-parity row counters (set per launch)
+    unsigned long long* ec_boards;   // [2] per cohort: boards the evaluator ran on in searches that consulted the cache (cumulative;
+                                     // this launch's cohort entry while a search runs)
+    int ec_par;                  // parity of this launch's step
+    unsigned long long* ec_gstats;   // [max_games][4] lookups, hits, inserts, dropped inserts (cumulative)
+    uint32_t* ec_ghits;          // [max_games] hits of the last search
 };
 
 }  // namespace szb
@@ -132,6 +160,9 @@ struct szb_ctx {
     // self-play records
     int32_t* d_moves = nullptr;
     int32_t sample_plies = 0;                  // szb_exploration.sample_plies: sampled moves only while the root's ply is below it
+    // evaluation cache (szb_set_eval_cache): one allocation for the tables, freed when the cache is resized or switched off
+    void* ec_mem = nullptr;
+    uint64_t ec_bytes = 0;
     // profiling
     bool profiling = false;
     std::vector<cudaEvent_t> prof_events;
@@ -179,7 +210,7 @@ int fail(szb_ctx* ctx, int code, const char* fmt, ...);
 int cuda_fail(szb_ctx* ctx, cudaError_t e, const char* what);
 void* ctx_stage(szb_ctx* ctx, size_t bytes);
 // net.cu: evaluate games [g0, g0 + n) of d.planes -> d.policy / d.value (softmax policy) on ctx->work.
-int net_evaluate_batch(szb_ctx* ctx, int evaluator, int g0, int n, bool fused);
+int net_evaluate_batch(szb_ctx* ctx, int evaluator, int g0, int n, bool fused, const int32_t* n_live = nullptr);
 bool net_fused_step(szb_ctx* ctx, int evaluator);
 void net_handover(szb_ctx* ctx, int g0, int n, unsigned short** in16, int32_t** ready, int* ready_n);
 int net_reset_error(szb_ctx* ctx);

@@ -392,7 +392,17 @@ struct TowerHeads {
     const float *v_w, *fc1_wT, *fc1_b, *fc2_w;
     const float* scalars;              // {value-conv BN shift, fc_v2 bias}
     int row_delta;
+    // Evaluation cache (engine.cu, szb_set_eval_cache): the tree kernel compacts the leaves that missed the cache into the first
+    // *n_live rows of its cohort and records each row's slot in row_slot.  The launch then serves min(n_boards, *n_live - live_off)
+    // boards, read after griddepcontrol.wait; mask, need_eval, policy and value stay addressed by slot.  n_live == null: the host's
+    // count, row = slot.
+    const int32_t* row_slot;
+    const int32_t* n_live;
+    int live_off;                      // rows of the cohort before this launch's first board (chunked launches)
 };
+// boards of this launch the tree kernel filled, and the slot of an input row (see TowerHeads)
+__device__ __forceinline__ int heads_live_boards(const TowerHeads& h, int n_boards) { return max(0, min(n_boards, *h.n_live - h.live_off)); }
+__device__ __forceinline__ long heads_slot(const TowerHeads& h, long row) { return h.row_slot ? (long)h.row_slot[row] : row; }
 
 struct TowerArgs {
     int n_pair_tiles;    // ceil(boards / 4)
@@ -418,17 +428,18 @@ struct TowerArgs {
 };
 
 struct TowerItem { int l, t, q, ns; };
-__device__ __forceinline__ TowerItem tower_item(const TowerArgs& a, int item) {
+// tiles / n_main: a.n_pair_tiles / a.n_main, or their values for the tiles the device count leaves (TowerHeads::n_live)
+__device__ __forceinline__ TowerItem tower_item(const TowerArgs& a, int item, int tiles, int n_main) {
     TowerItem it;
-    if (item < a.n_main) {
+    if (item < n_main) {
         const int ti = item / a.nsplit;
         it.q = item - ti * a.nsplit;
-        it.l = a.layer_begin + ti / a.n_pair_tiles;
-        it.t = ti % a.n_pair_tiles;
+        it.l = a.layer_begin + ti / tiles;
+        it.t = ti % tiles;
         it.ns = a.nsplit;
     } else {
         it.l = a.layer_end - 1;
-        it.t = item - a.n_main;
+        it.t = item - n_main;
         it.q = 0;
         it.ns = 1;
     }
@@ -500,6 +511,9 @@ __device__ __forceinline__ bool mma_chunk_3x3_big(uint32_t d_tmem, uint32_t chun
     return true;
 }
 
+// DEV_COUNT: the launch serves the evaluation cache's compacted rows (TowerHeads::n_live / row_slot).  A template parameter, so that
+// the launch without it is the same kernel as before.
+template <bool DEV_COUNT>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
 k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ TowerArgs a) {
     constexpr uint32_t IDESC_BASE = idesc_bf16(256, 0);                    // M = 256, N per layer
@@ -520,10 +534,20 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const uint32_t rank = cluster_ctarank();
     const int pair = blockIdx.x >> 1, n_pairs = gridDim.x >> 1;
-    const int n_items = a.n_items;
+    int n_items = a.n_items, n_main = a.n_main, tiles = a.n_pair_tiles, n_live = a.n_boards;
     volatile int* abort_flag = &abort_sh;
 
     pdl_trigger();                                                // the next tree kernel may start its set-up; it waits for my completion
+    auto slot_of = [&](long row) -> long { return DEV_COUNT ? heads_slot(a.heads, row) : row; };
+    if (DEV_COUNT) {
+        // evaluation cache: only the first n_live boards were filled (the cache misses).  The count is the tree kernel's, so every
+        // thread waits for it first; the items of the tiles past it are dropped from the round-robin, which stays the same in every role.
+        pdl_wait();
+        n_live = heads_live_boards(a.heads, a.n_boards);
+        tiles = (n_live + 3) / 4;
+        n_main = a.n_main / a.n_pair_tiles * tiles;
+        n_items = n_main + (a.n_items - a.n_main) / a.n_pair_tiles * tiles;
+    }
     if (threadIdx.x == 0) {
         if (a.span) {
             atomicMin(a.span, global_ns());
@@ -571,7 +595,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
             // keep the loads ~7 taps ahead of the MMAs
             pdl_wait();                                           // input rows and cleared counters come from the kernel before me
             for (int item = pair; item < n_items && ok; item += n_pairs) {
-                const int l = a.layer_begin + item / a.n_pair_tiles, t = item % a.n_pair_tiles;
+                const int l = a.layer_begin + item / tiles, t = item % tiles;
                 const TowerLayer L = a.L[l];
                 if (l > a.layer_begin && !(ok = wait_dependency(l, t))) break;
                 if (a.trace && rank == 0 && lane == 0) a.trace[(size_t)item * 4 + 0] = global_ns();      // dependency resolved
@@ -627,7 +651,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
             // the dependency wait (weights do not depend on the previous layer), then all activation chunks at once, then the
             // remaining weight stages.
             for (int item = pair; item < n_items && ok; item += n_pairs) {
-                const TowerItem it = tower_item(a, item);
+                const TowerItem it = tower_item(a, item, tiles, n_main);
                 const int l = it.l, t = it.t, q = it.q;
                 const TowerLayer L = a.L[l];
                 const CUtensorMap* tm_a = &maps.a[L.a_map];
@@ -693,7 +717,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
             bool ok = true;
             const bool big = a.nsplit == 1 && a.tps1 == 2;
             for (int item = pair; item < n_items && ok; item += n_pairs, local++) {
-                const TowerItem it = tower_item(a, item);
+                const TowerItem it = tower_item(a, item, tiles, n_main);
                 const TowerLayer L = a.L[it.l];
                 const uint32_t idesc = IDESC_BASE | ((uint32_t)(2 * L.n_half / it.ns >> 3) << 17);
                 const uint32_t acc = local & 1;
@@ -749,7 +773,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
         int local = 0;
         bool ok = true;
         for (int item = pair; item < n_items && ok; item += n_pairs, local++) {
-            const TowerItem it = tower_item(a, item);
+            const TowerItem it = tower_item(a, item, tiles, n_main);
             const int l = it.l, t = it.t, q = it.q;
             const TowerLayer L = a.L[l];
             const int n_item = 2 * L.n_half / it.ns, cb = q * n_item;         // this item's output channels: [cb, cb + n_item)
@@ -762,7 +786,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
             const int row = lane_group * 32 + lane;
             const int board = a.board0 + (t * 2 + (int)rank) * 2 + ((row >> 3) & 1);
             const int sq = (row >> 4) * 8 + (row & 7);
-            const bool live = board < a.board0 + a.n_boards;
+            const bool live = board < a.board0 + n_live;
             const uint32_t taddr = tmem_base + ((uint32_t)(lane_group * 32) << 16) + acc * ACC_COLS;
             const size_t pix = ((size_t)board * HALO + (sq >> 3) + 1) * HALO + (sq & 7) + 1;
             // The residual (output of layer l - 2) starts its way from L2 before the accumulator wait -- but only once this warp
@@ -793,11 +817,11 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                 // bit-identical to the unfused path's; only the legal moves' entries are written.
                 const int rb = (row >> 3) & 1;                                        // board within this CTA
                 const int cta_board0 = a.board0 + (t * 2 + (int)rank) * 2;
-                const long row_slot = (long)board + a.heads.row_delta;
+                const long row_slot = DEV_COUNT ? (live ? heads_slot(a.heads, (long)board + a.heads.row_delta) : 0) : (long)board + a.heads.row_delta;
                 const bool want = live && a.heads.need_eval[row_slot] != 0;
                 for (int i = etid; i < 2 * MASK_WORDS; i += 128) {
                     const int bb = i >= MASK_WORDS, w = i - bb * MASK_WORDS, brd = cta_board0 + bb;
-                    hd_mask[bb][w] = brd < a.board0 + a.n_boards ? a.heads.mask[(size_t)(brd + a.heads.row_delta) * MASK_STRIDE + w] : 0ull;
+                    hd_mask[bb][w] = brd < a.board0 + n_live ? a.heads.mask[(size_t)slot_of(brd + a.heads.row_delta) * MASK_STRIDE + w] : 0ull;
                 }
                 hd_vw[etid] = a.heads.v_w[etid];
                 hd_vw[etid + 128] = a.heads.v_w[etid + 128];
@@ -884,11 +908,12 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                 named_bar_sync<1, 128>();
                 if (etid < 2) {
                     const int brd = cta_board0 + etid;
-                    if (brd < a.board0 + a.n_boards && a.heads.need_eval[brd + a.heads.row_delta]) {
+                    const long bslot = DEV_COUNT ? (brd < a.board0 + n_live ? heads_slot(a.heads, brd + a.heads.row_delta) : 0) : brd + a.heads.row_delta;
+                    if (brd < a.board0 + n_live && a.heads.need_eval[bslot]) {
                         float tt = a.heads.scalars[1];
 #pragma unroll
                         for (int w = 0; w < 8; w++) tt = __fadd_rn(tt, hd_fc[etid][w]);
-                        a.heads.value[brd + a.heads.row_delta] = vh_tanh(tt);
+                        a.heads.value[bslot] = vh_tanh(tt);
                     }
                 }
                 continue;
@@ -1075,6 +1100,12 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
     volatile int* abort_flag = &abort_sh;
 
     pdl_trigger();
+    // evaluation cache: a cluster whose board lies past the tree kernel's count of filled rows has nothing to do (all its CTAs see
+    // the same board and leave together, before any cluster barrier)
+    if (a.heads.n_live) {
+        pdl_wait();
+        if (board - a.board0 >= heads_live_boards(a.heads, a.n_boards)) return;
+    }
     if (threadIdx.x == 0) {
         abort_sh = 0;
         for (int s = 0; s < CL_B_STAGES; s++) { mbar_init(smem_u32(&bar_b_full[s]), 1); mbar_init(smem_u32(&bar_b_empty[s]), 1); }
@@ -1310,7 +1341,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
             // softmax over the board's 73 x 64 logits gathered in this CTA's buffer 1, in k_softmax's order; thread = square (64 threads)
             ok = __all_sync(0xFFFFFFFFu, mbar_wait_cluster(smem_u32(&bar_lg), 0, abort_flag));
             const float* lg = reinterpret_cast<const float*>(smem_raw + (lg_base - smem_u32(smem_raw)));
-            const long row_slot = (long)board + a.heads.row_delta;
+            const long row_slot = heads_slot(a.heads, (long)board + a.heads.row_delta);
             const bool search = a.heads.mask != nullptr;
             const bool want = ok && (!search || a.heads.need_eval[row_slot] != 0);
             if (search)
@@ -1386,7 +1417,7 @@ k_tower_cl(const __grid_constant__ TowerMaps maps, const __grid_constant__ Clust
             }
             named_bar_sync<1, 128>();
             if (etid == 0 && ok) {
-                const long row_slot = (long)board + a.heads.row_delta;
+                const long row_slot = heads_slot(a.heads, (long)board + a.heads.row_delta);
                 if (a.heads.mask == nullptr || a.heads.need_eval[row_slot]) {
                     float tt = a.heads.scalars[1];
 #pragma unroll
@@ -1844,6 +1875,9 @@ struct TowerRun {
     bool in16_rows = false;      // the input planes of board b0 + i already sit in NHWC input row out_row + i (written by k_tree_step)
     bool ready_zeroed = false;   // the launch's completion counters were cleared by the kernel before it on the stream
     bool pdl = false;            // programmatic dependent launch behind the step's tree kernel
+    const int32_t* n_live = nullptr;     // evaluation cache: device count of the rows the tree kernel filled (TowerHeads::n_live)
+    const int32_t* row_slot = nullptr;
+    int live_off = 0;
 };
 
 // layers [layer_begin, layer_end) of the tower for n boards in one persistent CTA-pair launch
@@ -1852,9 +1886,10 @@ static int launch_tower(szb_ctx* ctx, Net* net, int b0, int n, int layer_begin, 
         // "exclusive" launches ask for all the shared memory a block can have, so that no other block fits on an SM next to a
         // tower CTA (every block also reserves 1 KiB of system shared memory): see Net::tower_pairs
         cudaFuncAttributes fa;
-        SZB_CUDA(ctx, cudaFuncGetAttributes(&fa, k_tower_tc2));
+        SZB_CUDA(ctx, cudaFuncGetAttributes(&fa, k_tower_tc2<false>));
         net->smem_exclusive = std::max(T2_SMEM, 232448 - (int)fa.sharedSizeBytes);
-        SZB_CUDA(ctx, cudaFuncSetAttribute(k_tower_tc2, cudaFuncAttributeMaxDynamicSharedMemorySize, net->smem_exclusive));
+        SZB_CUDA(ctx, cudaFuncSetAttribute(k_tower_tc2<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, net->smem_exclusive));
+        SZB_CUDA(ctx, cudaFuncSetAttribute(k_tower_tc2<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, net->smem_exclusive));
         // The pairs of a launch wait on one another (per-item completion counters), so every pair must be able to become
         // resident while the others spin: never launch more pairs than this device can hold at once.
         cudaLaunchConfig_t cfg = {};
@@ -1862,7 +1897,7 @@ static int launch_tower(szb_ctx* ctx, Net* net, int b0, int n, int layer_begin, 
         cfg.blockDim = dim3(TC_THREADS);
         cfg.dynamicSmemBytes = T2_SMEM;
         int clusters = 0;
-        if (cudaOccupancyMaxActiveClusters(&clusters, k_tower_tc2, &cfg) == cudaSuccess && clusters > 0)
+        if (cudaOccupancyMaxActiveClusters(&clusters, k_tower_tc2<false>, &cfg) == cudaSuccess && clusters > 0)
             net->pairs_resident = std::min(net->num_sms / 2, clusters);
         else
             cudaGetLastError();
@@ -1887,8 +1922,10 @@ static int launch_tower(szb_ctx* ctx, Net* net, int b0, int n, int layer_begin, 
         h.tower_out = net->act16[net->final_x];
         h.v_w = net->v_w; h.fc1_wT = net->fc1_w; h.fc1_b = net->fc1_b; h.fc2_w = net->fc2_w; h.scalars = net->head_scalars;
         h.row_delta = (out_row >= 0 ? out_row : b0) - b0;
+        h.row_slot = run.row_slot; h.n_live = run.n_live; h.live_off = run.live_off;
     } else {
         a.heads.mask = nullptr;
+        a.heads.row_slot = nullptr; a.heads.n_live = nullptr;
     }
     // Small batches leave most CTA pairs idle and the launch becomes a chain of 41 dependent layers: cut every (layer, tile)
     // into 2 or 4 items of N / nsplit output channels so that up to all pairs work on one layer.  Same MMAs per output, same K
@@ -1916,7 +1953,7 @@ static int launch_tower(szb_ctx* ctx, Net* net, int b0, int n, int layer_begin, 
         net->span_b0.push_back(b0);
     }
     const int grid = 2 * std::min(a.n_pair_tiles * a.nsplit, pairs);
-    SZB_CUDA(ctx, launch_kernel(k_tower_tc2, dim3(grid), dim3(TC_THREADS), (size_t)(exclusive ? net->smem_exclusive : T2_SMEM), ctx->work,
+    SZB_CUDA(ctx, launch_kernel(a.heads.mask && a.heads.n_live ? k_tower_tc2<true> : k_tower_tc2<false>, dim3(grid), dim3(TC_THREADS), (size_t)(exclusive ? net->smem_exclusive : T2_SMEM), ctx->work,
                                 run.pdl, *net->tower_maps, a));
     ctx->launches++;
     return 0;
@@ -1982,6 +2019,7 @@ static int launch_tower_cluster(szb_ctx* ctx, Net* net, int cs, int b0, int n, i
     if (run.heads) {
         const Dev& d = ctx->d;
         h.mask = d.mask; h.need_eval = d.need_eval; h.policy = d.policy; h.value = d.value;
+        h.row_slot = run.row_slot; h.n_live = run.n_live; h.live_off = run.live_off;
     } else {
         h.mask = nullptr; h.need_eval = nullptr; h.policy = nullptr;
         h.value = value_out - (ptrdiff_t)out_row;             // value[board + row_delta] == value_out[board - b0]
@@ -2157,6 +2195,7 @@ static int net_forward_chunked(szb_ctx* ctx, int evaluator, int b0, int n, const
     const int chunk = (evaluator == SZB_EVAL_NET_BF16 && net->tower_mode == 2 && net->chunk > 0) ? net->chunk : n;
     for (int off = 0; off < n; off += chunk) {
         const int m = std::min(chunk, n - off);
+        run.live_off = off;                                       // (evaluation cache: each chunk clamps itself to the device count)
         int rc = net_forward_device(ctx, evaluator, b0, m, planes + (size_t)off * stride, stride, value_out + off, b0 + off, run);
         if (rc) return rc;
         run.ready_zeroed = false;                                 // later chunks reuse the first chunk's counters: clear them again
@@ -2181,11 +2220,13 @@ void net_handover(szb_ctx* ctx, int g0, int n, unsigned short** in16, int32_t** 
 }
 
 // evaluate slots [g0, g0 + n) of the search batch (g0 a multiple of 4): d.planes -> d.policy (softmax; the legal entries only when the
-// heads are fused) / d.value, on ctx->work.  fused: the step's k_tree_step filled the input rows and cleared the counters.
-int net_evaluate_batch(szb_ctx* ctx, int evaluator, int g0, int n, bool fused) {
+// heads are fused) / d.value, on ctx->work.  fused: the step's k_tree_step filled the input rows and cleared the counters.  n_live
+// (fused only; evaluation cache): the step's device count of compacted input rows, whose slots are d.row_slot[g0 ..].
+int net_evaluate_batch(szb_ctx* ctx, int evaluator, int g0, int n, bool fused, const int32_t* n_live) {
     TowerRun run;
     run.heads = run.in16_rows = run.ready_zeroed = fused;
     run.pdl = fused && ctx->pdl;
+    if (fused && n_live) { run.n_live = n_live; run.row_slot = ctx->d.row_slot; }
     int rc = net_forward_chunked(ctx, evaluator, g0, n, ctx->d.planes + (size_t)g0 * PLANE_STRIDE, PLANE_STRIDE, ctx->d.value + g0, run);
     if (rc || fused) return rc;
     k_softmax<<<(n + 3) / 4, 256, 0, ctx->work>>>(ctx->net->logits + (size_t)g0 * N_ACTIONS, ctx->d.policy + (size_t)g0 * N_ACTIONS, n);
@@ -2269,6 +2310,7 @@ static int net_ensure_allocated(szb_ctx* ctx) {
 // fold + pack all tensors (DEVICE pointers) into the network's buffers; asynchronous on the context's stream, no host round trip
 static int net_fill_from_device(szb_ctx* ctx, const std::map<std::string, const float*>& sd) {
     Net* net = ctx->net;
+    ctx->d.ec_epoch++;                  // the one place the packed weights change: every evaluation cache entry is dead from here on
     auto at = [&](const std::string& k) { return sd.at(k); };
     auto bn_of = [&](const std::string& p) { return BN{at(p + ".weight"), at(p + ".bias"), at(p + ".running_mean"), at(p + ".running_var")}; };
     int rc;

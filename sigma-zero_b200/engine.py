@@ -236,6 +236,23 @@ class Engine:
         x = _lib.Exploration(float(alpha), float(epsilon), int(seed) & (2 ** 64 - 1), int(sample_plies), 0)
         self._check(self.lib.szb_set_exploration(self._h, ctypes.byref(x)))
 
+    def set_eval_cache(self, slots_per_game=0):
+        """Opt-in exact evaluation cache for the searches that follow (szb_set_eval_cache): per game a table of slots_per_game
+        entries (0 = off, else a power of two in [64, 65536]) keyed on the exact evaluator input, so that positions an earlier
+        search of the same game evaluated skip the network.  Results are bit-identical with the cache on and off."""
+        self._check(self.lib.szb_set_eval_cache(self._h, int(slots_per_game)))
+
+    def eval_cache_stats(self, game_hits=False):
+        """Cumulative counters of the evaluation cache (lookups, hits, inserts, dropped_inserts, boards_evaluated, bytes,
+        slots_per_game); with game_hits=True also each game's hits in the last search (uint32[n_games])."""
+        s = _lib.EvalCacheStats()
+        hits = np.zeros(max(self.n_games, 1), dtype=np.uint32) if game_hits else None
+        self._check(self.lib.szb_get_eval_cache_stats(self._h, ctypes.byref(s), _ptr(hits) if game_hits else None))
+        out = {n: getattr(s, n) for n, _ in _lib.EvalCacheStats._fields_ if n != "reserved"}
+        if game_hits:
+            out["game_hits"] = hits[:self.n_games]
+        return out
+
     def set_profiling(self, on=True):
         self._check(self.lib.szb_set_profiling(self._h, int(bool(on))))
 

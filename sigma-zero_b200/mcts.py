@@ -24,8 +24,10 @@ class MCTS0:
         eng = runtime.get_engine(min_games=1, min_searches=n, leaves_per_tree=runtime.leaves_of(args))
         runtime.sync_weights(eng, self.model)
         explore = runtime.exploration_of(args)
+        cache_slots = runtime.eval_cache_of(args)
         eng = self.game._engine()                    # replays the game into slot 0 if another game was there
         eng.set_exploration(seed=int(args.get('seed', 0)), **explore)
+        eng.set_eval_cache(cache_slots)
         white = bool(state.turn)
         eng.search(n, float(args['C']), bool(learning), runtime.evaluator_of(self.model),
                    want_visits=False, want_children=False)

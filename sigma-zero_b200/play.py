@@ -10,10 +10,11 @@ from .network import policyNN
 
 
 class PlayTensor:
-    def __init__(self, model_path=None, num_searches=200, C=2, chess960=False, precision="bf16", leaves_per_tree=1):
+    def __init__(self, model_path=None, num_searches=200, C=2, chess960=False, precision="bf16", leaves_per_tree=1, eval_cache_slots=0):
         """leaves_per_tree > 1: the opt-in multi-leaf search (virtual loss; ~7x faster move decisions for a single game at 8, but
-        not the reference's visit counts)"""
-        self.args = {"C": C, "num_searches": num_searches, "leaves_per_tree": leaves_per_tree}
+        not the reference's visit counts).  eval_cache_slots > 0 (a power of two in [64, 65536]): the exact evaluation cache, so
+        positions the previous move's search evaluated skip the network (the same moves)."""
+        self.args = {"C": C, "num_searches": num_searches, "leaves_per_tree": leaves_per_tree, "eval_cache_slots": eval_cache_slots}
         self.chess960 = chess960
         self.network = policyNN({"precision": precision})
         if model_path:                                    # play.py:25-28: torch.load(..., map_location) -> load_state_dict

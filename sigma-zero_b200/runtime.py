@@ -55,6 +55,17 @@ def exploration_of(args):
     return {"alpha": alpha, "epsilon": epsilon, "sample_plies": int(sample_plies)}
 
 
+def eval_cache_of(args):
+    """Engine.set_eval_cache's slots_per_game from the args-dict extension 'eval_cache_slots' (absent = 0 = off).  Raises
+    ValueError unless it is 0 or a power of two in [64, 65536]."""
+    slots = (args or {}).get('eval_cache_slots', 0)
+    if slots is None:
+        slots = 0
+    if int(slots) != slots or not (int(slots) == 0 or (64 <= int(slots) <= 65536 and int(slots) & (int(slots) - 1) == 0)):
+        raise ValueError("eval_cache_slots must be 0 or a power of two in [64, 65536], not %r" % (slots,))
+    return int(slots)
+
+
 def evaluator_of(model):
     prec = getattr(model, "precision", DEFAULT_PRECISION)
     return EVAL_NET_FP32 if prec == "fp32" else EVAL_NET_BF16

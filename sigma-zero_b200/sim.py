@@ -23,9 +23,11 @@ def selfplay_batch(model, args, num_games, c960=False, seed=None, start_ids=None
     959), chess_tensor.py:69), the moves sampled from the visit counts (sim.py:68) and the root noise of the opt-in exploration
     -- is a function of (seed, global game id = game_id_base + index) only, so a job sharded over ranks plays exactly the games
     a single process would.  args may carry 'dirichlet_alpha', 'dirichlet_epsilon' and 'sample_plies' (runtime.exploration_of);
-    without them the engine's exploration is switched off."""
+    without them the engine's exploration is switched off.  'eval_cache_slots' (runtime.eval_cache_of) switches the exact
+    evaluation cache on: the same games, fewer network evaluations."""
     n_search = int(args['num_searches'])
     explore = runtime.exploration_of(args)
+    cache_slots = runtime.eval_cache_of(args)
     eng = runtime.get_engine(min_games=num_games, min_searches=n_search, leaves_per_tree=runtime.leaves_of(args))
     runtime.sync_weights(eng, model)
     eng.owner = None
@@ -37,6 +39,7 @@ def selfplay_batch(model, args, num_games, c960=False, seed=None, start_ids=None
     eng.reset(start_ids)
     eng.set_game_id_base(game_id_base)
     eng.set_exploration(seed=int(seed), **explore)
+    eng.set_eval_cache(cache_slots)
     seed64 = int(seed)
     games = [_empty_history() for _ in range(num_games)]
     evaluator = runtime.evaluator_of(model)
@@ -86,6 +89,7 @@ def selfplay_records(model, args, num_games, c960=False, seed=None, start_ids=No
     per game: 1 white won, -1 black won, 0 draw, 2 unfinished (max_plies)."""
     n_search = int(args['num_searches'])
     explore = runtime.exploration_of(args)
+    cache_slots = runtime.eval_cache_of(args)
     eng = runtime.get_engine(min_games=num_games, min_searches=n_search, leaves_per_tree=runtime.leaves_of(args))
     runtime.sync_weights(eng, model)
     eng.owner = None
@@ -97,6 +101,7 @@ def selfplay_records(model, args, num_games, c960=False, seed=None, start_ids=No
     eng.reset(start_ids)
     eng.set_game_id_base(game_id_base)
     eng.set_exploration(seed=int(seed), **explore)
+    eng.set_eval_cache(cache_slots)
     evaluator = runtime.evaluator_of(model)
     col = np.arange(256)[None, :]
     st, gm, pl, ix, pr, ln = [], [], [], [], [], []

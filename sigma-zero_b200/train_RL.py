@@ -359,8 +359,9 @@ def main(args=None, model=None, weights=None, num_games=None, out_dir=".", seed=
 
 def build_parser():
     """the command line of `python -m sigma_zero_b200.train_RL`: DEFAULT_ARGS as flags plus the run's settings and the opt-in
-    extensions of the args dict (--leaves_per_tree, and --dirichlet_alpha / --dirichlet_epsilon / --sample_plies for AlphaZero's
-    root noise and sampling horizon in self-play; the defaults are the reference's behaviour)"""
+    extensions of the args dict (--leaves_per_tree, --dirichlet_alpha / --dirichlet_epsilon / --sample_plies for AlphaZero's
+    root noise and sampling horizon in self-play, and --eval_cache_slots for the exact evaluation cache; the defaults are the
+    reference's behaviour)"""
     import argparse
     ap = argparse.ArgumentParser(description="self-play + fine-tuning loop of the reference's train_RL.py on the B200 engine "
                                              "(under torchrun the games of an epoch are split over the ranks)")
@@ -376,10 +377,14 @@ def build_parser():
     ap.add_argument("--dirichlet_epsilon", type=float, default=0.25, help="weight of the root noise")
     ap.add_argument("--sample_plies", type=int, default=0,
                     help="sample moves from the visit counts for this many plies of a game, then play the arg-max; 0 = sample every ply")
+    ap.add_argument("--eval_cache_slots", type=int, default=0,
+                    help="exact evaluation cache for self-play: entries per game, a power of two in [64, 65536] (e.g. 2048; "
+                         "max_games x slots x 928 bytes of GPU memory); 0 = off.  The games are bit-identical either way")
     return ap
 
 
-CLI_ARGS = list(DEFAULT_ARGS) + ["start_epoch", "leaves_per_tree", "dirichlet_alpha", "dirichlet_epsilon", "sample_plies"]
+CLI_ARGS = list(DEFAULT_ARGS) + ["start_epoch", "leaves_per_tree", "dirichlet_alpha", "dirichlet_epsilon", "sample_plies",
+                                 "eval_cache_slots"]
 
 
 if __name__ == "__main__":
