@@ -1,12 +1,14 @@
 // engine.cu -- games, flat SoA search tree, batched MCTS step kernels, perft, and the C ABI around them.
 //
-// One simulation step of mcts.py:49-109 for ALL running games at once is four launches (finished games take no slot:
-// k_search_begin closes terminal roots, k_active_list numbers the rest):
-//   k_select  : warp per tree, PUCT descent with shuffle arg-max           (mctsnode.py:23-37, mcts.py:54-55)
-//   k_expand  : one thread per tree (own warp at search sizes), make-move + legality + terminal + planes (mcts.py:57-70, chess_tensor.py:88-172)
-//   evaluator : hash kernel or the network (net.cu)                         (mcts.py:72-75)
-//   k_finish  : warp per tree, mask/normalise/noise, child allocation, backup (mcts.py:77-109, mctsnode.py:39-63)
-// Opt-in multi-leaf mode (szb_config.leaves_per_tree > 1, not the reference's algorithm): k_select_vl / k_finish_vl.
+// One simulation step of mcts.py:49-109 runs for ALL running games at once (finished games take no slot: k_search_begin closes
+// terminal roots, k_active_list numbers the rest), a warp per tree through every phase:
+//   select    : PUCT descent, one warp arg-max per level (puct_pick)                 (mctsnode.py:23-37, mcts.py:54-55)
+//   expand    : make-move + legality + terminal + legal mask + planes (expand_warp)  (mcts.py:57-70, chess_tensor.py:88-172)
+//   evaluator : hash kernel or the network (net.cu)                                   (mcts.py:72-75)
+//   finish    : mask/normalise/noise, child allocation, backup (finish_block)         (mcts.py:77-109, mctsnode.py:39-63)
+// A search runs select, expand and finish in one kernel, k_tree_step, between evaluator launches.  Profiled searches (and
+// SZB_NO_FUSE) run the same code as the phase kernels k_select / k_expand / k_finish, and the opt-in multi-leaf mode
+// (szb_config.leaves_per_tree > 1, not the reference's algorithm) as k_select_vl / k_expand / k_finish_vl.
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -217,6 +219,32 @@ __global__ void __launch_bounds__(1024) k_active_list(Dev d) {
     if (threadIdx.x == 0) *d.n_active = base_sh;
 }
 
+// PUCT arg-max over the n children at edge e0 by one warp (mctsnode.py:23-37): lane t scores the children t, t + 32, ..., a shuffle
+// reduction picks the winner, the first index winning ties.  Returns its index; its visit count and e_link go to cn / lk.  All three
+// are the same in every lane.
+__device__ __forceinline__ int puct_pick(const Dev& d, int e0, int n, float sq, float c_puct, int lane, int& cn, unsigned long long& lk) {
+    float best = -INFINITY;
+    int besti = 0x7FFFFFFF, best_n = 0;
+    unsigned long long best_link = 0;
+    for (int i = lane; i < n; i += 32) {
+        const int c = d.e_n[e0 + i];
+        const unsigned long long l = d.e_link[e0 + i];
+        const float s = puct_score(c, d.e_w[e0 + i], d.e_p[e0 + i], sq, c_puct);
+        if (s > best || besti == 0x7FFFFFFF) { best = s; besti = i; best_n = c; best_link = l; }
+    }
+#pragma unroll
+    for (int off = 16; off > 0; off >>= 1) {
+        const float ob = __shfl_down_sync(0xFFFFFFFFu, best, off);
+        const int oi = __shfl_down_sync(0xFFFFFFFFu, besti, off);
+        if (oi != 0x7FFFFFFF && (besti == 0x7FFFFFFF || ob > best || (ob == best && oi < besti))) { best = ob; besti = oi; }
+    }
+    besti = __shfl_sync(0xFFFFFFFFu, besti, 0);
+    // child i was scored by lane i % 32, which still holds its visit count and link
+    cn = __shfl_sync(0xFFFFFFFFu, best_n, besti & 31);
+    lk = __shfl_sync(0xFFFFFFFFu, best_link, besti & 31);
+    return besti;
+}
+
 // PUCT descent of one tree by one warp (mctsnode.py:23-37, mcts.py:54-55).  One dependent memory round trip per level: the four
 // edge arrays of the node's children are read side by side, and the chosen child's header (child count, first edge) rides on its
 // edge (e_link), like its visit count and node index: the winning lane already holds them.  The edges walked are recorded
@@ -234,27 +262,8 @@ __device__ __forceinline__ void select_tree(const Dev& d, int slot, int lane, fl
             if (lane == 0) { d.sel_node[slot] = node; d.sel_edge[slot] = -1; }
             break;
         }
-        const float sq = sqrt_parent(np);
-        float best = -INFINITY;
-        int besti = 0x7FFFFFFF, best_n = 0;
-        unsigned long long best_link = 0;
-        for (int i = lane; i < n; i += 32) {
-            const int cn = d.e_n[e0 + i];
-            const unsigned long long lk = d.e_link[e0 + i];
-            const float s = puct_score(cn, d.e_w[e0 + i], d.e_p[e0 + i], sq, c_puct);
-            if (s > best || besti == 0x7FFFFFFF) { best = s; besti = i; best_n = cn; best_link = lk; }
-        }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            const float ob = __shfl_down_sync(0xFFFFFFFFu, best, off);
-            const int oi = __shfl_down_sync(0xFFFFFFFFu, besti, off);
-            if (oi != 0x7FFFFFFF && (besti == 0x7FFFFFFF || ob > best || (ob == best && oi < besti))) { best = ob; besti = oi; }
-        }
-        besti = __shfl_sync(0xFFFFFFFFu, besti, 0);
-        // child i was scored by lane i % 32, which still holds its visit count and link
-        np = __shfl_sync(0xFFFFFFFFu, best_n, besti & 31);
-        const unsigned long long lk = __shfl_sync(0xFFFFFFFFu, best_link, besti & 31);
-        const int e = e0 + besti;
+        unsigned long long lk;
+        const int e = e0 + puct_pick(d, e0, n, sqrt_parent(np), c_puct, lane, np, lk);
         if (lane == 0 && depth < PATH_CAP) path[depth] = e;
         depth++;
         scanned += (unsigned long long)n;
@@ -281,59 +290,6 @@ __global__ void __launch_bounds__(128) k_select(Dev d, float c_puct) {
     const int slot = d.g_begin + ((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     if (slot >= d.g_end) return;
     select_tree(d, slot, threadIdx.x & 31, c_puct);
-}
-
-// Expansion of path slot ps by ONE thread (mcts.py:57-70, chess_tensor.py:88-172,190-218): make the selected move, repetition
-// flags, legal moves, outcome, the 119 planes and the 4672-bit legal mask.  Returns whether the leaf needs the evaluator.
-// planes_out: where the packed planes go (the slot's row in d.planes, or a shared-memory copy the caller spreads afterwards).
-__device__ __forceinline__ bool expand_path(const Dev& d, const Tables& T, int ps, uint64_t* planes_out) {
-    const int g = d.order[ps / d.K];
-    const size_t r = (size_t)g * d.nodes_per_game;
-    Pos* gp = d.pool + (size_t)g * d.pool_stride;
-    const int e = d.sel_edge[ps];
-    if (e == PATH_DROPPED) { d.need_eval[ps] = 0; return false; }
-    int node = d.sel_node[ps];
-    uint16_t mv[MAX_MOVES];
-    int cnt = 0;
-    Pos q;
-    if (e >= 0) {
-        const int parent = node;
-        node = d.K == 1 ? ++d.node_count[g] : d.sel_new[ps];      // multi-leaf mode: numbered by k_select_vl
-        const int pslot = state_slot(d, g, parent);
-        const Pos pp = gp[pslot];
-        const uint16_t m = index_to_move(pp, d.e_move[e]);
-        make_move(T, pp, m, q);
-        q.prev = (uint32_t)pslot;
-        set_repetition_flags(gp, q);
-        analyse(T, q, mv, cnt);
-        gp[RING + node] = q;
-        set_ancestors(d, g, RING + node, (uint32_t)pslot);
-        d.node_pedge[r + node] = e;
-        d.node_pnode[r + node] = (uint16_t)parent;
-        d.node_nchild[r + node] = 0;
-        d.node_edge0[r + node] = -1;
-        d.node_term[r + node] = q.outcome != OUT_NONE;
-        d.node_tval[r + node] = q.outcome == OUT_CHECKMATE ? -1.0f : 0.0f;
-        d.e_link[e] = link_pack(-1, 0, (uint32_t)node);
-        d.sel_node[ps] = node;
-    } else {
-        q = gp[state_slot(d, g, node)];
-        if (!d.node_term[r + node]) cnt = gen_legal(T, q, mv);
-    }
-    if (d.node_term[r + node]) {
-        d.leaf_value[ps] = d.node_tval[r + node];
-        d.need_eval[ps] = 0;
-        return false;
-    }
-    uint64_t* mrow = d.mask + (size_t)ps * MASK_STRIDE;
-    for (int w = 0; w < MASK_STRIDE; w++) mrow[w] = 0;
-    for (int k = 0; k < cnt; k++) {
-        const int idx = move_to_index(q, mv[k]);
-        mrow[idx >> 6] |= bit(idx & 63);
-    }
-    pack_planes(gp, q, planes_out);
-    d.need_eval[ps] = 1;
-    return true;
 }
 
 // Legal moves of p by a whole warp (same SET as gen_legal, chess.cuh: the order differs, and nothing downstream depends on it).
@@ -471,50 +427,10 @@ __device__ __forceinline__ int gen_legal_warp(const Tables& T, const Pos& p, uin
     return __shfl_sync(0xFFFFFFFFu, incl, 31);
 }
 
-// legal indices (ascending) and/or planes + mask of the current positions.  Warp per game: the same warp-cooperative move
-// generation the search step uses (gen_legal_warp), so every szb_legal_moves / szb_encode call -- and every test built on them --
-// exercises it; perft and szb_games_push use the one-thread form (gen_legal, chess.cuh).
-__global__ void __launch_bounds__(128) k_games_encode(Dev d, int n, const int32_t* game, uint16_t* index_out, uint16_t* count_out,
-                                                      uint64_t* planes_out, uint64_t* mask_out) {
-    __shared__ Tables T;
-    __shared__ Pos p_sh[4];
-    __shared__ uint16_t mv_sh[4][MAX_MOVES];
-    __shared__ uint64_t m_sh[4][MASK_STRIDE];
-    load_tables(&T, d.tables);
-    const int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-    if (i >= n) return;
-    const int g = game ? game[i] : i;
-    if (g < 0 || g >= d.n_games) { if (count_out && lane == 0) count_out[i] = 0; return; }
-    const Pos* gp = d.pool + (size_t)g * d.pool_stride;
-    if (lane == 0) p_sh[wib] = gp[d.cur[g]];
-    for (int w = lane; w < MASK_STRIDE; w += 32) m_sh[wib][w] = 0;
-    __syncwarp();
-    const Pos& p = p_sh[wib];
-    const int cnt = gen_legal_warp(T, p, mv_sh[wib], lane);
-    __syncwarp();
-    for (int k = lane; k < cnt; k += 32) {
-        const int idx = move_to_index(p, mv_sh[wib][k]);
-        atomicOr(reinterpret_cast<unsigned long long*>(&m_sh[wib][idx >> 6]), 1ull << (idx & 63));
-    }
-    __syncwarp();
-    if (mask_out) for (int w = lane; w < MASK_WORDS; w += 32) mask_out[(size_t)i * MASK_WORDS + w] = m_sh[wib][w];
-    if (lane == 0) {
-        if (index_out) {
-            int k = 0;
-            for (int w = 0; w < MASK_WORDS; w++) {
-                uint64_t x = m_sh[wib][w];
-                while (x) { index_out[(size_t)i * SZB_MAX_MOVES + k++] = (uint16_t)(w * 64 + lsb(x)); x &= x - 1; }
-            }
-        }
-        if (count_out) count_out[i] = (uint16_t)cnt;
-        if (planes_out) pack_planes(gp, p, planes_out + (size_t)i * N_PLANES);
-    }
-}
-
 // The 119 planes of `now` (pool slot qslot of game g) by nine lanes: lane t < 8 packs history step t, whose position it loads
 // through the recorded predecessor slots (d.anc) -- eight independent loads instead of a walk along Pos::prev -- and lane 8 the
-// seven constant planes.  Same planes as pack_planes (chess.cuh), which k_expand / k_games_encode use: a step exists when every
-// link up to it holds (predecessor recorded and exactly one ply older: a recycled ring slot breaks the chain).
+// seven constant planes.  Same planes as pack_planes (chess.cuh), the host harness's form: a step exists when every link up to
+// it holds (predecessor recorded and exactly one ply older: a recycled ring slot breaks the chain).
 __device__ __forceinline__ void pack_planes_warp(const Dev& d, int g, const Pos* gp, int qslot, const Pos& now, uint64_t* out, int lane) {
     const bool white = now.flags & F_WHITE;
     const int own = white ? BB_WHITE : BB_BLACK, opp = white ? BB_BLACK : BB_WHITE;
@@ -556,28 +472,84 @@ __device__ __forceinline__ void pack_planes_warp(const Dev& d, int g, const Pos*
     }
 }
 
-// Expansion of the tree in `slot` by its warp (the latency-critical form k_tree_step uses; same results as expand_path): lane 0
-// makes the move and generates the legal moves into shared memory, then the lanes share the rest -- policy indices of the moves
-// into the shared-memory legal mask, history planes from eight independent position loads, coalesced copies out.
+// the legal moves mv[0 .. cnt) of p -> their policy indices in the 4672-bit mask (shared memory, zeroed by the caller), by a warp
+__device__ __forceinline__ void mask_moves(const Pos& p, const uint16_t* mv, int cnt, uint64_t* mask, int lane) {
+    for (int k = lane; k < cnt; k += 32) {
+        const int idx = move_to_index(p, mv[k]);
+        atomicOr(reinterpret_cast<unsigned long long*>(&mask[idx >> 6]), 1ull << (idx & 63));
+    }
+}
+
+// legal indices (ascending) and/or planes + mask of the current positions.  Warp per game, with the search step's own code for
+// moves, mask and planes (gen_legal_warp, mask_moves, pack_planes_warp): every szb_legal_moves / szb_encode call -- and every
+// test built on them -- checks what a search feeds its evaluator.  Perft and szb_games_push use the one-thread move generation
+// (gen_legal, chess.cuh).
+__global__ void __launch_bounds__(128) k_games_encode(Dev d, int n, const int32_t* game, uint16_t* index_out, uint16_t* count_out,
+                                                      uint64_t* planes_out, uint64_t* mask_out) {
+    __shared__ Tables T;
+    __shared__ Pos p_sh[4];
+    __shared__ uint16_t mv_sh[4][MAX_MOVES];
+    __shared__ uint64_t m_sh[4][MASK_STRIDE];
+    load_tables(&T, d.tables);
+    const int i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
+    if (i >= n) return;
+    const int g = game ? game[i] : i;
+    if (g < 0 || g >= d.n_games) { if (count_out && lane == 0) count_out[i] = 0; return; }
+    const Pos* gp = d.pool + (size_t)g * d.pool_stride;
+    const int qslot = d.cur[g];
+    if (lane == 0) p_sh[wib] = gp[qslot];
+    for (int w = lane; w < MASK_STRIDE; w += 32) m_sh[wib][w] = 0;
+    __syncwarp();
+    const Pos& p = p_sh[wib];
+    const int cnt = gen_legal_warp(T, p, mv_sh[wib], lane);
+    __syncwarp();
+    mask_moves(p, mv_sh[wib], cnt, m_sh[wib], lane);
+    __syncwarp();
+    if (mask_out) for (int w = lane; w < MASK_WORDS; w += 32) mask_out[(size_t)i * MASK_WORDS + w] = m_sh[wib][w];
+    if (lane == 0) {
+        if (index_out) {
+            int k = 0;
+            for (int w = 0; w < MASK_WORDS; w++) {
+                uint64_t x = m_sh[wib][w];
+                while (x) { index_out[(size_t)i * SZB_MAX_MOVES + k++] = (uint16_t)(w * 64 + lsb(x)); x &= x - 1; }
+            }
+        }
+        if (count_out) count_out[i] = (uint16_t)cnt;
+    }
+    if (planes_out) pack_planes_warp(d, g, gp, qslot, p, planes_out + (size_t)i * N_PLANES, lane);
+}
+
+// Expansion of path slot ps by its warp (mcts.py:57-70, chess_tensor.py:88-172,190-218): make the selected move, repetition
+// flags, legal moves, outcome, the 4672-bit legal mask and the 119 planes.  Lane 0 makes the move, the whole warp generates the
+// legal moves into shared memory, then the lanes share the rest -- policy indices of the moves into the shared-memory legal mask,
+// history planes from eight independent position loads, coalesced copies out.  Returns whether the leaf needs the evaluator.
+// K1 = true: the caller (k_tree_step) runs the reference-exact mode only, so the step kernel carries none of the multi-leaf mode's
+// code; K1 = false: K is read from d -- the tree is order[ps / K], and with K > 1 k_select_vl numbers the new nodes and may have
+// dropped the path.
 struct ExpandShared {
     Pos q;
     uint16_t mv[MAX_MOVES];
     uint64_t mask[MASK_STRIDE];
     uint64_t planes[PLANE_STRIDE];
 };
-__device__ __forceinline__ bool expand_warp(const Dev& d, const Tables& T, int slot, int lane, ExpandShared& S, unsigned long long* tr = nullptr) {
-    const int g = d.order[slot];
+template <bool K1>
+__device__ __forceinline__ bool expand_warp(const Dev& d, const Tables& T, int ps, int lane, ExpandShared& S, unsigned long long* tr = nullptr) {
+    if (!K1 && d.sel_edge[ps] == PATH_DROPPED) {
+        if (lane == 0) d.need_eval[ps] = 0;
+        return false;
+    }
+    const int g = d.order[K1 ? ps : ps / d.K];
     const size_t r = (size_t)g * d.nodes_per_game;
     Pos* gp = d.pool + (size_t)g * d.pool_stride;
     for (int w = lane; w < MASK_STRIDE; w += 32) S.mask[w] = 0;
     // lane 0: the position the leaf stands for (a new node: the parent's position + the selected move; else the node's own)
     int qslot = 0, term = -1, node = 0, e = 0, parent = 0;      // term: -1 = not known yet (a new node)
     if (lane == 0) {
-        e = d.sel_edge[slot];
-        node = d.sel_node[slot];
+        e = d.sel_edge[ps];
+        node = d.sel_node[ps];
         if (e >= 0) {
             parent = node;
-            node = ++d.node_count[g];
+            node = K1 || d.K == 1 ? ++d.node_count[g] : d.sel_new[ps];
             const int pslot = state_slot(d, g, parent);
             const Pos pp = gp[pslot];
             const uint16_t m = index_to_move(pp, d.e_move[e]);
@@ -615,45 +587,38 @@ __device__ __forceinline__ bool expand_warp(const Dev& d, const Tables& T, int s
             d.node_term[r + node] = (uint8_t)term;
             d.node_tval[r + node] = S.q.outcome == OUT_CHECKMATE ? -1.0f : 0.0f;
             d.e_link[e] = link_pack(-1, 0, (uint32_t)node);
-            d.sel_node[slot] = node;
+            d.sel_node[ps] = node;
         }
         if (term) {
-            d.leaf_value[slot] = d.node_tval[r + node];
-            d.need_eval[slot] = 0;
+            d.leaf_value[ps] = d.node_tval[r + node];
+            d.need_eval[ps] = 0;
         } else {
-            d.need_eval[slot] = 1;
+            d.need_eval[ps] = 1;
         }
     }
     __syncwarp();
     if (tr) tr[5] = global_ns();
     term = __shfl_sync(0xFFFFFFFFu, term, 0);
     if (term) return false;
-    for (int k = lane; k < cnt; k += 32) {
-        const int idx = move_to_index(S.q, S.mv[k]);
-        atomicOr(reinterpret_cast<unsigned long long*>(&S.mask[idx >> 6]), 1ull << (idx & 63));
-    }
+    mask_moves(S.q, S.mv, cnt, S.mask, lane);
     pack_planes_warp(d, g, gp, qslot, S.q, S.planes, lane);
     __syncwarp();
-    uint64_t* mrow = d.mask + (size_t)slot * MASK_STRIDE;
+    uint64_t* mrow = d.mask + (size_t)ps * MASK_STRIDE;
     for (int w = lane; w < MASK_STRIDE; w += 32) mrow[w] = S.mask[w];
-    uint64_t* prow = d.planes + (size_t)slot * PLANE_STRIDE;
+    uint64_t* prow = d.planes + (size_t)ps * PLANE_STRIDE;
     for (int i = lane; i < N_PLANES; i += 32) prow[i] = S.planes[i];
     return true;
 }
 
-// One thread per tree does the work; LPT = lanes per tree.  LPT = 1 packs 32 trees into a warp (bulk throughput: every lane
-// busy, but the lanes diverge through move generation and run one after the other); LPT = 32 gives every tree its own warp
-// (one active lane, no divergence: the latency of a step at the batch sizes of a search, a few thousand trees at most).
-template <int LPT>
+// warp per path slot: the expansion phase of a search that runs the phase kernels (profiling, the multi-leaf mode).  A path slot
+// is one in-flight simulation: slot * K + j (K = leaves per tree and step; 1 in the reference-exact mode).
 __global__ void __launch_bounds__(128) k_expand(Dev d) {
     __shared__ Tables T;
+    __shared__ ExpandShared ex_sh[4];
     load_tables(&T, d.tables);
-    const int tid = blockIdx.x * blockDim.x + threadIdx.x;
-    if (LPT > 1 && (tid % LPT) != 0) return;
-    // a path slot = one in-flight simulation: slot * K + j (K = leaves per tree and step; 1 in the reference-exact mode)
-    const int ps = d.g_begin * d.K + tid / LPT;
+    const int ps = d.g_begin * d.K + ((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     if (ps >= d.g_end * d.K) return;
-    expand_path(d, T, ps, d.planes + (size_t)ps * PLANE_STRIDE);
+    expand_warp<false>(d, T, ps, threadIdx.x & 31, ex_sh[threadIdx.x >> 5]);
 }
 
 // block per tree: policy[i] / value from the integer hash of the packed planes.  EC (evaluation cache, fused step): block i serves
@@ -1004,7 +969,7 @@ __global__ void __launch_bounds__(32 * FINISH_WARPS) k_tree_step(Dev d, float c_
     __syncwarp();
     stamp(3);
     ExpandShared& S = ex_sh[wib];
-    if (!expand_warp(d, T, slot, lane, S, tr)) return;
+    if (!expand_warp<true>(d, T, slot, lane, S, tr)) return;
     stamp(6);
     int row = slot;
     if (EC) {
@@ -1089,26 +1054,10 @@ __global__ void __launch_bounds__(128) k_select_vl(Dev d, float c_puct, int num_
                 if (lane == 0) { d.sel_node[ps] = node; d.sel_edge[ps] = -1; }
                 break;
             }
-            const float sq = sqrt_parent(np);
-            float best = -INFINITY;
-            int besti = 0x7FFFFFFF, best_n = 0;
-            uint16_t best_child = NO_CHILD;
-            for (int i = lane; i < n; i += 32) {
-                const int cn = d.e_n[e0 + i];
-                const uint16_t cc = link_child(d.e_link[e0 + i]);
-                const float sc = puct_score(cn, d.e_w[e0 + i], d.e_p[e0 + i], sq, c_puct);
-                if (sc > best || besti == 0x7FFFFFFF) { best = sc; besti = i; best_n = cn; best_child = cc; }
-            }
-#pragma unroll
-            for (int off = 16; off > 0; off >>= 1) {
-                const float ob = __shfl_down_sync(0xFFFFFFFFu, best, off);
-                const int oi = __shfl_down_sync(0xFFFFFFFFu, besti, off);
-                if (oi != 0x7FFFFFFF && (besti == 0x7FFFFFFF || ob > best || (ob == best && oi < besti))) { best = ob; besti = oi; }
-            }
-            besti = __shfl_sync(0xFFFFFFFFu, besti, 0);
-            np = __shfl_sync(0xFFFFFFFFu, best_n, besti & 31);
-            const uint16_t c = (uint16_t)__shfl_sync(0xFFFFFFFFu, (int)best_child, besti & 31);
-            const int e = e0 + besti;
+            // (only the pick: the headers come from node_nchild / node_edge0, because k_finish_vl does not keep e_link's up to date)
+            unsigned long long lk;
+            const int e = e0 + puct_pick(d, e0, n, sqrt_parent(np), c_puct, lane, np, lk);
+            const uint16_t c = link_child(lk);
             depth++;
             scanned += (unsigned long long)n;
             if (c == CHILD_PENDING) { dropped = true; break; }
@@ -1797,8 +1746,7 @@ static int run_search(szb_ctx* ctx, int num_searches, float c_puct, int learning
         if (K == 1) k_select<<<warp_blocks, 128, 0, cs>>>(dc, c_puct);
         else k_select_vl<<<warp_blocks, 128, 0, cs>>>(dc, c_puct, num_searches);
         if (ev) cudaEventRecord(ev[1], cs);
-        if (paths <= 8192) k_expand<32><<<(paths + 3) / 4, 128, 0, cs>>>(dc);
-        else k_expand<1><<<(paths + 127) / 128, 128, 0, cs>>>(dc);
+        k_expand<<<(paths + 3) / 4, 128, 0, cs>>>(dc);
         if (ev) cudaEventRecord(ev[2], cs);
         ctx->launches += 2;
         int rc_eval = 0;
