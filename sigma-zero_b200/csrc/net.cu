@@ -18,6 +18,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <cmath>
+#include <array>
 #include <map>
 #include <string>
 #include "engine.cuh"
@@ -101,6 +102,11 @@ struct Net {
     bool span_on = false;
     std::vector<int> span_boards, span_b0;
     std::string span_path;
+    // SZB_TOWER_TRACE inside searches: per-item stamps of the last TRACE_RING large-batch whole-tower launches (ring, dumped at destroy)
+    unsigned long long* trace_ring = nullptr;
+    std::string trace_path;
+    std::vector<std::array<long long, 5>> trace_meta;   // per ring slot: {launch ordinal, boards, tiles, pairs, span index or -1}
+    long long trace_launches = 0;
     int num_sms = 148;
     int pairs_resident = 74;             // CTA pairs of k_tower_tc2 this device holds at once (cudaOccupancyMaxActiveClusters)
     bool attr_set = false;               // per context (= per device): dynamic shared memory opt-ins done
@@ -357,6 +363,9 @@ constexpr int MAX_TOWER_LAYERS = 41;                      // stem + 38 tower con
 constexpr int POLICY_LAYER = MAX_TOWER_LAYERS - 1;
 constexpr int READY_PER_ITEM = 8;                         // 4 epilogue warps x 2 CTAs
 constexpr int SPAN_CAP = 1 << 17;                         // launches recorded by szb_tower_spans_record / SZB_TOWER_SPAN (a c2 bench run: 32,000)
+constexpr int TRACE_STAMPS = 5;                           // SZB_TOWER_TRACE stamps per item (TowerArgs::trace)
+constexpr int TRACE_RING = 64;                            // large-batch launches inside searches kept by SZB_TOWER_TRACE
+constexpr int TRACE_MAX_TILES = 128;                      // ... of at most 512 boards
 
 struct TowerLayer {
     uint8_t a_map;       // 0: input planes (128 ch), 1..3: activation buffer 0..2
@@ -422,7 +431,9 @@ struct TowerArgs {
     __nv_bfloat16* act[3];
     float* logits;       // [boards][4672]
     int32_t* error;
-    unsigned long long* trace;   // measurement aid (SZB_TOWER_TRACE): [item][4] %globaltimer stamps of the leader CTA, or null
+    unsigned long long* trace;   // measurement aid (SZB_TOWER_TRACE): [item][TRACE_STAMPS] %globaltimer stamps of the leader CTA, or null:
+                                 // 0 dependency resolved, 1 first chunk in shared memory, 2 accumulator complete, 3 stored and released,
+                                 // 4 last MMA of the item issued
     unsigned long long* span;    // measurement aid (SZB_TOWER_SPAN): {first CTA start, last CTA end (%globaltimer), CTA 0's SM cycles, CTA 0's ns}, or null
     TowerLayer L[MAX_TOWER_LAYERS];
 };
@@ -444,6 +455,18 @@ __device__ __forceinline__ TowerItem tower_item(const TowerArgs& a, int item, in
         it.ns = 1;
     }
     return it;
+}
+
+// 256-bit global accesses (sm_100): 16 bf16 channels of one pixel per instruction.  The tower epilogue's lanes hold different
+// pixels, so every instruction touches 32 lines whatever its width; twice the width is half the instructions and L1 wavefronts.
+// p must be 32-byte aligned.
+__device__ __forceinline__ void ldcg_256(const void* p, uint4& a, uint4& b) {
+    asm volatile("ld.global.cg.v8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                 : "=r"(a.x), "=r"(a.y), "=r"(a.z), "=r"(a.w), "=r"(b.x), "=r"(b.y), "=r"(b.z), "=r"(b.w) : "l"(p) : "memory");
+}
+__device__ __forceinline__ void st_256(void* p, const uint4& a, const uint4& b) {
+    asm volatile("st.global.v8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};"
+                 :: "l"(p), "r"(a.x), "r"(a.y), "r"(a.z), "r"(a.w), "r"(b.x), "r"(b.y), "r"(b.z), "r"(b.w) : "memory");
 }
 
 // one definition for every kernel that must agree bit for bit (k_softmax, the fused heads, k_value_head)
@@ -598,7 +621,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                 const int l = a.layer_begin + item / tiles, t = item % tiles;
                 const TowerLayer L = a.L[l];
                 if (l > a.layer_begin && !(ok = wait_dependency(l, t))) break;
-                if (a.trace && rank == 0 && lane == 0) a.trace[(size_t)item * 4 + 0] = global_ns();      // dependency resolved
+                if (a.trace && rank == 0 && lane == 0) a.trace[(size_t)item * TRACE_STAMPS + 0] = global_ns();      // dependency resolved
                 const CUtensorMap* tm_a = &maps.a[L.a_map];
                 const int board0 = a.board0 + (t * 2 + (int)rank) * 2 + (L.a_map == 0 ? a.in_delta : 0);
                 const int wrow = l * C_TOWER + (int)rank * L.n_half;
@@ -685,7 +708,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                 if (!ok) break;
                 pdl_wait();                                       // (weights above do not depend on the kernel before me; everything below does)
                 if (l > a.layer_begin && !(ok = wait_dependency(l, t))) break;
-                if (a.trace && rank == 0 && lane == 0) a.trace[(size_t)item * 4 + 0] = global_ns();      // dependency resolved
+                if (a.trace && rank == 0 && lane == 0) a.trace[(size_t)item * TRACE_STAMPS + 0] = global_ns();      // dependency resolved
                 for (int kc = 0; kc < L.kchunks && ok; kc++) {
                     if (!(ok = warp_mbar_wait(bar_ae0 + ac * 8, a_phase ^ 1, abort_flag))) break;
                     if (elect_one()) {
@@ -731,7 +754,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                 // N <= 128 MMAs of small-batch items -- so the nine taps of a K chunk are straight-line code (mma_chunk_3x3).
                 for (int kc = 0; kc < L.kchunks && ok; kc++) {
                     if (!(ok = warp_mbar_wait(bar_af0 + ac * 8, a_phase, abort_flag))) break;
-                    if (a.trace && kc == 0 && lane == 0) a.trace[(size_t)item * 4 + 1] = global_ns();     // first activation chunk in shared memory
+                    if (a.trace && kc == 0 && lane == 0) a.trace[(size_t)item * TRACE_STAMPS + 1] = global_ns();     // first activation chunk in shared memory
                     const uint32_t chunk_lo = a_lo0 + ac * (T2_A_CHUNK_BYTES >> 4);
                     if (L.taps == 9) {
                         // a weight stage holds nsplit consecutive taps of 128 / nsplit rows per CTA (see the producer)
@@ -761,6 +784,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                     __syncwarp();
                     if (++ac == T2_A_CHUNKS) { ac = 0; a_phase ^= 1; }
                 }
+                if (a.trace && lane == 0) a.trace[(size_t)item * TRACE_STAMPS + 4] = global_ns();        // last MMA of the item issued
                 if (ok && elect_one()) tc2_commit(bar_cf0 + acc * 8);
                 __syncwarp();
             }
@@ -796,20 +820,20 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
             const __nv_bfloat16* resp = (L.mode == 0 && L.res != 255 && live) ? a.act[L.res] + pix * C_TOWER + cb : nullptr;
             uint4 rnext[4];
             const bool early = l == a.layer_begin || ld_acquire_gpu(a.ready + (size_t)(l - 1) * a.n_pair_tiles + t) >= READY_PER_ITEM * a.nsplit;
-            if (resp && early) {
-#pragma unroll
-                for (int u = 0; u < 4; u++) rnext[u] = __ldcg(reinterpret_cast<const uint4*>(resp) + u);      // written by another SM: bypass L1
+            if (resp && early) {                                                                  // written by another SM: bypass L1
+                ldcg_256(resp, rnext[0], rnext[1]);
+                ldcg_256(resp + 16, rnext[2], rnext[3]);
             }
             ok = mbar_wait(smem_u32(&bar_acc_full[acc]), acc_phase, abort_flag);
             ok = __all_sync(0xFFFFFFFFu, ok);
             if (!ok) break;
             tc_fence_after();
             if (resp && !early) {
-#pragma unroll
-                for (int u = 0; u < 4; u++) rnext[u] = __ldcg(reinterpret_cast<const uint4*>(resp) + u);
+                ldcg_256(resp, rnext[0], rnext[1]);
+                ldcg_256(resp + 16, rnext[2], rnext[3]);
             }
             const bool tracer = a.trace && rank == 0 && warp == 2 && lane == 0;
-            if (tracer) a.trace[(size_t)item * 4 + 2] = global_ns();                    // accumulator complete
+            if (tracer) a.trace[(size_t)item * TRACE_STAMPS + 2] = global_ns();                    // accumulator complete
             if (L.mode == 1 && a.heads.mask != nullptr) {
                 // ===== fused heads (an unsplit item: all 73 planes of this CTA's two boards sit in this accumulator) =====
                 // Thread = (board, square) row with its 73 logits in TMEM.  softmax over the board's 4672 logits in the order
@@ -880,15 +904,16 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                 // ---- value head (network.py:156-174) on the tower output of this thread's pixel, same arithmetic as k_value_head ----
                 float p4[4] = {0.f, 0.f, 0.f, 0.f};
                 if (live) {
-                    const uint4* tp = reinterpret_cast<const uint4*>(a.heads.tower_out + pix * C_TOWER);
+                    const __nv_bfloat16* tp = a.heads.tower_out + pix * C_TOWER;
 #pragma unroll
                     for (int part = 0; part < 4; part++) {
 #pragma unroll
-                        for (int qq = 0; qq < 8; qq++) {
-                            const uint4 u = __ldcg(tp + part * 8 + qq);                 // written by other SMs during this launch
-                            const __nv_bfloat16* h8 = reinterpret_cast<const __nv_bfloat16*>(&u);
+                        for (int qq = 0; qq < 8; qq += 2) {
+                            uint4 u[2];
+                            ldcg_256(tp + part * 64 + qq * 8, u[0], u[1]);              // written by other SMs during this launch
+                            const __nv_bfloat16* h8 = reinterpret_cast<const __nv_bfloat16*>(u);
 #pragma unroll
-                            for (int j = 0; j < 8; j++) p4[part] = fmaf(__bfloat162float(h8[j]), hd_vw[part * 64 + qq * 8 + j], p4[part]);
+                            for (int j = 0; j < 16; j++) p4[part] = fmaf(__bfloat162float(h8[j]), hd_vw[part * 64 + qq * 8 + j], p4[part]);
                         }
                     }
                 }
@@ -949,8 +974,8 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
 #pragma unroll
                     for (int u = 0; u < 4; u++) rcur[u] = rnext[u];
                     if (c0 + 32 < n_item) {
-#pragma unroll
-                        for (int u = 0; u < 4; u++) rnext[u] = __ldcg(reinterpret_cast<const uint4*>(resp + c0 + 32) + u);
+                        ldcg_256(resp + c0 + 32, rnext[0], rnext[1]);
+                        ldcg_256(resp + c0 + 48, rnext[2], rnext[3]);
                     }
                 }
                 tmem_ld_wait();
@@ -970,9 +995,8 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                         if (L.relu) { x0 = fmaxf(x0, 0.f); x1 = fmaxf(x1, 0.f); }
                         ob[j] = __floats2bfloat162_rn(x0, x1);
                     }
-                    uint4* op = reinterpret_cast<uint4*>(outp + c0);
-#pragma unroll
-                    for (int u = 0; u < 4; u++) op[u] = o[u];
+                    st_256(outp + c0, o[0], o[1]);
+                    st_256(outp + c0 + 16, o[2], o[3]);
                 }
             }
             tc_fence_before();
@@ -983,7 +1007,7 @@ k_tower_tc2(const __grid_constant__ TowerMaps maps, const __grid_constant__ Towe
                 // orders its TMA (async-proxy) loads after its acquire with fence.proxy.async
                 fence_proxy_async_global();
                 red_release_gpu_add(a.ready + (size_t)l * a.n_pair_tiles + t, 1);
-                if (tracer) a.trace[(size_t)item * 4 + 3] = global_ns();                // outputs stored and released
+                if (tracer) a.trace[(size_t)item * TRACE_STAMPS + 3] = global_ns();                // outputs stored and released
             }
         }
     }
@@ -1721,6 +1745,39 @@ void net_destroy(szb_ctx* ctx) {
             }
         }
     }
+    if (ctx->net->trace_ring && ctx->net->trace_launches > 0) {
+        // the last TRACE_RING large-batch launches of the searches, oldest first; times relative to each launch's first stamp (or its
+        // first CTA's start when SZB_TOWER_SPAN records it too)
+        Net* net = ctx->net;
+        const size_t per = (size_t)MAX_TOWER_LAYERS * TRACE_MAX_TILES * TRACE_STAMPS;
+        std::vector<unsigned long long> h(per * TRACE_RING), sp(4 * net->span_boards.size());
+        cudaDeviceSynchronize();
+        if (cudaMemcpy(h.data(), net->trace_ring, h.size() * 8, cudaMemcpyDeviceToHost) == cudaSuccess &&
+            (sp.empty() || cudaMemcpy(sp.data(), net->span, sp.size() * 8, cudaMemcpyDeviceToHost) == cudaSuccess)) {
+            if (FILE* f = fopen(net->trace_path.c_str(), "a")) {
+                fprintf(f, "launch,boards,pairs,start_ns,end_ns,item,layer,tile,dep_ns,operands_ns,acc_ns,released_ns,last_mma_ns\n");
+                for (long long k = std::max(0ll, net->trace_launches - TRACE_RING); k < net->trace_launches; k++) {
+                    const std::array<long long, 5>& m = net->trace_meta[k % TRACE_RING];
+                    const unsigned long long* tr = h.data() + (size_t)(k % TRACE_RING) * per;
+                    const int tiles = (int)m[2];
+                    const size_t n_st = (size_t)MAX_TOWER_LAYERS * tiles * TRACE_STAMPS;
+                    unsigned long long t0 = ~0ull, s0 = 0, s1 = 0;
+                    if (m[4] >= 0) { s0 = sp[4 * m[4]]; s1 = sp[4 * m[4] + 1]; t0 = s0; }
+                    else for (size_t i = 0; i < n_st; i++) if (tr[i] && tr[i] < t0) t0 = tr[i];
+                    for (int item = 0; item < MAX_TOWER_LAYERS * tiles; item++) {
+                        fprintf(f, "%lld,%lld,%lld,%lld,%lld,%d,%d,%d", m[0], m[1], m[3], s0 ? 0ll : -1ll, s1 ? (long long)(s1 - t0) : -1ll,
+                                item, item / tiles, item % tiles);
+                        for (int j = 0; j < TRACE_STAMPS; j++) {
+                            const unsigned long long v = tr[(size_t)item * TRACE_STAMPS + j];
+                            fprintf(f, ",%lld", v ? (long long)(v - t0) : -1ll);
+                        }
+                        fprintf(f, "\n");
+                    }
+                }
+                fclose(f);
+            }
+        }
+    }
     for (void* p : ctx->net->allocs) cudaFree(p);
     delete ctx->net->tower_maps;
     delete ctx->net->tower_args;
@@ -1816,6 +1873,13 @@ static int net_setup_tower(szb_ctx* ctx, Net* net) {
     if ((rc = net_span_reset(ctx, net))) return rc;
     if (const char* sp = getenv("SZB_TOWER_SPAN")) {
         if (sp[0]) { net->span_path = sp; net->span_on = true; }
+    }
+    if (const char* tp = getenv("SZB_TOWER_TRACE")) {
+        if (tp[0]) {
+            net->trace_path = tp;
+            if ((rc = net_alloc(ctx, net, &net->trace_ring, (size_t)TRACE_RING * MAX_TOWER_LAYERS * TRACE_MAX_TILES * TRACE_STAMPS))) return rc;
+            net->trace_meta.assign(TRACE_RING, std::array<long long, 5>{-1, 0, 0, 0, -1});
+        }
     }
     net->tower_pairs = net->num_sms / 2;
     if (const char* e = getenv("SZB_TOWER_PAIRS")) { if (atoi(e) > 0) net->tower_pairs = std::min(atoi(e), net->num_sms / 2); }
@@ -1953,6 +2017,12 @@ static int launch_tower(szb_ctx* ctx, Net* net, int b0, int n, int layer_begin, 
         net->span_b0.push_back(b0);
     }
     const int grid = 2 * std::min(a.n_pair_tiles * a.nsplit, pairs);
+    if (net->trace_ring && !a.trace && a.nsplit == 1 && !a.heads.n_live && layers == MAX_TOWER_LAYERS && a.n_pair_tiles <= TRACE_MAX_TILES) {
+        const int slot = (int)(net->trace_launches % TRACE_RING);
+        a.trace = net->trace_ring + (size_t)slot * MAX_TOWER_LAYERS * TRACE_MAX_TILES * TRACE_STAMPS;
+        net->trace_meta[slot] = {net->trace_launches, n, a.n_pair_tiles, grid / 2, a.span ? (long long)net->span_boards.size() - 1 : -1};
+        net->trace_launches++;
+    }
     SZB_CUDA(ctx, launch_kernel(a.heads.mask && a.heads.n_live ? k_tower_tc2<true> : k_tower_tc2<false>, dim3(grid), dim3(TC_THREADS), (size_t)(exclusive ? net->smem_exclusive : T2_SMEM), ctx->work,
                                 run.pdl, *net->tower_maps, a));
     ctx->launches++;
@@ -2504,7 +2574,7 @@ int szb_time_kernel(szb_ctx* ctx, int32_t which, int32_t n, int32_t iters, float
     }
     if (which == 5 && trace_path && trace_path[0]) {
         const int tiles = (n + 3) / 4;
-        const size_t slots = (size_t)MAX_TOWER_LAYERS * tiles * 8 * 4;
+        const size_t slots = (size_t)MAX_TOWER_LAYERS * tiles * 8 * TRACE_STAMPS;
         unsigned long long* d_tr = nullptr;
         SZB_CUDA(ctx, cudaMalloc((void**)&d_tr, slots * 8));
         SZB_CUDA(ctx, cudaMemsetAsync(d_tr, 0, slots * 8, ctx->stream));
@@ -2519,12 +2589,13 @@ int szb_time_kernel(szb_ctx* ctx, int32_t which, int32_t n, int32_t iters, float
         unsigned long long t0 = ~0ull;
         for (unsigned long long v : h) if (v && v < t0) t0 = v;
         if (FILE* f = fopen(trace_path, "a")) {
-            fprintf(f, "boards,nsplit,item,layer,tile,q,dep_ns,operands_ns,acc_ns,released_ns\n");
+            fprintf(f, "boards,nsplit,item,layer,tile,q,dep_ns,operands_ns,acc_ns,released_ns,last_mma_ns\n");
             const int nsplit = net->last_nsplit;
             for (int item = 0; item < MAX_TOWER_LAYERS * tiles * nsplit; item++) {
                 const int ti = item / nsplit;
                 fprintf(f, "%d,%d,%d,%d,%d,%d", n, nsplit, item, ti / tiles, ti % tiles, item % nsplit);
-                for (int k = 0; k < 4; k++) fprintf(f, ",%lld", h[(size_t)item * 4 + k] ? (long long)(h[(size_t)item * 4 + k] - t0) : -1ll);
+                for (int k = 0; k < TRACE_STAMPS; k++)
+                    fprintf(f, ",%lld", h[(size_t)item * TRACE_STAMPS + k] ? (long long)(h[(size_t)item * TRACE_STAMPS + k] - t0) : -1ll);
                 fprintf(f, "\n");
             }
             fclose(f);
